@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- decode tok/s (+ verified tok/s) of the blama hot path on B200, one model replica per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--shape llama-3.1-8b-q4km]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--shape llama-3.1-8b-q4km] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...        (one rank per GPU)
 
 A "step" is one /complete request of BASELINE.json configs[1]: a 512-token synthetic prompt, then 256 new tokens on
@@ -14,6 +14,10 @@ random-init Llama-3.1-8B-arch Q4_K_M weights.  Printed JSON line (rank 0):
            against the measured HBM copy bandwidth in MEASURED_PEAKS.json
   cpu_baseline  the oracle (CPU restatement of the reference's ggml-cpu arithmetic, kind "port") on the box's host cores
 --impl reference times that CPU port on the same metric (the real blama CPU build cannot be produced offline, DESIGN.md).
+--dump-outputs DIR writes what the last timed step returned (rank 0) as DIR/<name>.npy, float32 or float64: the /complete
+tokens and top-10 lists, the logits row and top-10 after the device-resident loop, and (--verify > 0) the score of the last
+verify request.
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -347,6 +351,11 @@ def run_ours(args, rank: int, world: int, local_rank: int):
             dev_ms.append(ms); e2e_s.append(t2 - t1); prompt_ms.append((t1 - t0) * 1e3)
             e2e_tokens += len(toks)                # complete() stops early at an end-of-generation token
         assert len(toks) > 0
+        if args.dump_outputs and s == total - 1:      # read back after the timer stopped: the timed region is unchanged
+            loop_top = ctx.topk(10)
+            outputs = {"complete_tokens": toks, "complete_top10_tokens": top["token"], "complete_top10_logits": top["logit"],
+                       "decode_loop_logits": ctx.logits(), "decode_loop_top10_tokens": loop_top["token"],
+                       "decode_loop_top10_logits": loop_top["logit"]}
     barrier()
     sampler.stop_flag.set()
     launches = ctx.kernel_launches - (launches0 or 0)
@@ -376,6 +385,8 @@ def run_ours(args, rank: int, world: int, local_rank: int):
             inst.stop_session()
             if r > 0 or args.sequential_verify:
                 vt.append(dt)
+        if args.dump_outputs:
+            outputs["verify_score"] = np.array([score])
         t_v = max_over_ranks(statistics.median(vt))
         verify = {"tokens": int(len(vt_l)), "tok_s": sum_over_ranks(float(len(vt_l))) / t_v, "ms": t_v * 1e3, "reps": len(vt),
                   "ms_min": min(vt) * 1e3, "ms_max": max(vt) * 1e3, "timing": "median wall time of the timed requests (host buffers in, score out), L2 flushed before each",
@@ -414,6 +425,8 @@ def run_ours(args, rank: int, world: int, local_rank: int):
                               "traffic_source": "profiles/r2_ncu_verify_summary.json (sum of dram__bytes over the kernels of one verify prefill)" if traffic_v else None,
                               "note": "flops = executed work (claimed-id rows of the head only); flops_if_full_vocab_head = SURVEY 8d's count"}
 
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, outputs)
     if rank != 0:
         dist.close()
         return
@@ -624,6 +637,22 @@ def emit(line: dict):
         os.write(_JSON_FD, data)
 
 
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def write_outputs(out_dir: str, arrays: dict) -> None:
+    """--dump-outputs: DIR/<name>.npy per array; float32 stays float32, everything else (token ids, scores) becomes float64,
+    which holds every int32 exactly.  Refuses to write more than DUMP_LIMIT_BYTES in all."""
+    conv = {name: np.ascontiguousarray(a, dtype=np.float32 if np.asarray(a).dtype == np.float32 else np.float64)
+            for name, a in arrays.items()}
+    total = sum(a.nbytes for a in conv.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in conv.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -644,7 +673,12 @@ def main():
     ap.add_argument("--workers-per-gpu", type=int, default=1, help="--mode stream / mix: Server workers (Instances) sharing each replica: with 2, "
                     "one request's host work (claimed-id preparation, LogitComparer) overlaps the other's prefill")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="--mode step: write the outputs of the last timed step (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.impl != "ours" or args.mode != "step"):
+        ap.error("--dump-outputs applies to --impl ours --mode step")
     rank, world, local_rank = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     if not (args.gpus > 1 and world == 1 and args.mode == "step"):
         quiet_stdout()

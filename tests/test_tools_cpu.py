@@ -1,10 +1,12 @@
-"""CPU checks of the measurement helpers: the parity bookkeeping of bench.py / the GPU tests, and the ncu launch-list summariser."""
+"""CPU checks of the measurement helpers: the parity bookkeeping of bench.py / the GPU tests, bench.py's output dump, and the ncu
+launch-list summariser."""
 import json
 import os
 import subprocess
 import sys
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -25,6 +27,26 @@ def test_parity_stats_top10_figures():
     assert s["floor_top10_id_match_frac"] == 1.0 and s["floor_top1_match_frac"] == 1.0 and s["floor_top10_overlap_mean"] == 1.0
     assert s["within_floor"] is False                            # 0.05 of noise against a floor of 1e-6
     assert abs(s["max_abs"] - err) < 1e-9
+
+
+def test_bench_write_outputs_dtypes_and_limit(tmp_path):
+    import bench
+
+    toks = np.array([5, 128255, 2**31 - 1], dtype=np.int32)
+    logits = np.linspace(-3, 3, 7, dtype=np.float32)
+    bench.write_outputs(str(tmp_path / "d"), {"tokens": toks, "logits": logits, "score": np.array([0.25])})
+    got = {p.stem: np.load(p) for p in (tmp_path / "d").iterdir()}
+    assert sorted(got) == ["logits", "score", "tokens"]
+    assert got["tokens"].dtype == np.float64 and np.array_equal(got["tokens"], toks)
+    assert got["logits"].dtype == np.float32 and np.array_equal(got["logits"], logits)
+    assert got["score"].dtype == np.float64 and got["score"][0] == 0.25
+    with pytest.raises(ValueError):
+        bench.write_outputs(str(tmp_path / "big"), {"x": np.zeros(bench.DUMP_LIMIT_BYTES // 8 + 1)})
+    assert not (tmp_path / "big").exists()
+    # the reference arm has no device outputs to write: refused before any work
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path / "ref")],
+                       capture_output=True, text=True)
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr and not (tmp_path / "ref").exists()
 
 
 def test_ncu_summary_selects_the_last_pass(tmp_path):
