@@ -12,7 +12,7 @@ from typing import Optional, Sequence, Tuple
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-# BLAMA_B200_LIB: an alternative build of the same library (kernel A/B experiments: tools/decode_ab.py)
+# BLAMA_B200_LIB: an alternative build of the same library (build-against-build A/B runs: tools/decode_lib_ab.py)
 LIB_PATH = os.environ.get("BLAMA_B200_LIB") or os.path.join(HERE, "lib", "libblama_b200.so")
 
 TD_DTYPE = np.dtype([("token", np.int32), ("logit", np.float32)])

@@ -643,24 +643,6 @@ __global__ void __launch_bounds__(1024) topk_select_kernel(TopkArgs a) {
     if (tid == 0) { *a.count = 0u; *a.done = 0u; }
 }
 
-// L2 prefetch of upcoming weights.  Batch-1 decode alternates short HBM-bound mat-vecs with latency-bound glue
-// (attention, norms); on its own the memory system idles during the glue.  These kernels run on a second stream, one
-// phase ahead of the consumer, and pull the next matrices into the 126 MB L2 so HBM streams continuously and the
-// mat-vecs then read L2-resident data.  Pure hint: no data dependency, results are unaffected.
-struct PrefetchArgs {
-    const uint8_t* ptr[8];
-    unsigned long long bytes[8];
-    int n;
-};
-__global__ void __launch_bounds__(256) l2_prefetch_kernel(const PrefetchArgs a) {
-    const size_t tid = (size_t)blockIdx.x * blockDim.x + threadIdx.x, nthr = (size_t)gridDim.x * blockDim.x;
-    for (int r = 0; r < a.n; r++) {
-        const size_t lines = (a.bytes[r] + 127) >> 7;
-        for (size_t i = tid; i < lines; i += nthr)
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(a.ptr[r] + (i << 7)));
-    }
-}
-
 __global__ void gather_logits_kernel(const float* __restrict__ logits, int n_vocab, const int32_t* __restrict__ ids, int n, float* out) {
     pdl_launch_dependents(); pdl_wait();
     const int i = blockIdx.x * blockDim.x + threadIdx.x;

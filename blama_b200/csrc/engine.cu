@@ -164,15 +164,6 @@ bool mega_geometry(int K, int& W, int& L, int& rpc) {
     return W <= MG_WARPS;
 }
 
-// QKV of a 4096-wide model: 3072 row pairs over 148 x 16 warps is 1.3 pairs per warp -- a third of the warps carry two pairs = four
-// chunks, one more than the ring holds, so the phase waits for an HBM round trip.  With two warps per pair every warp has two or
-// three (half as long) chunks, all prefetched.  (0 = keep the geometry of mega_geometry)
-int mega_default_w_qkv(int K) {
-    static const int forced = [] { const char* e = getenv("BLK_MEGA_W_QKV_DEFAULT"); return e ? atoi(e) : -1; }();
-    if (forced >= 0) return forced;
-    return 0;
-}
-
 MegaPlan mega_plan(blk_model* m, GgufFile& f, int n_sms) {
     MegaPlan pl;
     blk_mega_model& mg = m->mega;
@@ -182,41 +173,20 @@ MegaPlan mega_plan(blk_model* m, GgufFile& f, int n_sms) {
     auto ttype = [&](const std::string& n) -> int { const GgufTensor* t = f.find(n); return t ? t->type : -1; };
     const bool tied = f.find("output.weight") == nullptr;
     mg.n_cta = n_sms;
-    {   // BLK_MEGA_CTAS: CTAs of the persistent kernel (<= SMs).  Fewer CTAs than SMs can divide the row pairs of every phase evenly
-        // (4096 / 14336-wide models: 128 CTAs x 16 warps = 2048 warps -> 3 / 1 / 7 / 4 items per warp group, no remainder round)
-        const char* e = getenv("BLK_MEGA_CTAS");
-        if (e && atoi(e) >= m->n_head_kv && atoi(e) <= n_sms) mg.n_cta = atoi(e);
-    }
-    int64_t rot_acc = 0;
     int max_items = 1, slot = 0, kmax = 0;
     bool bad = false;
     auto add_phase = [&](int layer, int K, int src, std::initializer_list<std::tuple<std::string, int, int, int, int>> segs /*tensor, n_pairs, kind, rowmap, ab*/) {
         MegaPhase ph{};
         if (!mega_geometry(K, ph.W, ph.L, ph.rpc)) { bad = true; return; }
-        {   // finer K split of a phase (more, shorter chunks per row pair: every warp's share fits its ring, smaller remainder):
-            // BLK_MEGA_W_QKV / _WO / _GU / _DOWN / _HEAD = warps per row pair
-            const int kind0 = std::get<2>(*segs.begin());
-            const char* key = kind0 == MK_Q ? "BLK_MEGA_W_QKV" : kind0 == MK_SWIGLU ? "BLK_MEGA_W_GU" : kind0 == MK_LOGITS ? "BLK_MEGA_W_HEAD" :
-                              (src == MSRC_ATTN ? "BLK_MEGA_W_WO" : "BLK_MEGA_W_DOWN");
-            const char* e = getenv(key);
-            int w = e ? atoi(e) : (kind0 == MK_Q ? mega_default_w_qkv(K) : 0);
-            const int halfs = K / 128;
-            if (w > ph.W && w <= MG_WARPS && (MG_WARPS % w) == 0 && halfs % (2 * w) == 0) {
-                ph.W = w; ph.L = halfs / w; ph.rpc = (2 * ph.L <= 32) ? 2 : 1;
-            }
-        }
         ph.K = K; ph.src = src; ph.layer = layer; ph.nseg = 0;
         const int NGtot = mg.n_cta * (MG_WARPS / ph.W);
         int items = 0;
         // The segments of a phase occupy consecutive warp groups, starting so that the chain ENDS at the last group: the groups that
         // carry one pair more than the others are the highest CTAs.  CTAs 0 .. n_head_kv * n_split - 1 run the attention stages (and
         // CTAs 0 .. n_head_kv - 1 the split combine), so the extra QKV pairs and the idle groups of Wo keep off the attention's path.
-        {
-            int64_t total = 0;
-            for (auto& sgd : segs) if (!(std::get<2>(sgd) == MK_SWIGLU && std::get<4>(sgd) == 1)) total += std::get<1>(sgd);
-            static const bool top = [] { const char* e = getenv("BLK_ROT_TOP"); return !(e && e[0] == '0'); }();
-            if (top) rot_acc = (NGtot - total % NGtot) % NGtot;          // first group of the chain
-        }
+        int64_t total = 0;
+        for (auto& sgd : segs) if (!(std::get<2>(sgd) == MK_SWIGLU && std::get<4>(sgd) == 1)) total += std::get<1>(sgd);
+        int64_t rot_acc = (NGtot - total % NGtot) % NGtot;          // first group of the chain
         const int pi = (int)mg.phases.size();
         for (auto& sgd : segs) {
             const std::string& name = std::get<0>(sgd);
@@ -557,8 +527,6 @@ blk_ctx::~blk_ctx() {
     if (ev0) cudaEventDestroy(ev0);
     if (ev1) cudaEventDestroy(ev1);
     for (int i = 0; i < 4; i++) { if (pn_filled[i]) cudaEventDestroy(pn_filled[i]); if (pn_start[i]) cudaEventDestroy(pn_start[i]); }
-    if (pf_fork) cudaEventDestroy(pf_fork);
-    if (pf_join) cudaEventDestroy(pf_join);
     if (pf_stream) cudaStreamDestroy(pf_stream);
     if (stream) cudaStreamDestroy(stream);
 }
@@ -643,39 +611,6 @@ void matvec(blk_ctx* c, GemvArgs& a, const float* in, const float* norm_w, const
     prof_mark(c, name);
 }
 
-// launch an L2 prefetch of the given matrices on the prefetch stream, ordered after everything enqueued so far on the
-// main stream (i.e. it starts when the previous phase has completed and overlaps the phase enqueued next)
-void prefetch_after_current(blk_ctx* c, std::initializer_list<const QMat*> mats, int which = 0, size_t max_bytes = (size_t)96 << 20) {
-    if (!c->use_prefetch || !((c->pf_mask >> which) & 1)) return;
-    PrefetchArgs pa{};
-    size_t budget = max_bytes;
-    for (const QMat* W : mats) {
-        const uint8_t* planes[4] = {W->p0, W->p1, W->p2, W->p3};
-        size_t sizes[4] = {0, 0, 0, 0};
-        const size_t nsb = (size_t)W->N * (W->K / 256), nb32 = (size_t)W->N * (W->K / 32);
-        switch (W->type) {
-            case QT_Q4_K: sizes[0] = nsb * 128; sizes[1] = nsb * 16; break;
-            case QT_Q5_K: sizes[0] = nsb * 128; sizes[1] = nsb * 16; sizes[2] = nsb * 32; break;
-            case QT_Q6_K: sizes[0] = nsb * 128; sizes[1] = nsb * 64; sizes[2] = nsb * 16; sizes[3] = nsb * 2; break;
-            case QT_Q8_0: sizes[0] = nb32 * 32; sizes[1] = nb32 * 2; break;
-            default: sizes[0] = W->bytes; break;
-        }
-        for (int i = 0; i < 4 && pa.n < 8; i++) {
-            if (!planes[i] || !sizes[i] || !budget) continue;
-            const size_t take = std::min(sizes[i], budget);
-            pa.ptr[pa.n] = planes[i]; pa.bytes[pa.n] = take; pa.n++;
-            budget -= take;
-        }
-    }
-    if (!pa.n) return;
-    BLK_CUDA(cudaEventRecord(c->pf_fork, c->stream));
-    BLK_CUDA(cudaStreamWaitEvent(c->pf_stream, c->pf_fork, 0));
-    l2_prefetch_kernel<<<c->pf_ctas, c->pf_threads, 0, c->pf_stream>>>(pa);
-    BLK_CUDA(cudaGetLastError());
-    c->launches++;
-    c->pf_used = true;
-}
-
 // one decode step on c->stream: token id in c->d_tok, position in c->d_pos.
 // Per layer: QKV mat-vec (RMSNorm prologue; +bias, RoPE, KV-page write) | attention | Wo mat-vec (+residual) |
 // gate/up mat-vec (RMSNorm prologue; SwiGLU) | down mat-vec (+residual); then final norm + lm_head mat-vec + top-k.
@@ -710,10 +645,8 @@ void enqueue_step(blk_ctx* c, bool with_head, bool feedback = false) {
     BLK_CUDA(launch_pdl(embed_kernel, dim3(1), dim3(256), 0, c->stream, m->tok_embd, c->d_tok, c->d_pos, c->x, c->rope_cs, dh / 2, m->theta_scale, m->rope_freqs));
     c->launches++;
     prof_mark(c, "embed");
-    c->pf_used = false;
     for (int l = 0; l < m->n_layer; l++) {
         const LayerWeights& L = m->layers[l];
-        if (!c->profiling) prefetch_after_current(c, {&L.wo}, 0);                          // overlaps the QKV mat-vec
         {
             GemvArgs a{};
             a.nseg = 3;
@@ -727,7 +660,6 @@ void enqueue_step(blk_ctx* c, bool with_head, bool feedback = false) {
             matvec<EPI_QKV>(c, a, c->x, L.attn_norm, c->act_d, "gemv_qkv");
         }
         {
-            if (!c->profiling) prefetch_after_current(c, {&L.gate, &L.up}, 1);             // overlaps attention + Wo
             if (c->attn_cluster > 0) {
                 AttnClusterArgs ac{};
                 ac.q = c->qbuf; ac.k_pool = c->k_pool[l]; ac.v_pool = c->v_pool[l]; ac.page_table = c->page_table; ac.pos = c->d_pos;
@@ -770,15 +702,10 @@ void enqueue_step(blk_ctx* c, bool with_head, bool feedback = false) {
             a.nseg = 1; a.seg[0] = {L.wo, nullptr, 0, 0}; a.total_pairs = d / 2; a.out = c->x;
             matvec<EPI_RESID>(c, a, c->act_q.f32, nullptr, c->act_q2, "gemv_wo");
         }
-        if (!c->profiling) prefetch_after_current(c, {&L.down}, 2);                        // overlaps the gate/up mat-vec
         {
             GemvArgs a{};
             a.nseg = 2; a.seg[0] = {L.gate, nullptr, 0, 0}; a.seg[1] = {L.up, nullptr, 0, 0}; a.total_pairs = ff; a.out = c->hbuf;
             matvec<EPI_SWIGLU>(c, a, c->x, L.ffn_norm, c->act_d, "gemv_gate_up");
-        }
-        if (!c->profiling) {                                                            // overlaps the down mat-vec
-            if (l + 1 < m->n_layer) prefetch_after_current(c, {&m->layers[l + 1].wq, &m->layers[l + 1].wk, &m->layers[l + 1].wv}, 3);
-            else if (with_head) prefetch_after_current(c, {&m->output}, 4);
         }
         {
             GemvArgs a{};
@@ -798,10 +725,6 @@ void enqueue_step(blk_ctx* c, bool with_head, bool feedback = false) {
         BLK_CUDA(launch_pdl(topk_select_kernel, dim3(16), dim3(1024), 0, c->stream, tk));
         c->launches++;
         prof_mark(c, "topk_select");
-    }
-    if (c->pf_used) {      // join the prefetch branch back into the main stream
-        BLK_CUDA(cudaEventRecord(c->pf_join, c->pf_stream));
-        BLK_CUDA(cudaStreamWaitEvent(c->stream, c->pf_join, 0));
     }
     BLK_CUDA(launch_pdl(advance_pos_kernel, dim3(1), dim3(32), 0, c->stream, c->d_pos, 1));
     c->launches++;
@@ -1013,13 +936,10 @@ void ensure_prefill_bufs(blk_ctx* c, int T) {
     c->pf_g = dalloc<float>(c, t * ff); c->pf_u = dalloc<float>(c, t * ff);
     c->pf_h = dalloc<__nv_bfloat16>(c, t * ff);
     {   // split-K workspace of the prefill GEMMs (few-token batches): splits * tiles <= SMs, a tile is 256 x 256 f32
-        const char* e = getenv("BLK_SPLITK");
         int sms = 0; BLK_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, m->device));
-        c->pf_splitk_elems = (e && e[0] == '0') ? 0 : (size_t)sms * 65536;
-        c->pf_splitk = c->pf_splitk_elems ? dalloc<float>(c, c->pf_splitk_elems) : nullptr;
+        c->pf_splitk_elems = (size_t)sms * 65536;
+        c->pf_splitk = dalloc<float>(c, c->pf_splitk_elems);
     }
-    // opt-in (measured neutral: 28.0 against 27.4-28.3 ms per 2048-token verify): work items of the prefill GEMMs taken with atomicAdd
-    { const char* e = getenv("BLK_GEMM_DYNAMIC"); c->pf_sched = (e && e[0] == '1') ? dalloc<int>(c, blk_ctx::PF_SCHED_CAP) : nullptr; }
     c->pf_logit_rows = 512;     // rows of one lm_head chunk: two M tiles share every weight tile through L2
     c->pf_logits = dalloc<float>(c, (size_t)c->pf_logit_rows * m->n_vocab);
     if (prefill_attn_tc_supported(dh, m->n_head, m->n_head_kv)) {      // transposed-V scratch of the tcgen05 attention (one layer at a time)
@@ -1060,20 +980,18 @@ void launch_attn_gqa(const PrefillAttnArgs& pa, int n, int n_head_kv, cudaStream
 void launch_prefill_attn(blk_ctx* c, const PrefillAttnArgs& pa, int n, cudaStream_t st) {
     const blk_model* m = c->m;
     const int dh = m->d_head, gq = m->n_head / m->n_head_kv;
-    static const bool per_head = [] { const char* e = getenv("BLK_ATTN_PER_HEAD"); return e && e[0] == '1'; }();
-    static const bool no_tc = [] { const char* e = getenv("BLK_ATTN_TC"); return e && e[0] == '0'; }();
-    if (!no_tc && !per_head && c->pf_vt && prefill_attn_tc_supported(dh, m->n_head, m->n_head_kv)) {
+    if (c->pf_vt && prefill_attn_tc_supported(dh, m->n_head, m->n_head_kv)) {
         // tcgen05 attention: the layer's pools are recovered from the arguments
         BLK_CUDA(prefill_attn_tc(pa.q, pa.k_pool, pa.v_pool, pa.page_table, c->n_pages, pa.pos0, c->n_past, pa.out, c->pf_vt, c->pf_vt_pad, n,
                                  m->n_head, m->n_head_kv, pa.kv_dim, pa.scale, st));
         return;
     }
-    if (!per_head && dh == 128 && gq == 4) launch_attn_gqa<128, 4>(pa, n, m->n_head_kv, st);
-    else if (!per_head && dh == 128 && gq == 8) launch_attn_gqa<128, 8>(pa, n, m->n_head_kv, st);
-    else if (!per_head && dh == 128 && gq == 2) launch_attn_gqa<128, 2>(pa, n, m->n_head_kv, st);
-    else if (!per_head && dh == 64 && gq == 4) launch_attn_gqa<64, 4>(pa, n, m->n_head_kv, st);
-    else if (!per_head && dh == 64 && gq == 8) launch_attn_gqa<64, 8>(pa, n, m->n_head_kv, st);
-    else if (!per_head && dh == 64 && gq == 2) launch_attn_gqa<64, 2>(pa, n, m->n_head_kv, st);
+    if (dh == 128 && gq == 4) launch_attn_gqa<128, 4>(pa, n, m->n_head_kv, st);
+    else if (dh == 128 && gq == 8) launch_attn_gqa<128, 8>(pa, n, m->n_head_kv, st);
+    else if (dh == 128 && gq == 2) launch_attn_gqa<128, 2>(pa, n, m->n_head_kv, st);
+    else if (dh == 64 && gq == 4) launch_attn_gqa<64, 4>(pa, n, m->n_head_kv, st);
+    else if (dh == 64 && gq == 8) launch_attn_gqa<64, 8>(pa, n, m->n_head_kv, st);
+    else if (dh == 64 && gq == 2) launch_attn_gqa<64, 2>(pa, n, m->n_head_kv, st);
     else {
         const dim3 agrid((n + 63) / 64, m->n_head);
         if (dh == 128) prefill_attn_kernel<128><<<agrid, 128, 3 * 64 * (128 + 8) * 2, st>>>(pa);
@@ -1105,8 +1023,7 @@ void prefill_chunk(blk_ctx* c, const int32_t* tokens, int n, const VerifyIo* ver
     //   starts (its panel's previous user, GEMM i-3, is then done), so fills overlap GEMMs, not the small bandwidth-bound kernels.
     // verify without the verifier's own per-position top-10: only the logits at the claimed ids are needed (what the reference's
     // fillCtx reads, Session.cpp:263-282) -> sparse rows of the vocabulary projection instead of the T x V GEMM
-    static const bool full_head_env = [] { const char* e = getenv("BLK_VERIFY_FULL_HEAD"); return e && e[0] == '1'; }();
-    const bool sparse_head = verify && !verify->top && !full_head_env && m->output.type != QT_F32 && m->output.type != QT_F16 && (d % 64) == 0;
+    const bool sparse_head = verify && !verify->top && m->output.type != QT_F32 && m->output.type != QT_F16 && (d % 64) == 0;
     const int n_ops = 4 * m->n_layer + (verify && !sparse_head ? 1 : 0);
     // GEMM form per matrix: resident bf16 panel (model cache) -> TMA-fed GEMM at every batch size; otherwise many tokens: the matrix is
     // de-quantised ONCE into a streaming panel (second stream, one GEMM ahead); few tokens: the fused form (weights de-quantised
@@ -1147,11 +1064,9 @@ void prefill_chunk(blk_ctx* c, const int32_t* tokens, int n, const VerifyIo* ver
     auto after_gemm = [&](int) {};
     if (panel && !res_op(0)) { BLK_CUDA(cudaEventRecord(c->pn_start[0], st)); BLK_CUDA(cudaStreamWaitEvent(c->pf_stream, c->pn_start[0], 0)); }   // after whatever ran before
     fill_op(0);
-    int sched_next = 0;
-    if (c->pf_sched) BLK_CUDA(cudaMemsetAsync(c->pf_sched, 0, blk_ctx::PF_SCHED_CAP * sizeof(int), st));
     // few-token batches: the split-K reduce of Wo / down (accumulates onto the residual stream) is folded into the RMSNorm that follows
     PendingReduce pend;
-    const SplitKWs sk{c->pf_splitk, c->pf_splitk_elems, c->pf_sched, &sched_next, blk_ctx::PF_SCHED_CAP, &pend};
+    const SplitKWs sk{c->pf_splitk, c->pf_splitk_elems, &pend};
     SplitKWs sk_last = sk; sk_last.defer = nullptr;      // the last down GEMM of a pass that is not followed by the final RMSNorm kernel
     for (int l = 0; l < m->n_layer; l++) {
         const LayerWeights& L = m->layers[l];
@@ -1314,11 +1229,6 @@ extern "C" blk_ctx* blk_ctx_create(blk_model* m, int32_t n_ctx, int32_t n_batch)
         BLK_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
         BLK_CUDA(cudaEventCreate(&c->ev0)); BLK_CUDA(cudaEventCreate(&c->ev1));
         BLK_CUDA(cudaStreamCreateWithFlags(&c->pf_stream, cudaStreamNonBlocking));
-        BLK_CUDA(cudaEventCreateWithFlags(&c->pf_fork, cudaEventDisableTiming)); BLK_CUDA(cudaEventCreateWithFlags(&c->pf_join, cudaEventDisableTiming));
-        { const char* e = getenv("BLK_PREFETCH"); c->use_prefetch = (e && e[0] == '1'); }   // opt-in: measured slower (DESIGN.md)
-        { const char* e = getenv("BLK_PF_MASK"); c->pf_mask = e ? atoi(e) : 31; }
-        { const char* e = getenv("BLK_PF_THREADS"); c->pf_threads = e ? atoi(e) : 256; }
-        { const char* e = getenv("BLK_PF_CTAS"); c->pf_ctas = e ? atoi(e) : 148; }
         const int d = m->n_embd, dh = m->d_head, dq = m->n_head * dh, dkv = m->n_head_kv * dh, ff = m->n_ff;
         c->n_pages = (c->n_ctx + KV_PAGE - 1) / KV_PAGE;
         c->k_pool.resize(m->n_layer); c->v_pool.resize(m->n_layer);
@@ -1346,8 +1256,7 @@ extern "C" blk_ctx* blk_ctx_create(blk_model* m, int32_t n_ctx, int32_t n_batch)
             c->attn_cluster = 8;
             c->attn_cap = (c->n_pages * KV_PAGE + c->attn_cluster - 1) / c->attn_cluster;
             const size_t smem = (size_t)gq * (c->attn_cap + (ATTN_THREADS / 32) * m->d_head) * sizeof(float);
-            const char* e = getenv("BLK_NO_CLUSTER_ATTN");
-            if (smem > 160 * 1024 || (e && e[0] == '1')) c->attn_cluster = 0;
+            if (smem > 160 * 1024) c->attn_cluster = 0;
             else {
                 BLK_CUDA(cudaFuncSetAttribute(attn_cluster_kernel<128, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 164 * 1024));
                 BLK_CUDA(cudaFuncSetAttribute(attn_cluster_kernel<128, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 164 * 1024));
@@ -1380,18 +1289,16 @@ extern "C" blk_ctx* blk_ctx_create(blk_model* m, int32_t n_ctx, int32_t n_batch)
             MegaParams& P = c->mega_params;
             P.phases = mg.d_phases; P.n_phases = (int)mg.phases.size(); P.n_layer = m->n_layer;
             P.chunk_list = mg.d_list; P.chunk_counts = mg.d_counts; P.list_stride = mg.list_stride;
-            P.n_cta = mg.n_cta; P.slot_bytes = mg.slot_bytes; P.max_items = mg.max_items; P.act_bytes = mg.act_bytes; P.ts_cap = mg.ts_cap; P.ts_target = mg.ts_cap; { const char* e = getenv("BLK_ATTN_TS"); if (e && atoi(e) >= 8) P.ts_target = std::min(mg.ts_cap, atoi(e)); } P.attn_off = mg.attn_off;
+            P.n_cta = mg.n_cta; P.slot_bytes = mg.slot_bytes; P.max_items = mg.max_items; P.act_bytes = mg.act_bytes; P.ts_cap = mg.ts_cap; P.attn_off = mg.attn_off;
             P.tok_embd = m->tok_embd;
             P.n_embd = d; P.n_head = m->n_head; P.n_head_kv = m->n_head_kv; P.d_head = dh; P.n_ff = ff; P.n_vocab = m->n_vocab; P.neox = m->neox ? 1 : 0;
             P.eps = m->rms_eps; P.theta_scale = m->theta_scale; P.attn_scale = 1.0f / sqrtf((float)dh); P.rope_freqs = m->rope_freqs;
             P.tok = c->d_tok; P.pos = c->d_pos;
-            P.score_stride = c->n_pages * KV_PAGE;
             P.max_split = std::max(1, std::min(32, mg.n_cta / m->n_head_kv));
             auto ll = [&](size_t n) { uint2* p = dalloc<uint2>(c.get(), n); BLK_CUDA(cudaMemset(p, 0, n * sizeof(uint2))); return p; };
             P.x2 = ll(d); P.q2 = ll(dq); P.h2 = ll(ff); P.ao2 = ll(dq);
-            P.sc2 = ll((size_t)m->n_head * P.score_stride); P.po2 = ll((size_t)P.max_split * dq); P.kvn2 = ll(2 * (size_t)dkv);
+            P.po2 = ll((size_t)P.max_split * dq); P.kvn2 = ll(2 * (size_t)dkv);
             P.st2 = ll((size_t)m->n_head * P.max_split * 2);
-            { const char* e = getenv("BLK_ATTN_LOCAL"); P.attn_local = (e && e[0] == '0') ? 0 : 1; }
 
             P.k_pools = c->d_kpools; P.v_pools = c->d_vpools; P.page_table = c->page_table; P.kv_dim = dkv;
             P.logits = c->logits; P.chunk_max = c->chunk_max; P.chunk_shift = c->chunk_shift;
@@ -1667,7 +1574,7 @@ extern "C" blk_status blk_decode_batch(blk_ctx* ws, blk_ctx* const* ctxs, const 
         const long long ldq = dq + 2 * dkv;
         const ChainPdl chain_scope(n);
         PendingReduce pend;      // split-K reduce of Wo / down folded into the RMSNorm that follows
-        const SplitKWs sk{ws->pf_splitk, ws->pf_splitk_elems, nullptr, nullptr, 0, &pend};
+        const SplitKWs sk{ws->pf_splitk, ws->pf_splitk_elems, &pend};
         // matrices with a resident bf16 panel (model cache) take the TMA-fed GEMM: the step then streams the panels at HBM speed
         // instead of waiting for the de-quantising producers of the fused form
         const std::vector<__nv_bfloat16*>& res = model_panels(ws);
@@ -2221,9 +2128,6 @@ extern "C" blk_status blk_test_prefill_attn(int32_t device, const float* q, cons
         BLK_CUDA(cudaGetLastError());
         BLK_CUDA(cudaMemcpyAsync(out, fo, (size_t)T * dq * 4, cudaMemcpyDeviceToHost, c.stream));
         BLK_CUDA(cudaStreamSynchronize(c.stream));
-        if (used_tc) {
-            static const bool no_tc = [] { const char* e = getenv("BLK_ATTN_TC"); return e && e[0] == '0'; }();
-            *used_tc = (tc && !no_tc) ? 1 : 0;
-        }
+        if (used_tc) *used_tc = tc ? 1 : 0;
     });
 }

@@ -91,10 +91,7 @@ struct blk_ctx {
     int n_pages = 0, n_split = 1;
     int verify_mode = 0;
     cudaStream_t stream = nullptr;
-    cudaStream_t pf_stream = nullptr;      // L2 weight prefetch, one phase ahead of the mat-vecs
-    cudaEvent_t pf_fork = nullptr, pf_join = nullptr;
-    bool use_prefetch = true, pf_used = false;
-    int pf_mask = 31, pf_threads = 256, pf_ctas = 148;
+    cudaStream_t pf_stream = nullptr;      // side stream of the prefill panel fills (one GEMM ahead of the main stream) and the model panel cache
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     std::vector<void*> allocs;
     std::vector<void*> host_allocs;
@@ -143,7 +140,6 @@ struct blk_ctx {
     float* pf_logits = nullptr;
     __half* pf_vt = nullptr; int pf_vt_pad = 0;           // transposed V of one layer for the tcgen05 prefill attention
     float* pf_splitk = nullptr; size_t pf_splitk_elems = 0;               // partial sums of the split-K prefill GEMMs (few-token batches)
-    int* pf_sched = nullptr; static constexpr int PF_SCHED_CAP = 1024;    // work-distribution counters of the prefill GEMMs (one per launch of a pass, zeroed at its start)
     __nv_bfloat16* pf_panel[4] = {nullptr, nullptr, nullptr, nullptr};     // bf16 weight panels of the two-pass GEMM form, one per GEMM kind
     cudaEvent_t pn_filled[4] = {nullptr, nullptr, nullptr, nullptr}, pn_start[4] = {nullptr, nullptr, nullptr, nullptr};
     int panel_min = 257;  // matrices that are NOT resident (model panel cache): streamed two-pass GEMM form from this many tokens per chunk on

@@ -461,13 +461,11 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
 // prologue (barrier initialisation, TMEM allocation) hide under the tail of the current one.  Measured on the 8B model: a 32-token
 // prompt 4.71 -> 4.01 ms, 512 tokens 8.84 -> 8.36, a 32-row batched decode step 5.14 -> 4.67 ms; at 2048 tokens nothing (28.3-29.5 ms
 // either way, if anything slower), so a pass switches it on only up to CHAIN_PDL_MAX_TOKENS (ChainPdl scope, per host thread).
-// BLK_PREFILL_PDL=0: plain launches everywhere (the two instructions are then no-ops); =1: at every size.
 constexpr int CHAIN_PDL_MAX_TOKENS = 1024;
-inline int chain_pdl_env() { static const int v = [] { const char* e = getenv("BLK_PREFILL_PDL"); return e ? (e[0] == '0' ? 0 : 2) : 1; }(); return v; }
 inline bool& chain_pdl_flag() { static thread_local bool on = false; return on; }
 struct ChainPdl {      // RAII: the launches of this host thread inside the scope are programmatic dependents of their predecessors
     bool prev;
-    explicit ChainPdl(int n_tokens) : prev(chain_pdl_flag()) { const int e = chain_pdl_env(); chain_pdl_flag() = e == 2 || (e == 1 && n_tokens <= CHAIN_PDL_MAX_TOKENS); }
+    explicit ChainPdl(int n_tokens) : prev(chain_pdl_flag()) { chain_pdl_flag() = n_tokens <= CHAIN_PDL_MAX_TOKENS; }
     ~ChainPdl() { chain_pdl_flag() = prev; }
 };
 template <class... KArgs, class... Args>

@@ -11,7 +11,6 @@ size_t mega_smem_bytes(const MegaParams& P) {
     b += (size_t)P.max_items * MG_WARPS * sizeof(float2);
     b += (size_t)(P.d_head / 2) * sizeof(float2);
     b += 8 * MG_WARPS * sizeof(double);
-    b += 8 * MG_WARPS * sizeof(float);
     b += 32 * sizeof(float);
     b += 32 * sizeof(int);
     b += (size_t)P.act_bytes;

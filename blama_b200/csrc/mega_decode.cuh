@@ -315,7 +315,7 @@ __global__ void mg_chunk_list_kernel(const MegaPhase* phases, int n_phases, int 
 
 // ---- shared memory carve-up ------------------------------------------------------------------------------------------
 struct MgSmem {
-    uint64_t* bars; MegaPhase* ph; __half** kp; __half** vp; float2* part; float2* rope; double* redd; float* redf; float* stat; int* misc;
+    uint64_t* bars; MegaPhase* ph; __half** kp; __half** vp; float2* part; float2* rope; double* redd; float* stat; int* misc;
     unsigned char* act;        // quantised activations of the running phase
     unsigned char* attn;       // attention tiles (behind the activations of an n_embd-long row, so they can be filled early)
 };
@@ -329,7 +329,6 @@ __device__ __forceinline__ MgSmem mg_carve(const MegaParams& P, unsigned char* s
     s.part = reinterpret_cast<float2*>(sp); sp += (size_t)P.max_items * MG_WARPS * sizeof(float2);
     s.rope = reinterpret_cast<float2*>(sp); sp += (size_t)(P.d_head / 2) * sizeof(float2);
     s.redd = reinterpret_cast<double*>(sp); sp += 8 * MG_WARPS * sizeof(double);
-    s.redf = reinterpret_cast<float*>(sp); sp += 8 * MG_WARPS * sizeof(float);
     s.stat = reinterpret_cast<float*>(sp); sp += 32 * sizeof(float);
     s.misc = reinterpret_cast<int*>(sp); sp += 32 * sizeof(int);
     s.act = sp;
@@ -390,13 +389,11 @@ __device__ __forceinline__ MgAttn mg_attn_get(const MgSmem& S) {   // computed o
     MgAttn a; a.hk = S.misc[1]; a.split = S.misc[2]; a.n_split = S.misc[3]; a.t0 = S.misc[4]; a.nt = S.misc[5]; a.on = S.misc[6] != 0; return a;
 }
 __device__ __forceinline__ void mg_attn_setup(const MegaParams& P, int n_kv, const MgSmem& S) {
-    const int n_split = max(1, min(P.max_split, (n_kv + P.ts_target - 1) / P.ts_target));
+    const int n_split = max(1, min(P.max_split, (n_kv + P.ts_cap - 1) / P.ts_cap));
     const int hk = (int)blockIdx.x % P.n_head_kv, split = (int)blockIdx.x / P.n_head_kv;
     const int per = (n_kv + n_split - 1) / n_split;
     const int t0 = split * per;
     S.misc[1] = hk; S.misc[2] = split; S.misc[3] = n_split; S.misc[4] = t0; S.misc[5] = max(0, min(n_kv, t0 + per) - t0); S.misc[6] = split < n_split ? 1 : 0;
-    // the soft-max runs on the CTA's OWN scores (local maximum and sum, merged by the CTAs of the head): the scores never leave the CTA
-    S.misc[8] = P.attn_local ? 1 : 0;      // (a slice longer than one tile is walked tile by tile with a running maximum, mg_attn_pv_local)
 }
 __device__ __forceinline__ size_t mg_kv_row(const MegaParams& P, int hk, int t) {
     return ((size_t)P.page_table[t / KV_PAGE] * KV_PAGE + (t % KV_PAGE)) * P.kv_dim + (size_t)hk * P.d_head;
@@ -412,8 +409,7 @@ __device__ __forceinline__ MgAttnSmem mg_attn_carve(const MegaParams& P, unsigne
     s.red = reinterpret_cast<float*>(s.k);          // [token group][gq][dh] partial outputs, once the tiles are dead
     return s;
 }
-// rows [tile0, tile0 + cn) of the slice, restricted to tokens < t_limit -> shared memory
-template <bool ASYNC>
+// rows [tile0, tile0 + cn) of the slice, restricted to tokens < t_limit -> shared memory (cp.async)
 __device__ __forceinline__ void mg_attn_load_rows(const MegaParams& P, const MgAttn& a, const __half* pool, __half* dst, int tile0, int cn, int t_limit) {
     const int dh = P.d_head, csh = dh == 128 ? 4 : 3;               // 16-byte chunks per row: dh / 8
     for (int idx = threadIdx.x; idx < (cn << csh); idx += MG_THREADS) {
@@ -421,8 +417,7 @@ __device__ __forceinline__ void mg_attn_load_rows(const MegaParams& P, const MgA
         const int t = a.t0 + tile0 + tl;
         if (t >= t_limit) continue;
         const __half* src = pool + mg_kv_row(P, a.hk, t) + c * 8;
-        if (ASYNC) cp_async16(dst + (size_t)tl * dh + c * 8, src);
-        else *reinterpret_cast<uint4*>(dst + (size_t)tl * dh + c * 8) = __ldcg(reinterpret_cast<const uint4*>(src));
+        cp_async16(dst + (size_t)tl * dh + c * 8, src);
     }
 }
 
@@ -432,16 +427,14 @@ __device__ __noinline__ void mg_attn_prefetch(const MegaParams& P, int layer, in
     if (!a.on || a.nt == 0) return;
     const MgAttnSmem s = mg_attn_carve(P, S.attn);
     const int cn = min(a.nt, P.ts_cap);
-    mg_attn_load_rows<true>(P, a, S.kp[layer], s.k, 0, cn, n_kv - 1);
-    mg_attn_load_rows<true>(P, a, S.vp[layer], s.v, 0, cn, n_kv - 1);
+    mg_attn_load_rows(P, a, S.kp[layer], s.k, 0, cn, n_kv - 1);
+    mg_attn_load_rows(P, a, S.vp[layer], s.v, 0, cn, n_kv - 1);
     cp_async_commit();
 }
 
-// scaled scores of ONE tile (rows [0, cn) of s.k = tokens a.t0 + c0 ..) against the gq query heads in s.q: 8 lanes per token,
-// dh / 8 dims each.  keep: into s.sc (the CTA's own soft-max); publish: as LL words (legacy form, statistics over the whole row)
+// scaled scores of ONE tile (rows [0, cn) of s.k) against the gq query heads in s.q -> s.sc: 8 lanes per token, dh / 8 dims each
 template <int GQ>
-__device__ __forceinline__ void mg_scores_tile(const MegaParams& P, const MgAttn& a, const MgAttnSmem& s, int c0, int cn, int gq, int dh,
-                                               bool publish, uint32_t tag_out, bool keep) {
+__device__ __forceinline__ void mg_scores_tile(const MegaParams& P, const MgAttnSmem& s, int cn, int gq, int dh) {
     const int tid = threadIdx.x;
     const int ld = tid & 7, tl = tid >> 3;
     const int DL = dh >> 3;
@@ -471,21 +464,19 @@ __device__ __forceinline__ void mg_scores_tile(const MegaParams& P, const MgAttn
         v += __shfl_xor_sync(0xffffffffu, v, 2);
         v += __shfl_xor_sync(0xffffffffu, v, 4);
         v = __fmul_rn(v, P.attn_scale);
-        if (tl < cn && ld == 0) {
-            if (publish) ll_st(P.sc2 + (size_t)(a.hk * gq + gI) * P.score_stride + a.t0 + c0 + tl, v, tag_out);
-            if (keep) s.sc[gI * P.ts_cap + tl] = v;
-        }
+        if (tl < cn && ld == 0) s.sc[gI * P.ts_cap + tl] = v;
     }
 }
 
-// stage 1: scaled scores of this CTA's token slice for the gq query heads of its KV head -> LL words (+ shared for tile 0)
+// stage 1: scaled scores of the first tile of this CTA's token slice for the gq query heads of its KV head -> shared memory
+// (stage 2 scores the later tiles)
 template <int GQ>
-__device__ __noinline__ void mg_attn_scores(const MegaParams& P, int layer, int phi, int n_kv, const MgSmem& S) {
+__device__ __noinline__ void mg_attn_scores(const MegaParams& P, int phi, int n_kv, const MgSmem& S) {
     const MgAttn a = mg_attn_get(S);
     if (!a.on || a.nt == 0) return;
     const MgAttnSmem s = mg_attn_carve(P, S.attn);
     const int tid = threadIdx.x, dh = P.d_head, gq = P.n_head / P.n_head_kv;
-    const uint32_t tag_in = mg_tag(P.seq, phi, 0), tag_out = mg_tag(P.seq, phi, 1);
+    const uint32_t tag_in = mg_tag(P.seq, phi, 0);
     // poll: the query heads, and (slice holding the new token only) the K / V rows this layer's QKV phase produced
     const int cn0 = min(P.ts_cap, a.nt);
     const int tl_new = n_kv - 1 - a.t0;                             // local index of the token being decoded
@@ -515,20 +506,11 @@ __device__ __noinline__ void mg_attn_scores(const MegaParams& P, int layer, int 
         }
     }
     cp_async_wait_all();
-    for (int c0 = 0; c0 < a.nt; c0 += P.ts_cap) {
-        const int cn = min(P.ts_cap, a.nt - c0);
-        if (c0 > 0) {       // legacy form, long context: further tiles are fetched synchronously (the local form walks them in stage 2)
-            if (S.misc[8]) break;
-            __syncthreads();
-            mg_attn_load_rows<false>(P, a, S.kp[layer], s.k, c0, cn, n_kv - 1);
-            if (tl_new >= c0 && tl_new < c0 + cn) for (int j = tid; j < dh; j += MG_THREADS) s.k[(size_t)(tl_new - c0) * dh + j] = __float2half_rn(__uint_as_float(ll_ld(P.kvn2 + a.hk * dh + j).x));
-        }
-        __syncthreads();
-        mg_scores_tile<GQ>(P, a, s, c0, cn, gq, dh, !S.misc[8], tag_out, c0 == 0);
-    }
+    __syncthreads();
+    mg_scores_tile<GQ>(P, s, cn0, gq, dh);
 }
 
-// stage 2, local form: soft-max over the CTA's OWN scores.
+// stage 2: soft-max over the CTA's OWN scores (local maximum and sum, merged by the CTAs of the head): the scores never leave the CTA.
 //   one slice (n_split == 1): that is the whole row -- ggml's order exactly (max -> expf -> sum in double -> p * (1/sum) -> f16 -> V.p),
 //     the result goes straight to the attention output;
 //   several slices: flash-style -- p = f16(expf(s - m_local)), o = sum p v, and (m_local, l_local) travel with the partial; the CTAs
@@ -538,10 +520,9 @@ __device__ __noinline__ void mg_attn_scores(const MegaParams& P, int layer, int 
 //     statistics pass over the whole row.
 //   a slice longer than one shared-memory tile (contexts beyond max_split x ts_cap = 1152 tokens on the 8B model) is walked tile by
 //     tile with a running maximum: the later tiles' K / V rows are fetched synchronously, their scores computed here, and the
-//     accumulator rescaled by expf(m_old - m_new) -- the same flash order, now inside the CTA too.  (Before, such contexts fell back to
-//     the round-1 form with every score exchanged between the CTAs: 496 tok/s at 1024 tokens of context, 440 at 1152, 404 at 2048.)
+//     accumulator rescaled by expf(m_old - m_new) -- the same flash order, now inside the CTA too.
 template <int GQ, bool TR>
-__device__ __noinline__ void mg_attn_pv_local(const MegaParams& P, int layer, int phi, int n_kv, const MgSmem& S) {
+__device__ __noinline__ void mg_attn_pv(const MegaParams& P, int layer, int phi, int n_kv, const MgSmem& S) {
     const MgAttn a = mg_attn_get(S);
     if (!a.on) return;
     const MgAttnSmem s = mg_attn_carve(P, S.attn);
@@ -559,7 +540,7 @@ __device__ __noinline__ void mg_attn_pv_local(const MegaParams& P, int layer, in
     if (a.nt > 0) {
         // later tiles travel behind the computation: K of tile c + 1 is requested when the scores of tile c are done (the K rows are
         // dead), V of tile c + 1 when P.V of tile c is (cp.async groups in that order)
-        if (multi) { mg_attn_load_rows<true>(P, a, S.kp[layer], s.k, P.ts_cap, min(P.ts_cap, a.nt - P.ts_cap), n_kv - 1); cp_async_commit(); }
+        if (multi) { mg_attn_load_rows(P, a, S.kp[layer], s.k, P.ts_cap, min(P.ts_cap, a.nt - P.ts_cap), n_kv - 1); cp_async_commit(); }
         for (int c0 = 0; c0 < a.nt; c0 += P.ts_cap) {
             const int cn = min(P.ts_cap, a.nt - c0);
             const bool more = c0 + P.ts_cap < a.nt;
@@ -567,7 +548,7 @@ __device__ __noinline__ void mg_attn_pv_local(const MegaParams& P, int layer, in
             const bool new_here = c0 > 0 && tl_new >= 0 && tl_new < cn;
             if (c0 > 0) {
                 __syncthreads();                           // P.V of the previous tile has read its V rows and probabilities
-                mg_attn_load_rows<true>(P, a, S.vp[layer], s.v, c0, cn, n_kv - 1);
+                mg_attn_load_rows(P, a, S.vp[layer], s.v, c0, cn, n_kv - 1);
                 cp_async_commit();
                 cp_async_wait_group<1>();                  // this tile's K rows have landed (its V rows may still fly)
                 if (new_here && tid < dh) {
@@ -578,9 +559,9 @@ __device__ __noinline__ void mg_attn_pv_local(const MegaParams& P, int layer, in
                     s.k[(size_t)tl_new * dh + tid] = __float2half_rn(__uint_as_float(w.x));
                 }
                 __syncthreads();
-                mg_scores_tile<GQ>(P, a, s, c0, cn, gq, dh, false, 0u, true);
+                mg_scores_tile<GQ>(P, s, cn, gq, dh);
                 __syncthreads();
-                if (more) { mg_attn_load_rows<true>(P, a, S.kp[layer], s.k, c0 + P.ts_cap, min(P.ts_cap, a.nt - c0 - P.ts_cap), n_kv - 1); cp_async_commit(); }
+                if (more) { mg_attn_load_rows(P, a, S.kp[layer], s.k, c0 + P.ts_cap, min(P.ts_cap, a.nt - c0 - P.ts_cap), n_kv - 1); cp_async_commit(); }
             }
             if (warp < gq) {                               // warp g: statistics and probabilities of query head g
                 float* row = s.sc + warp * P.ts_cap;
@@ -695,131 +676,6 @@ __device__ __noinline__ void mg_attn_pv_local(const MegaParams& P, int layer, in
         float o = 0.0f;
         for (int s0 = 0; s0 < ns; s0++) o += wgt[g * 32 + s0] * wp[tid * ns + s0];
         ll_st(P.ao2 + (size_t)a.hk * E + e, o * S.stat[g], tag_ao);
-    }
-}
-
-// stage 2: soft-max statistics over the whole context (redundantly per CTA), probabilities of the own slice rounded to f16,
-// partial V.p -> LL words; the CTA of split 0 sums the split partials in split order.
-template <int GQ, bool TR>
-__device__ __noinline__ void mg_attn_pv(const MegaParams& P, int layer, int phi, int n_kv, const MgSmem& S) {
-    if (S.misc[8]) { mg_attn_pv_local<GQ, TR>(P, layer, phi, n_kv, S); return; }      // soft-max on the CTA's own scores
-    const MgAttn a = mg_attn_get(S);
-    if (!a.on) return;
-    const MgAttnSmem s = mg_attn_carve(P, S.attn);
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, dh = P.d_head, gq = P.n_head / P.n_head_kv;
-    const uint32_t tag_sc = mg_tag(P.seq, phi, 1), tag_po = mg_tag(P.seq, phi, 2), tag_ao = mg_tag(P.seq, phi, 3);
-    const int TG = MG_THREADS / dh;                                          // token groups
-    const int d = tid & (dh - 1), tg = dh == 128 ? tid >> 7 : tid >> 6;
-    float acc[GQ];
-#pragma unroll
-    for (int gI = 0; gI < GQ; gI++) acc[gI] = 0.0f;
-    if (a.nt > 0) {
-        // -- row max, then row sum of expf(s - max) in double, over the WHOLE context: warps (g*ng .. g*ng+ng-1) serve head g.
-        //    Up to 8 scores per lane are polled as ONE batch and kept in registers for both passes. --
-        const int ng = S.misc[7];                                            // MG_WARPS / gq
-        const int wq = S.misc[9 + 0] ? warp >> S.misc[9 + 1] : warp / ng;    // power-of-two ng: shift
-        const int g_w = min(wq, gq - 1), part = warp - wq * ng;
-        const bool w_on = wq < gq;
-        const uint2* sr = P.sc2 + (size_t)(a.hk * gq + g_w) * P.score_stride;
-        const int stride = ng * 32;
-        float M = -INFINITY;
-        float sv[8];
-        for (int b0 = 0; b0 < n_kv; b0 += 8 * stride) {
-            int spins = 0;
-            bool ok;
-            do {
-                ok = true;
-#pragma unroll
-                for (int i = 0; i < 8; i++) {
-                    const int t = b0 + i * stride + part * 32 + lane;
-                    if (w_on && t < n_kv) { const uint2 w = ll_ld(sr + t); sv[i] = __uint_as_float(w.x); ok = ok && w.y == tag_sc; } else sv[i] = -INFINITY;
-                }
-                if (mg_spin_out(S, spins)) { mg_poll_timeout(P, S, 2); break; }
-            } while (!__all_sync(0xffffffffu, ok));
-#pragma unroll
-            for (int i = 0; i < 8; i++) M = fmaxf(M, sv[i]);
-        }
-        M = warp_max(M);
-        if (lane == 0) S.redf[warp] = M;
-        __syncthreads();
-        M = -INFINITY;
-        for (int w = 0; w < ng; w++) M = fmaxf(M, S.redf[g_w * ng + w]);
-        double sum = 0.0;
-        for (int b0 = 0; b0 < n_kv; b0 += 8 * stride) {
-            if (n_kv > 8 * stride) {          // long context: the first pass could not keep the row in registers (all tags seen valid)
-#pragma unroll
-                for (int i = 0; i < 8; i++) { const int t = b0 + i * stride + part * 32 + lane; sv[i] = (w_on && t < n_kv) ? __uint_as_float(ll_ld(sr + t).x) : -INFINITY; }
-            }
-            float e[8];
-#pragma unroll
-            for (int i = 0; i < 8; i++) e[i] = expf(sv[i] - M);             // expf(-inf) = 0 for the padding
-            // ggml sums the row in double; any order gives the same double to ~1e-16, i.e. the same float reciprocal
-            sum += ((double)e[0] + (double)e[1]) + ((double)e[2] + (double)e[3]) + (((double)e[4] + (double)e[5]) + ((double)e[6] + (double)e[7]));
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
-        if (lane == 0) S.redd[warp] = sum;
-        __syncthreads();
-        double tot = 0.0;
-        for (int w = 0; w < ng; w++) tot += S.redd[g_w * ng + w];
-        const float inv = (float)(1.0 / tot);
-        mg_tr<TR>(P, S, 13);
-        for (int c0 = 0; c0 < a.nt; c0 += P.ts_cap) {
-            const int cn = min(P.ts_cap, a.nt - c0);
-            if (c0 > 0) {
-                __syncthreads();
-                mg_attn_load_rows<false>(P, a, S.vp[layer], s.v, c0, cn, n_kv - 1);
-                const int tn = n_kv - 1 - a.t0;
-                if (tn >= c0 && tn < c0 + cn) for (int j = tid; j < dh; j += MG_THREADS) s.v[(size_t)(tn - c0) * dh + j] = __float2half_rn(__uint_as_float(ll_ld(P.kvn2 + P.kv_dim + a.hk * dh + j).x));
-            }
-            // probabilities of this tile: the warps of head g handle head g (they hold its max and 1/sum)
-            if (w_on) for (int tl = part * 32 + lane; tl < cn; tl += stride) {
-                const float scv = (c0 == 0) ? s.sc[g_w * P.ts_cap + tl] : __uint_as_float(ll_ld(sr + a.t0 + c0 + tl).x);
-                s.sc[g_w * P.ts_cap + tl] = __half2float(__float2half_rn(__fmul_rn(expf(scv - M), inv)));
-            }
-            __syncthreads();
-            for (int tl = tg; tl < cn; tl += TG) {
-                const float v = __half2float(s.v[(size_t)tl * dh + d]);
-#pragma unroll
-                for (int gI = 0; gI < GQ; gI++) if (gI < gq) acc[gI] += s.sc[gI * P.ts_cap + tl] * v;
-            }
-        }
-    }
-    // token groups meet in shared memory (the tiles are dead), summed in fixed order
-    __syncthreads();
-    mg_tr<TR>(P, S, 14);
-#pragma unroll
-    for (int gI = 0; gI < GQ; gI++) if (gI < gq) s.red[(tg * gq + gI) * dh + d] = acc[gI];
-    __syncthreads();
-    const int E = gq * dh, NO = P.n_head * dh;
-    for (int e = tid; e < E; e += MG_THREADS) {
-        float o = 0.0f;
-        for (int k = 0; k < TG; k++) o += s.red[k * E + e];
-        ll_st(P.po2 + (size_t)a.split * NO + a.hk * E + e, o, tag_po);
-    }
-    mg_tr<TR>(P, S, 15);
-    // the CTA of split 0 sums the split partials of its KV head in split order
-    if (a.split == 0) {
-        for (int e = tid; e < E; e += MG_THREADS) {
-            const uint2* pp = P.po2 + a.hk * E + e;
-            float o = 0.0f;
-            for (int s0 = 0; s0 < a.n_split; s0 += 8) {        // batches of 8 polled together, added in split order
-                float pv[8];
-                int spins = 0;
-                bool ok;
-                do {
-                    ok = true;
-#pragma unroll
-                    for (int i = 0; i < 8; i++) {
-                        if (s0 + i < a.n_split) { const uint2 w = ll_ld(pp + (size_t)(s0 + i) * NO); pv[i] = __uint_as_float(w.x); ok = ok && w.y == tag_po; } else pv[i] = 0.0f;
-                    }
-                    if (mg_spin_out(S, spins)) { mg_poll_timeout(P, S, 3); break; }
-                } while (!ok);
-#pragma unroll
-                for (int i = 0; i < 8; i++) o += pv[i];
-            }
-            ll_st(P.ao2 + (size_t)a.hk * E + e, o, tag_ao);
-        }
     }
 }
 
@@ -1007,9 +863,6 @@ __global__ void __launch_bounds__(MG_THREADS, 1) mega_decode_kernel(const __grid
     if (tid == 0) {
         S.misc[0] = P.page_table[pos / KV_PAGE]; S.misc[16] = 0; S.misc[20] = 0;
         mg_attn_setup(P, n_kv, S);
-        const int gq = P.n_head / P.n_head_kv, ng = MG_WARPS / gq;
-        int sh = 0; while ((1 << sh) < ng) sh++;
-        S.misc[7] = ng; S.misc[9] = (1 << sh) == ng ? 1 : 0; S.misc[10] = sh;
     }
     __syncthreads();
 
@@ -1164,7 +1017,7 @@ __global__ void __launch_bounds__(MG_THREADS, 1) mega_decode_kernel(const __grid
         mg_epilogue(P, ph, phi, pos, S, res, have_res);
         mg_tr<TR>(P, S, trk | 6);
         if (is_qkv) {
-            mg_attn_scores<GQ>(P, layer, phi, n_kv, S);
+            mg_attn_scores<GQ>(P, phi, n_kv, S);
             mg_tr<TR>(P, S, 11);
             mg_attn_pv<GQ, TR>(P, layer, phi, n_kv, S);
             mg_tr<TR>(P, S, 16);

@@ -69,8 +69,7 @@ struct MegaParams {
     const uint4* chunk_list; const int* chunk_counts; int list_stride;     // per (cta, warp): chunk descriptors {addr.lo, addr.hi, bytes, 0}
     int n_cta; int slot_bytes; int max_items; int act_bytes;
     int attn_off;            // offset of the attention tiles inside the activation scratch (behind an n_embd-long row's activations)
-    int ts_target;           // tokens per context split the attention aims for (<= ts_cap: more, shorter splits)
-    int ts_cap;              // tokens of one attention tile (K and V rows of a CTA's context slice held in shared memory)
+    int ts_cap;              // tokens of one attention tile (K and V rows of a CTA's context slice held in shared memory) = tokens per context split
     // model
     QMat tok_embd;
     int n_embd, n_head, n_head_kv, d_head, n_ff, n_vocab, neox;
@@ -79,11 +78,10 @@ struct MegaParams {
     // context
     const int32_t* tok; int32_t* pos;
     // cross-CTA vectors as LL words {value bits, epoch tag} (mega_decode.cuh): residual stream, q, SwiGLU output, attention output,
-    // scores [n_head][score_stride], split partials [max_split][n_head * d_head], the new token's K | V rows [2][kv_dim]
-    uint2* x2; uint2* q2; uint2* h2; uint2* ao2; uint2* sc2; uint2* po2; uint2* kvn2;
-    uint2* st2;              // soft-max statistics of the split partials [n_head][max_split] x {local max, local sum} (local attention form)
-    int score_stride; int max_split;
-    int attn_local;          // 1: slices that fit one tile run the soft-max on their own scores (BLK_ATTN_LOCAL=0 switches back)
+    // split partials [max_split][n_head * d_head], the new token's K | V rows [2][kv_dim]
+    uint2* x2; uint2* q2; uint2* h2; uint2* ao2; uint2* po2; uint2* kvn2;
+    uint2* st2;              // soft-max statistics of the split partials [n_head][max_split] x {local max, local sum}
+    int max_split;
     uint32_t seq;            // launch counter of the context (epoch base of every tag)
     int* err;                // mapped host word: set when a poll timed out
     __half* const* k_pools; __half* const* v_pools; const int32_t* page_table; int kv_dim;

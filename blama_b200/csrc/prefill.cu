@@ -1,6 +1,5 @@
 // prefill.cu -- launchers of the multi-token prefill path (tcgen05 GEMM + helpers).
 #include "prefill.hpp"
-#include <cstdlib>
 #include "prefill_gemm.cuh"
 #include "prefill_attn_tc.cuh"
 
@@ -88,8 +87,6 @@ cudaError_t launch_gemm(PrefillGemmArgs& a, int ta, int tb, const __nv_bfloat16*
     // the SMs; partial sums go to the workspace and are added in split order by a second kernel (deterministic).  Every split gets
     // at least 8 K blocks (hence never an empty one); a wave that is at least half full is left alone.
     a.k_splits = 1; a.n_whole = tiles; a.ws = nullptr;
-    a.sched = nullptr;
-    if (sk && sk->sched && sk->sched_next && *sk->sched_next < sk->sched_cap && tiles > sms) a.sched = sk->sched + (*sk->sched_next)++;      // more items than CTAs: dynamic
     if (sk && sk->ws && sms > 0) {
         const int n_whole = (tiles / sms) * sms, rem = tiles - n_whole;
         if (rem > 0 && 2 * rem <= sms && n_whole <= 2 * sms) {      // (after many whole waves the partial one is a small share: not worth a second kernel)
@@ -119,10 +116,6 @@ cudaError_t launch_gemm(PrefillGemmArgs& a, int ta, int tb, const __nv_bfloat16*
 
 // first pass of the two-pass form: W -> panel rows [row0, row0 + W.N)
 cudaError_t panel_dequant(const QMat& W, __nv_bfloat16* panel, long long row0, cudaStream_t st) {
-    // BLK_PANEL_NOFILL=1 (measurement only, results are garbage): skip the de-quantisation pass so that the GEMMs read whatever the
-    // panel holds -- the difference in wall time is what the panel fills (their HBM traffic and power) cost a verify
-    static const bool nofill = [] { const char* e = getenv("BLK_PANEL_NOFILL"); return e && e[0] == '1'; }();
-    if (nofill) return cudaSuccess;
     if (row0 % 128) return cudaErrorInvalidValue;
     const long long total = (long long)((W.N + 127) / 128) * 128 * (W.K >> 6);
     const unsigned grid = (unsigned)((total + 255) / 256);

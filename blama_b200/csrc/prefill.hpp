@@ -14,12 +14,10 @@ namespace blk {
 // tiles from there by TMA -- for many-token batches, where the fused form would dequantise every weight tile T / 256 times.
 // sk != nullptr: workspace for the deterministic split-K of the last, partial wave of tiles (all tiles when the batch has fewer
 // tiles than SMs); n_sm * 65536 floats always suffice (split tiles * splits never exceeds the SM count)
-// split-K workspace + the pool of zeroed work-distribution counters of a prefill pass (one per GEMM launch: sched_next counts them on the
-// host; exhausted or absent -> that launch uses the static schedule)
 // a split-K ACCUMULATE (C += X W^T over the residual stream, every tile split) whose partial sums are still in the workspace: the RMSNorm
 // that follows adds them while it reads the row anyway (rmsnorm_bf16_launch), instead of a reduce kernel of its own
 struct PendingReduce { const float* ws = nullptr; int S = 0, m_tiles = 0; };
-struct SplitKWs { float* ws; size_t elems; int* sched = nullptr; int* sched_next = nullptr; int sched_cap = 0; PendingReduce* defer = nullptr; };
+struct SplitKWs { float* ws; size_t elems; PendingReduce* defer = nullptr; };
 cudaError_t prefill_gemm(const QMat& W, const __nv_bfloat16* X, int T, float* C, long long ldc, const float* bias, int mode, cudaStream_t st,
                          __nv_bfloat16* panel = nullptr, bool panel_fill = true, const SplitKWs* sk = nullptr);
 // rows a matrix of N rows occupies in a panel (tile aligned)

@@ -63,9 +63,6 @@ struct PrefillGemmArgs {
     // applies the epilogue (bias / accumulate / SwiGLU).  k_splits == 1: off.
     int n_whole, k_splits;
     float* ws;
-    // dynamic work distribution: a zeroed device counter; CTAs take work items in increasing order with atomicAdd instead of the static
-    // stride (item = blockIdx.x + i gridDim.x).  nullptr: static.  Which CTA computes an item does not change a bit of the result.
-    int* sched;
 };
 
 // ---- PTX wrappers ---------------------------------------------------------------------------------------------------
@@ -355,10 +352,7 @@ __global__ void __launch_bounds__(PG_THREADS, 1) prefill_gemm_kernel(const __gri
     uint64_t* empty = bars + PG_STAGES_FEW;         // [n_st]  tcgen05.commit
     uint64_t* tmem_full = bars + 2 * PG_STAGES_FEW;     // accumulators complete
     uint64_t* tmem_empty = bars + 2 * PG_STAGES_FEW + 1;    // epilogue drained them (8 warps)
-    uint64_t* sch_full = bars + 2 * PG_STAGES_FEW + 2;      // [2] the TMA thread has published the next work item
-    uint64_t* sch_empty = bars + 2 * PG_STAGES_FEW + 4;     // [2] the MMA thread and the 8 producer / epilogue warps have read it
-    uint32_t* tmem_base_slot = reinterpret_cast<uint32_t*>(bars + 2 * PG_STAGES_FEW + 6);
-    int* sch_item = reinterpret_cast<int*>(tmem_base_slot + 2);     // [2]
+    uint32_t* tmem_base_slot = reinterpret_cast<uint32_t*>(bars + 2 * PG_STAGES_FEW + 2);
     // stage geometry: kernel-uniform (few = every tile has one M half only)
     const bool few = a.T <= 128;
     const int n_st = few ? PG_STAGES_FEW : PG_STAGES;
@@ -370,7 +364,6 @@ __global__ void __launch_bounds__(PG_THREADS, 1) prefill_gemm_kernel(const __gri
         for (int s = 0; s < PG_STAGES_FEW; s++) { mbar_init(full + s, PANEL ? 1 : 1 + PG_PRODUCER_THREADS / 32); mbar_init(empty + s, 1); }
         mbar_init(tmem_full, 1);
         mbar_init(tmem_empty, 8);
-        for (int i = 0; i < 2; i++) { mbar_init(sch_full + i, 1); mbar_init(sch_empty + i, 9); }
         mbar_fence_init();
     }
     if (warp == 9) {    // one warp allocates all 512 TMEM columns (two 128 x 256 f32 accumulators)
@@ -395,15 +388,8 @@ __global__ void __launch_bounds__(PG_THREADS, 1) prefill_gemm_kernel(const __gri
         if (lane == 0) {
             int s = 0; uint32_t ph = 0;                        // stage and its phase
             for (int wi = 0;; wi++) {
-                int item;
-                if (a.sched) {      // take the next item and hand it to the other roles through a two-slot queue
-                    mbar_wait(sch_empty + (wi & 1), ((wi >> 1) & 1) ^ 1);
-                    item = atomicAdd(a.sched, 1);
-                    if (item >= total_tiles) item = -1;
-                    sch_item[wi & 1] = item;
-                    mbar_arrive(sch_full + (wi & 1));
-                } else { item = (int)blockIdx.x + wi * (int)gridDim.x; if (item >= total_tiles) item = -1; }
-                if (item < 0) break;
+                const int item = (int)blockIdx.x + wi * (int)gridDim.x;
+                if (item >= total_tiles) break;
                 const PgItem w = pg_item(item, n_whole, n_split, k_per, k_blocks_all);
                 const int tile = w.tile, kb0 = w.kb0, kb1 = w.kb1;
                 const int m0 = (tile % m_tiles) * PG_BM, nt = tile / m_tiles;
@@ -431,13 +417,8 @@ __global__ void __launch_bounds__(PG_THREADS, 1) prefill_gemm_kernel(const __gri
             constexpr uint32_t idesc = umma_idesc_bf16(128, PG_BN);
             int s = 0; uint32_t ph = 0;
             for (int tile_i = 0;; tile_i++) {
-                int item;
-                if (a.sched) {
-                    mbar_wait(sch_full + (tile_i & 1), (tile_i >> 1) & 1);
-                    item = sch_item[tile_i & 1];
-                    mbar_arrive(sch_empty + (tile_i & 1));
-                } else { item = (int)blockIdx.x + tile_i * (int)gridDim.x; if (item >= total_tiles) item = -1; }
-                if (item < 0) break;
+                const int item = (int)blockIdx.x + tile_i * (int)gridDim.x;
+                if (item >= total_tiles) break;
                 const PgItem w = pg_item(item, n_whole, n_split, k_per, k_blocks_all);
                 const int kb0 = w.kb0, kb1 = w.kb1;
                 const bool two = (w.tile % m_tiles) * PG_BM + 128 < a.T;      // the second accumulator's token rows exist
@@ -467,14 +448,8 @@ __global__ void __launch_bounds__(PG_THREADS, 1) prefill_gemm_kernel(const __gri
         const int r = threadIdx.x;                                // B-tile row handled by this thread
         int s = 0; uint32_t ph = 0;
         for (int tile_i = 0;; tile_i++) {
-            int item;
-            if (a.sched) {
-                mbar_wait(sch_full + (tile_i & 1), (tile_i >> 1) & 1);
-                item = sch_item[tile_i & 1];
-                __syncwarp();
-                if (lane == 0) mbar_arrive(sch_empty + (tile_i & 1));
-            } else { item = (int)blockIdx.x + tile_i * (int)gridDim.x; if (item >= total_tiles) item = -1; }
-            if (item < 0) break;
+            const int item = (int)blockIdx.x + tile_i * (int)gridDim.x;
+            if (item >= total_tiles) break;
             const PgItem w = pg_item(item, n_whole, n_split, k_per, k_blocks_all);
             const int tile = w.tile, kb0 = w.kb0, kb1 = w.kb1;
             const int m0 = (tile % m_tiles) * PG_BM, nt = tile / m_tiles;

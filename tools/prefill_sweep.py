@@ -1,4 +1,4 @@
-"""Prompt prefill time vs token count: split-K off / on for the two-pass GEMM form (BLK_SPLITK), and the fused form for reference."""
+"""Prompt prefill time vs token count: the two-pass GEMM form and the fused form (BLK_PANEL_MIN)."""
 import os, sys, time
 sys.path.insert(0, '.')
 from bench import ensure_model
@@ -6,8 +6,8 @@ from blama_b200 import capi, gguf_synth
 shape = sys.argv[1] if len(sys.argv) > 1 else "llama-3.1-8b-q4km"
 path = ensure_model(shape, 0, lambda: None)
 m = capi.Model(path)
-for name, pm, sk in (("fused form        ", 1 << 30, "0"), ("fused + split-K   ", 1 << 30, "1"), ("two-pass          ", 32, "0"), ("two-pass + split-K", 32, "1")):
-    os.environ["BLK_PANEL_MIN"] = str(pm); os.environ["BLK_SPLITK"] = sk
+for name, pm in (("fused form", 1 << 30), ("two-pass  ", 32)):
+    os.environ["BLK_PANEL_MIN"] = str(pm)
     c = capi.Ctx(m, 2304)
     row = []
     for T in (32, 64, 128, 256, 384, 512, 768, 1024, 2048):

@@ -1,10 +1,8 @@
 """Wall time of a 2048-token verify request (fillCtx + LogitComparer through the host API, L2 flushed before each, median of 5) for the
-form selected by the environment: default two-pass (bf16 panels), BLK_PANEL_MIN=0 (de-quantisation fused into the GEMM),
-BLK_PANEL_NOFILL=1 (two-pass without the fill pass: what the fills cost; results are garbage)."""
+form selected by the environment: default two-pass (bf16 panels), BLK_PANEL_MIN=0 (de-quantisation fused into the GEMM)."""
 import os, statistics, sys, time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-import numpy as np
 from bench import ensure_model
 from blama_b200 import gguf_synth, host_api
 shape = sys.argv[1] if len(sys.argv) > 1 else "llama-3.1-8b-q4km"
@@ -14,11 +12,7 @@ hm = host_api.Model(path)
 inst = host_api.Instance(hm, T + 128)
 ctx = inst.raw_ctx()
 prompt = gguf_synth.synth_prompt(shape, 32, 1)
-nofill = os.environ.get("BLK_PANEL_NOFILL") == "1"
-if nofill:      # the prover run needs real weights: take synthetic claims instead
-    toks = gguf_synth.synth_prompt(shape, T, 2); top = np.zeros((T, 10), dtype=host_api.TD_DTYPE); top["token"] = np.arange(10)[None, :] + 5; top["logit"] = np.linspace(3, 1, 10)[None, :]
-else:
-    inst.start_session(seed=1).set_initial_prompt(prompt); toks, top = inst.complete(T); inst.stop_session()
+inst.start_session(seed=1).set_initial_prompt(prompt); toks, top = inst.complete(T); inst.stop_session()
 ts = []
 for r in range(6):
     ctx.flush_l2()
@@ -26,4 +20,4 @@ for r in range(6):
     t0 = time.perf_counter(); score = inst.verify(toks, top); dt = time.perf_counter() - t0
     inst.stop_session()
     if r: ts.append(dt * 1e3)
-print(f"{shape} T={T} PANEL_MIN={os.environ.get('BLK_PANEL_MIN','default')} NOFILL={int(nofill)}: median {statistics.median(ts):.2f} ms (min {min(ts):.2f}, max {max(ts):.2f}), score {score:.5f}")
+print(f"{shape} T={T} PANEL_MIN={os.environ.get('BLK_PANEL_MIN','default')}: median {statistics.median(ts):.2f} ms (min {min(ts):.2f}, max {max(ts):.2f}), score {score:.5f}")
