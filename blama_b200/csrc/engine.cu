@@ -411,7 +411,6 @@ extern "C" blk_model* blk_model_load(const char* path, int32_t device, blk_progr
         }
         m->out_norm = vec("output_norm.weight", d, true);
         if (f.find("output.weight")) m->output = mat("output.weight", d, m->n_vocab); else m->output = m->tok_embd;
-        m->act_fmt_out = act_format_for(m->output.type);
         m->rope_freqs = vec("rope_freqs.weight", m->d_head / 2, false);
         wb += (int64_t)m->output.bytes + 4 * d;
         m->weight_bytes_per_token = wb;
@@ -491,13 +490,6 @@ extern "C" int32_t blk_model_vocab_only(const blk_model* m) { return m->vocab_on
 extern "C" int32_t blk_model_add_bos(const blk_model* m) { return m->add_bos ? 1 : 0; }
 extern "C" int32_t blk_model_device(const blk_model* m) { return m->device; }
 extern "C" int64_t blk_model_weight_bytes_per_token(const blk_model* m) { return m->weight_bytes_per_token; }
-extern "C" int64_t blk_model_panel_bytes(blk_model* m, int32_t* n_resident, int32_t* n_matrices) {
-    if (!m) return 0;
-    std::lock_guard<std::mutex> lk(m->panels.mu);
-    if (n_resident) *n_resident = m->panels.n_resident;
-    if (n_matrices) *n_matrices = 4 * m->n_layer + 1;
-    return (int64_t)m->panels.bytes;
-}
 extern "C" int64_t blk_model_kv_bytes_per_token(const blk_model* m) { return (int64_t)m->n_layer * m->n_head_kv * m->d_head * 2 * 2; }
 extern "C" int32_t blk_model_token_text(const blk_model* m, int32_t tok, char* buf, int32_t cap) {
     if (tok < 0 || tok >= (int)m->vocab.size()) return 0;
@@ -611,6 +603,15 @@ void matvec(blk_ctx* c, GemvArgs& a, const float* in, const float* norm_w, const
     prof_mark(c, name);
 }
 
+// the threshold top-k of the context's own logits row (c->logits -> c->top_ids / c->top_logits)
+TopkArgs own_topk_args(const blk_ctx* c) {
+    TopkArgs tk{};
+    tk.logits = c->logits; tk.n = c->m->n_vocab; tk.chunk_max = c->chunk_max; tk.n_chunks = c->n_chunks;
+    tk.cand_l = c->cand_l; tk.cand_i = c->cand_i; tk.cap = c->cand_cap; tk.count = c->counters + 1; tk.done = c->counters + 2;
+    tk.out_ids = c->top_ids; tk.out_logits = c->top_logits;
+    return tk;
+}
+
 // one decode step on c->stream: token id in c->d_tok, position in c->d_pos.
 // Per layer: QKV mat-vec (RMSNorm prologue; +bias, RoPE, KV-page write) | attention | Wo mat-vec (+residual) |
 // gate/up mat-vec (RMSNorm prologue; SwiGLU) | down mat-vec (+residual); then final norm + lm_head mat-vec + top-k.
@@ -627,10 +628,8 @@ void enqueue_step(blk_ctx* c, bool with_head, bool feedback = false) {
         c->launches++;
         prof_mark(c, "mega_decode");
         if (with_head) {
-            TopkArgs tk{};
-            tk.logits = c->logits; tk.n = m->n_vocab; tk.chunk_max = c->chunk_max; tk.n_chunks = c->n_chunks;
-            tk.cand_l = c->cand_l; tk.cand_i = c->cand_i; tk.cap = c->cand_cap; tk.count = c->counters + 1; tk.done = c->counters + 2;
-            tk.out_ids = c->top_ids; tk.out_logits = c->top_logits; tk.feed_tok = feedback ? c->d_tok : nullptr;
+            TopkArgs tk = own_topk_args(c);
+            tk.feed_tok = feedback ? c->d_tok : nullptr;
             topk_select_kernel<<<16, 1024, 0, c->stream>>>(tk);
             BLK_CUDA(cudaGetLastError());
             c->launches++;
@@ -718,11 +717,7 @@ void enqueue_step(blk_ctx* c, bool with_head, bool feedback = false) {
         a.nseg = 1; a.seg[0] = {m->output, nullptr, 0, 0}; a.total_pairs = m->n_vocab / 2; a.out = c->logits;
         a.tail.kind = TAIL_CHUNKMAX; a.tail.chunk_max = c->chunk_max; a.tail.chunk_shift = c->chunk_shift;
         matvec<EPI_STORE>(c, a, c->x, m->out_norm, c->act_d, "gemv_lm_head");
-        TopkArgs tk{};
-        tk.logits = c->logits; tk.n = m->n_vocab; tk.chunk_max = c->chunk_max; tk.n_chunks = c->n_chunks;
-        tk.cand_l = c->cand_l; tk.cand_i = c->cand_i; tk.cap = c->cand_cap; tk.count = c->counters + 1; tk.done = c->counters + 2;
-        tk.out_ids = c->top_ids; tk.out_logits = c->top_logits;
-        BLK_CUDA(launch_pdl(topk_select_kernel, dim3(16), dim3(1024), 0, c->stream, tk));
+        BLK_CUDA(launch_pdl(topk_select_kernel, dim3(16), dim3(1024), 0, c->stream, own_topk_args(c)));
         c->launches++;
         prof_mark(c, "topk_select");
     }
@@ -845,21 +840,48 @@ namespace {
 // ------------------------------------------------------------------------------------------------------------------
 // multi-token prefill (tcgen05 GEMM path)
 // ------------------------------------------------------------------------------------------------------------------
+// The GEMMs of a multi-token pass, in pass order: op 4 l + {OP_QKV, OP_WO, OP_GATE_UP, OP_DOWN} of layer l, then the lm_head.
+// This index is shared by the model's resident panel cache, the per-context streaming panels and the pass itself.
+enum GemmKind { OP_QKV, OP_WO, OP_GATE_UP, OP_DOWN, OP_HEAD };
+struct GemmOp {
+    GemmKind kind;
+    int n_parts;
+    GemmPart part[3];                   // OP_GATE_UP: {gate, up}
+    const __nv_bfloat16* panel;         // set by GemmSchedule::next: the bf16 panel the GEMM reads (nullptr: fused form)
+    size_t panel_elems() const { return prefill_panel_elems(part, n_parts, kind == OP_GATE_UP); }
+    // false: the combination takes the fused GEMM form
+    bool fill_panel(__nv_bfloat16* p, cudaStream_t st, cudaError_t* err) const { return prefill_panel_fill(part, n_parts, kind == OP_GATE_UP, p, st, err); }
+};
+int n_gemm_ops(const blk_model* m) { return 4 * m->n_layer + 1; }
+GemmOp gemm_op(const blk_model* m, int i) {
+    const int l = i / 4;
+    if (l == m->n_layer) return {OP_HEAD, 1, {{&m->output, nullptr, 0}}, nullptr};
+    const LayerWeights& L = m->layers[l];
+    const int dq = m->n_head * m->d_head, dkv = m->n_head_kv * m->d_head;
+    switch (i % 4) {
+        case OP_QKV: return {OP_QKV, 3, {{&L.wq, L.bq, 0}, {&L.wk, L.bk, dq}, {&L.wv, L.bv, dq + dkv}}, nullptr};
+        case OP_WO: return {OP_WO, 1, {{&L.wo, nullptr, 0}}, nullptr};
+        case OP_GATE_UP: return {OP_GATE_UP, 2, {{&L.gate, nullptr, 0}, {&L.up, nullptr, 0}}, nullptr};
+        default: return {OP_DOWN, 1, {{&L.down, nullptr, 0}}, nullptr};
+    }
+}
 // Per-context streaming panels of the two-pass GEMM form (matrices that are not resident in the model's panel cache): one bf16
-// panel per GEMM kind, so the de-quantisation of the NEXT matrix (second stream) runs while the current GEMM does:
-//   [0] QKV   [1] Wo   [2] gate+up | lm_head   [3] down
+// panel per GEMM kind, so the de-quantisation of the NEXT matrix (second stream) runs while the current GEMM does.  The lm_head
+// shares the gate+up panel.
+int stream_panel(GemmKind k) { return k == OP_HEAD ? OP_GATE_UP : k; }
 void ensure_stream_panels(blk_ctx* c) {
     if (c->panel_tried) return;
     c->panel_tried = true;
     blk_model* m = c->m;
-    const int d = m->n_embd, dh = m->d_head, dq = m->n_head * dh, dkv = m->n_head_kv * dh, ff = m->n_ff;
-    auto rows = [](int n) { return (size_t)((n + 255) / 256) * 256; };
-    const size_t pe[4] = {(rows(dq) + 2 * rows(dkv)) * (size_t)d, rows(d) * (size_t)dq,
-                          std::max(2 * (size_t)((ff + 127) / 128) * 128 * (size_t)d, rows(m->n_vocab) * (size_t)d), rows(d) * (size_t)ff};
+    size_t elems[4] = {0, 0, 0, 0};      // each panel holds the largest op of its kind
+    for (int i = 0; i < n_gemm_ops(m); i++) {
+        const GemmOp g = gemm_op(m, i);
+        elems[stream_panel(g.kind)] = std::max(elems[stream_panel(g.kind)], g.panel_elems());
+    }
     bool ok = true;
     for (int i = 0; i < 4 && ok; i++) {
         void* p = nullptr;
-        ok = cudaMalloc(&p, pe[i] * sizeof(__nv_bfloat16)) == cudaSuccess;
+        ok = cudaMalloc(&p, elems[i] * sizeof(__nv_bfloat16)) == cudaSuccess;
         if (ok) { c->allocs.push_back(p); c->pf_panel[i] = reinterpret_cast<__nv_bfloat16*>(p); }
     }
     if (!ok) { (void)cudaGetLastError(); for (int i = 0; i < 4; i++) c->pf_panel[i] = nullptr; }
@@ -867,19 +889,6 @@ void ensure_stream_panels(blk_ctx* c) {
         BLK_CUDA(cudaEventCreateWithFlags(&c->pn_filled[i], cudaEventDisableTiming));
         BLK_CUDA(cudaEventCreateWithFlags(&c->pn_start[i], cudaEventDisableTiming));
     }
-}
-
-// fill of one op's panel (QKV | Wo | gate+up | down of layer l, or the lm_head); false: the combination takes the fused GEMM form
-bool fill_panel_op(blk_model* m, int i, __nv_bfloat16* panel, cudaStream_t ss, cudaError_t* err) {
-    const int dq = m->n_head * m->d_head, dkv = m->n_head_kv * m->d_head;
-    const int l = i >> 2, k = i & 3;
-    if (l >= m->n_layer) { const GemmPart o[1] = {{&m->output, nullptr, 0}}; return prefill_panel_fill(o, 1, panel, ss, err); }
-    const LayerWeights& L = m->layers[l];
-    if (k == 0) { const GemmPart q[3] = {{&L.wq, L.bq, 0}, {&L.wk, L.bk, dq}, {&L.wv, L.bv, dq + dkv}}; return prefill_panel_fill(q, 3, panel, ss, err); }
-    if (k == 1) { const GemmPart o[1] = {{&L.wo, nullptr, 0}}; return prefill_panel_fill(o, 1, panel, ss, err); }
-    if (k == 2) return prefill_panel_fill_swiglu(L.gate, L.up, panel, ss, err);
-    const GemmPart o[1] = {{&L.down, nullptr, 0}};
-    return prefill_panel_fill(o, 1, panel, ss, err);
 }
 
 // The model's resident panel cache (engine.hpp), built by the first multi-token pass: layer by layer while device memory beyond
@@ -890,7 +899,7 @@ const std::vector<__nv_bfloat16*>& model_panels(blk_ctx* c) {
     std::lock_guard<std::mutex> lk(pc.mu);
     if (pc.built) return pc.op;
     pc.built = true;
-    const int n_ops = 4 * m->n_layer + 1;
+    const int n_ops = n_gemm_ops(m);
     pc.op.assign(n_ops, nullptr);
     double cap_gb = 1e9;
     { const char* e = getenv("BLK_PANEL_CACHE_GB"); if (e) cap_gb = atof(e); }
@@ -901,18 +910,15 @@ const std::vector<__nv_bfloat16*>& model_panels(blk_ctx* c) {
     const size_t reserve = std::max((size_t)16 << 30, total_b / 6);
     size_t budget = free_b > reserve ? free_b - reserve : 0;
     budget = (size_t)std::min((double)budget, cap_gb * 1e9);
-    const int d = m->n_embd, dh = m->d_head, dq = m->n_head * dh, dkv = m->n_head_kv * dh, ff = m->n_ff;
-    auto rows = [](int n) { return (size_t)((n + 255) / 256) * 256; };
-    const size_t pe[5] = {(rows(dq) + 2 * rows(dkv)) * (size_t)d, rows(d) * (size_t)dq, 2 * (size_t)((ff + 127) / 128) * 128 * (size_t)d,
-                          rows(d) * (size_t)ff, rows(m->n_vocab) * (size_t)d};
     cudaStream_t ss = c->pf_stream;
     for (int i = 0; i < n_ops; i++) {
-        const size_t bytes = pe[i >= 4 * m->n_layer ? 4 : (i & 3)] * sizeof(__nv_bfloat16);
+        const GemmOp g = gemm_op(m, i);
+        const size_t bytes = g.panel_elems() * sizeof(__nv_bfloat16);
         if (pc.bytes + bytes > budget) break;
         void* p = nullptr;
         if (cudaMalloc(&p, bytes) != cudaSuccess) { (void)cudaGetLastError(); break; }
         cudaError_t err = cudaSuccess;
-        const bool ok = fill_panel_op(m, i, reinterpret_cast<__nv_bfloat16*>(p), ss, &err);
+        const bool ok = g.fill_panel(reinterpret_cast<__nv_bfloat16*>(p), ss, &err);
         if (!ok || err != cudaSuccess) { (void)cudaGetLastError(); cudaStreamSynchronize(ss); cudaFree(p); if (err != cudaSuccess) break; continue; }   // a type without a panel form: fused GEMM
         pc.allocs.push_back(p); pc.op[i] = reinterpret_cast<__nv_bfloat16*>(p); pc.bytes += bytes; pc.n_resident++;
     }
@@ -920,6 +926,64 @@ const std::vector<__nv_bfloat16*>& model_panels(blk_ctx* c) {
     log_msg(1, "resident bf16 panels: " + std::to_string(pc.n_resident) + " of " + std::to_string(n_ops) + " matrices, " + std::to_string(pc.bytes >> 20) + " MiB");
     return pc.op;
 }
+
+// Where each GEMM of a multi-token pass reads its weights from, in pass order (gemm_op):
+//  - a resident bf16 panel of the model cache: the TMA-fed GEMM at every batch size;
+//  - otherwise, from panel_min tokens on, a streaming panel: the matrix is de-quantised ONCE on pf_stream, one GEMM ahead of the
+//    main stream.  The fill of op i+1 starts when GEMM i starts (its panel's previous user, GEMM i-3, is then done), so fills
+//    overlap GEMMs, not the small bandwidth-bound kernels;
+//  - otherwise the fused form (weights de-quantised inside the GEMM, once per 256 tokens), which moves fewer bytes for few tokens.
+class GemmSchedule {
+  public:
+    // n_ops: the pass runs ops 0 .. n_ops - 1
+    GemmSchedule(blk_ctx* c, int n, int n_ops) : c_(c), n_ops_(n_ops), res_(model_panels(c)), filled_(n_ops, 0) {
+        bool all_res = true;
+        for (int i = 0; i < n_ops; i++) all_res = all_res && resident(i);
+        if (!all_res && c->panel_min > 0 && n >= c->panel_min) ensure_stream_panels(c);
+        stream_ = !all_res && c->pf_panel[0] && c->panel_min > 0 && n >= c->panel_min;
+        if (stream_ && !resident(0)) { BLK_CUDA(cudaEventRecord(c->pn_start[0], c->stream)); BLK_CUDA(cudaStreamWaitEvent(c->pf_stream, c->pn_start[0], 0)); }   // after whatever ran before
+        fill(0);
+    }
+    // main stream, right before the next GEMM of the pass (which must be of this kind): that op, with its panel
+    GemmOp next(GemmKind kind) {
+        const int i = next_++;
+        if (i >= n_ops_) throw BlkError(BLK_ERR_ARG, "multi-token pass: more GEMMs than scheduled");
+        GemmOp g = gemm_op(c_->m, i);
+        if (g.kind != kind) throw BlkError(BLK_ERR_ARG, "multi-token pass: GEMM op out of order");
+        const int b = stream_panel(g.kind);
+        const bool next_fill = stream_ && i + 1 < n_ops_ && !resident(i + 1);
+        if (next_fill) {
+            BLK_CUDA(cudaEventRecord(c_->pn_start[b], c_->stream));                 // GEMM i is about to start ...
+            BLK_CUDA(cudaStreamWaitEvent(c_->pf_stream, c_->pn_start[b], 0));       // ... so is the fill of op i + 1 (other panel; its last reader, GEMM i - 3, is done)
+        }
+        g.panel = resident(i);
+        if (!g.panel && stream_) {
+            BLK_CUDA(cudaStreamWaitEvent(c_->stream, c_->pn_filled[b], 0));
+            g.panel = filled_[i] ? c_->pf_panel[b] : nullptr;
+        }
+        if (next_fill) fill(i + 1);
+        return g;
+    }
+
+  private:
+    __nv_bfloat16* resident(int i) const { return i < (int)res_.size() ? res_[i] : nullptr; }
+    void fill(int i) {      // enqueue the fill of op i on the side stream
+        if (!stream_ || i >= n_ops_ || resident(i)) return;
+        const GemmOp g = gemm_op(c_->m, i);
+        const int b = stream_panel(g.kind);
+        cudaError_t err = cudaSuccess;
+        const bool ok = g.fill_panel(c_->pf_panel[b], c_->pf_stream, &err);
+        BLK_CUDA(err);
+        filled_[i] = ok ? 1 : 0;
+        BLK_CUDA(cudaEventRecord(c_->pn_filled[b], c_->pf_stream));
+        c_->launches += ok ? 2 : 0;
+    }
+    blk_ctx* c_;
+    int n_ops_, next_ = 0;
+    bool stream_ = false;
+    const std::vector<__nv_bfloat16*>& res_;
+    std::vector<char> filled_;
+};
 
 void ensure_prefill_bufs(blk_ctx* c, int T) {
     if (T <= c->pf_cap) return;
@@ -933,7 +997,6 @@ void ensure_prefill_bufs(blk_ctx* c, int T) {
     c->pf_qkv = dalloc<float>(c, t * (dq + 2 * dkv));
     c->pf_q = dalloc<__half>(c, t * dq);
     c->pf_ao = dalloc<__nv_bfloat16>(c, t * dq);
-    c->pf_g = dalloc<float>(c, t * ff); c->pf_u = dalloc<float>(c, t * ff);
     c->pf_h = dalloc<__nv_bfloat16>(c, t * ff);
     {   // split-K workspace of the prefill GEMMs (few-token batches): splits * tiles <= SMs, a tile is 256 x 256 f32
         int sms = 0; BLK_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, m->device));
@@ -949,7 +1012,6 @@ void ensure_prefill_bufs(blk_ctx* c, int T) {
     c->pf_claimed = dalloc<int32_t>(c, t * 10); c->pf_nclaimed = dalloc<int32_t>(c, t);
     c->pf_gath = dalloc<float>(c, t * 10); c->pf_topi = dalloc<int32_t>(c, t * 10); c->pf_topl = dalloc<float>(c, t * 10);
     c->pf_cap = cap;
-    BLK_CUDA(cudaFuncSetAttribute(prefill_attn_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, 3 * 64 * (128 + 8) * 2));
     BLK_CUDA(cudaFuncSetAttribute(prefill_attn_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, 3 * 64 * (64 + 8) * 2));
 }
 
@@ -958,11 +1020,7 @@ void topk_of_logits(blk_ctx* c) {
     blk_model* m = c->m;
     chunk_max_kernel<<<c->n_chunks, 256, 0, c->stream>>>(c->logits, m->n_vocab, c->chunk_shift, c->chunk_max);
     BLK_CUDA(cudaGetLastError()); c->launches++;
-    TopkArgs tk{};
-    tk.logits = c->logits; tk.n = m->n_vocab; tk.chunk_max = c->chunk_max; tk.n_chunks = c->n_chunks;
-    tk.cand_l = c->cand_l; tk.cand_i = c->cand_i; tk.cap = c->cand_cap; tk.count = c->counters + 1; tk.done = c->counters + 2;
-    tk.out_ids = c->top_ids; tk.out_logits = c->top_logits;
-    topk_select_kernel<<<16, 1024, 0, c->stream>>>(tk);
+    topk_select_kernel<<<16, 1024, 0, c->stream>>>(own_topk_args(c));
     BLK_CUDA(cudaGetLastError()); c->launches++;
     BLK_CUDA(cudaMemcpyAsync(c->h_top_ids, c->top_ids, TOPK_MAX * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
     BLK_CUDA(cudaMemcpyAsync(c->h_top_logits, c->top_logits, TOPK_MAX * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
@@ -977,27 +1035,61 @@ void launch_attn_gqa(const PrefillAttnArgs& pa, int n, int n_head_kv, cudaStream
     constexpr int BQ = 128 / GQ;
     prefill_attn_gqa_kernel<DH, GQ><<<dim3((n + BQ - 1) / BQ, n_head_kv), 256, smem, st>>>(pa);
 }
+// d_head 128: the tcgen05 kernel (GQA ratio <= 8, pf_vt allocated by ensure_prefill_bufs); d_head 64: the mma.sync kernels
 void launch_prefill_attn(blk_ctx* c, const PrefillAttnArgs& pa, int n, cudaStream_t st) {
     const blk_model* m = c->m;
     const int dh = m->d_head, gq = m->n_head / m->n_head_kv;
-    if (c->pf_vt && prefill_attn_tc_supported(dh, m->n_head, m->n_head_kv)) {
-        // tcgen05 attention: the layer's pools are recovered from the arguments
+    if (dh == 128) {
+        if (!c->pf_vt || !prefill_attn_tc_supported(dh, m->n_head, m->n_head_kv)) throw BlkError(BLK_ERR_ARG, "prefill attention: no kernel for this head shape");
+        // the layer's pools are recovered from the arguments
         BLK_CUDA(prefill_attn_tc(pa.q, pa.k_pool, pa.v_pool, pa.page_table, c->n_pages, pa.pos0, c->n_past, pa.out, c->pf_vt, c->pf_vt_pad, n,
                                  m->n_head, m->n_head_kv, pa.kv_dim, pa.scale, st));
         return;
     }
-    if (dh == 128 && gq == 4) launch_attn_gqa<128, 4>(pa, n, m->n_head_kv, st);
-    else if (dh == 128 && gq == 8) launch_attn_gqa<128, 8>(pa, n, m->n_head_kv, st);
-    else if (dh == 128 && gq == 2) launch_attn_gqa<128, 2>(pa, n, m->n_head_kv, st);
-    else if (dh == 64 && gq == 4) launch_attn_gqa<64, 4>(pa, n, m->n_head_kv, st);
-    else if (dh == 64 && gq == 8) launch_attn_gqa<64, 8>(pa, n, m->n_head_kv, st);
-    else if (dh == 64 && gq == 2) launch_attn_gqa<64, 2>(pa, n, m->n_head_kv, st);
-    else {
-        const dim3 agrid((n + 63) / 64, m->n_head);
-        if (dh == 128) prefill_attn_kernel<128><<<agrid, 128, 3 * 64 * (128 + 8) * 2, st>>>(pa);
-        else prefill_attn_kernel<64><<<agrid, 128, 3 * 64 * (64 + 8) * 2, st>>>(pa);
-    }
+    if (gq == 4) launch_attn_gqa<64, 4>(pa, n, m->n_head_kv, st);
+    else if (gq == 8) launch_attn_gqa<64, 8>(pa, n, m->n_head_kv, st);
+    else if (gq == 2) launch_attn_gqa<64, 2>(pa, n, m->n_head_kv, st);
+    else prefill_attn_kernel<64><<<dim3((n + 63) / 64, m->n_head), 128, 3 * 64 * (64 + 8) * 2, st>>>(pa);
     BLK_CUDA(cudaGetLastError());
+}
+
+// The layers of a multi-token pass over the n rows of c->pf_x: RMSNorm, QKV GEMM, attend(l) (pf_qkv -> pf_ao: RoPE, the new KV
+// cache rows and the attention of layer l), Wo GEMM (+residual), RMSNorm, gate+up GEMM (SwiGLU epilogue), down GEMM (+residual).
+// Few-token passes fold the split-K reduce of Wo / down into the RMSNorm that follows (pend).  final_norm: the caller runs the
+// final RMSNorm with pend after the last layer; otherwise the last down GEMM reduces its own partial sums.
+template <class Attend>
+void run_layers(blk_ctx* c, int n, GemmSchedule& sched, PendingReduce& pend, bool final_norm, Attend attend) {
+    blk_model* m = c->m;
+    const int d = m->n_embd, dq = m->n_head * m->d_head, dkv = m->n_head_kv * m->d_head, ff = m->n_ff;
+    const long long ldq = dq + 2 * dkv;
+    cudaStream_t st = c->stream;
+    const SplitKWs sk{c->pf_splitk, c->pf_splitk_elems, &pend};
+    SplitKWs sk_last = sk;
+    if (!final_norm) sk_last.defer = nullptr;
+    for (int l = 0; l < m->n_layer; l++) {
+        const LayerWeights& L = m->layers[l];
+        rmsnorm_bf16_launch(c->pf_x, L.attn_norm, d, m->rms_eps, c->pf_xn, n, st, &pend);
+        BLK_CUDA(cudaGetLastError());
+        prof_mark(c, "rmsnorm_bf16");
+        GemmOp g = sched.next(OP_QKV);
+        BLK_CUDA(prefill_gemm_multi(g.part, g.n_parts, c->pf_xn, n, c->pf_qkv, ldq, st, g.panel, &sk));
+        prof_mark(c, "gemm_qkv");
+        attend(l);
+        g = sched.next(OP_WO);
+        BLK_CUDA(prefill_gemm(*g.part[0].W, c->pf_ao, n, c->pf_x, d, nullptr, 1, st, g.panel, &sk));
+        prof_mark(c, "gemm_wo");
+        rmsnorm_bf16_launch(c->pf_x, L.ffn_norm, d, m->rms_eps, c->pf_xn, n, st, &pend);
+        BLK_CUDA(cudaGetLastError());
+        prof_mark(c, "rmsnorm_bf16");
+        g = sched.next(OP_GATE_UP);
+        BLK_CUDA(prefill_gemm_swiglu(*g.part[0].W, *g.part[1].W, c->pf_xn, n, c->pf_h, ff, st, g.panel, &sk));
+        prof_mark(c, "gemm_gate_up_swiglu");
+        g = sched.next(OP_DOWN);
+        BLK_CUDA(prefill_gemm(*g.part[0].W, c->pf_h, n, c->pf_x, d, nullptr, 1, st, g.panel, l + 1 < m->n_layer ? &sk : &sk_last));
+        prof_mark(c, "gemm_down");
+        c->launches += 6;
+    }
+    if (pend.ws && !final_norm) throw BlkError(BLK_ERR_CUDA, "multi-token pass: a deferred split-K reduce was left unconsumed");
 }
 
 // One causal prefill of n tokens at positions n_past.. .  verify != nullptr: logits of EVERY position go through the
@@ -1007,7 +1099,7 @@ struct VerifyIo { const int32_t* claimed; const int32_t* n_claimed; float* gathe
 
 void prefill_chunk(blk_ctx* c, const int32_t* tokens, int n, const VerifyIo* verify, int verify_row0) {
     blk_model* m = c->m;
-    const int d = m->n_embd, dh = m->d_head, dq = m->n_head * dh, dkv = m->n_head_kv * dh, ff = m->n_ff, V = m->n_vocab;
+    const int d = m->n_embd, dh = m->d_head, dq = m->n_head * dh, dkv = m->n_head_kv * dh, V = m->n_vocab;
     ensure_prefill_bufs(c, n);
     flush_pos_shift(c);
     note_new_cells(c, n);
@@ -1017,68 +1109,14 @@ void prefill_chunk(blk_ctx* c, const int32_t* tokens, int n, const VerifyIo* ver
     embed_kernel<<<n, 256, 0, st>>>(m->tok_embd, c->pf_tokens, c->d_pos, c->pf_x, c->pf_rope, dh / 2, m->theta_scale, m->rope_freqs);
     BLK_CUDA(cudaGetLastError()); c->launches++;
     prof_mark(c, "embed");
-    const long long ldq = dq + 2 * dkv;
-    // ---- two-pass form: the dequantisation passes run on the side stream, one GEMM ahead of the main stream ----
-    //   op 4l + {0: QKV, 1: Wo, 2: gate+up, 3: down}, op 4 n_layer: lm_head (panel 2).  The fill of op i+1 starts when GEMM i
-    //   starts (its panel's previous user, GEMM i-3, is then done), so fills overlap GEMMs, not the small bandwidth-bound kernels.
     // verify without the verifier's own per-position top-10: only the logits at the claimed ids are needed (what the reference's
     // fillCtx reads, Session.cpp:263-282) -> sparse rows of the vocabulary projection instead of the T x V GEMM
     const bool sparse_head = verify && !verify->top && m->output.type != QT_F32 && m->output.type != QT_F16 && (d % 64) == 0;
-    const int n_ops = 4 * m->n_layer + (verify && !sparse_head ? 1 : 0);
-    // GEMM form per matrix: resident bf16 panel (model cache) -> TMA-fed GEMM at every batch size; otherwise many tokens: the matrix is
-    // de-quantised ONCE into a streaming panel (second stream, one GEMM ahead); few tokens: the fused form (weights de-quantised
-    // inside the GEMM, once per 256 tokens) moves fewer bytes
-    const std::vector<__nv_bfloat16*>& res = model_panels(c);
-    auto res_op = [&](int i) -> __nv_bfloat16* { return i < (int)res.size() ? res[i] : nullptr; };
-    bool all_res = true;
-    for (int i = 0; i < n_ops; i++) all_res = all_res && res_op(i);
-    if (!all_res && c->panel_min > 0 && n >= c->panel_min) ensure_stream_panels(c);
-    const bool panel = !all_res && c->pf_panel[0] && c->panel_min > 0 && n >= c->panel_min;
-    std::vector<char> op_panel(n_ops + 1, 0);
-    auto panel_of = [&](int i) { return i >= 4 * m->n_layer ? 2 : (i & 3); };
-    auto fill_op = [&](int i) {      // enqueue the fill of op i on the side stream
-        if (!panel || i >= n_ops || res_op(i)) return;
-        const int b = panel_of(i);
-        cudaError_t err = cudaSuccess;
-        const bool ok = fill_panel_op(m, i, c->pf_panel[b], c->pf_stream, &err);
-        BLK_CUDA(err);
-        op_panel[i] = ok ? 1 : 0;
-        BLK_CUDA(cudaEventRecord(c->pn_filled[b], c->pf_stream));
-        c->launches += ok ? 2 : 0;
-    };
-    auto before_gemm = [&](int i) -> __nv_bfloat16* {      // main stream, right before GEMM i; returns its panel (nullptr: fused form)
-        const int b = panel_of(i);
-        const bool next_fill = panel && i + 1 < n_ops && !res_op(i + 1);
-        if (next_fill) {
-            BLK_CUDA(cudaEventRecord(c->pn_start[b], st));                      // GEMM i is about to start ...
-            BLK_CUDA(cudaStreamWaitEvent(c->pf_stream, c->pn_start[b], 0));     // ... so is the fill of op i + 1 (other panel; its last reader, GEMM i - 3, is done)
-        }
-        __nv_bfloat16* mine = res_op(i);
-        if (!mine && panel) {
-            BLK_CUDA(cudaStreamWaitEvent(st, c->pn_filled[b], 0));
-            mine = op_panel[i] ? c->pf_panel[b] : nullptr;
-        }
-        if (next_fill) fill_op(i + 1);
-        return mine;
-    };
-    auto after_gemm = [&](int) {};
-    if (panel && !res_op(0)) { BLK_CUDA(cudaEventRecord(c->pn_start[0], st)); BLK_CUDA(cudaStreamWaitEvent(c->pf_stream, c->pn_start[0], 0)); }   // after whatever ran before
-    fill_op(0);
-    // few-token batches: the split-K reduce of Wo / down (accumulates onto the residual stream) is folded into the RMSNorm that follows
+    GemmSchedule sched(c, n, n_gemm_ops(m) - (verify && !sparse_head ? 0 : 1));
     PendingReduce pend;
-    const SplitKWs sk{c->pf_splitk, c->pf_splitk_elems, &pend};
-    SplitKWs sk_last = sk; sk_last.defer = nullptr;      // the last down GEMM of a pass that is not followed by the final RMSNorm kernel
-    for (int l = 0; l < m->n_layer; l++) {
-        const LayerWeights& L = m->layers[l];
-        rmsnorm_bf16_launch(c->pf_x, L.attn_norm, d, m->rms_eps, c->pf_xn, n, st, &pend);
-        BLK_CUDA(cudaGetLastError());
-        prof_mark(c, "rmsnorm_bf16");
-        const GemmPart qkv_parts[3] = {{&L.wq, L.bq, 0}, {&L.wk, L.bk, dq}, {&L.wv, L.bv, dq + dkv}};
-        BLK_CUDA(prefill_gemm_multi(qkv_parts, 3, c->pf_xn, n, c->pf_qkv, ldq, st, before_gemm(4 * l), false, &sk));
-        after_gemm(4 * l);
-        prof_mark(c, "gemm_qkv");
+    run_layers(c, n, sched, pend, verify != nullptr, [&](int l) {
         QkvPostArgs qa{};
-        qa.qkv = c->pf_qkv; qa.ld = ldq; qa.rope_cs = c->pf_rope; qa.pos0 = c->d_pos; qa.q_out = c->pf_q;
+        qa.qkv = c->pf_qkv; qa.ld = dq + 2 * dkv; qa.rope_cs = c->pf_rope; qa.pos0 = c->d_pos; qa.q_out = c->pf_q;
         qa.k_pool = c->k_pool[l]; qa.v_pool = c->v_pool[l]; qa.page_table = c->page_table;
         qa.dq = dq; qa.dkv = dkv; qa.d_head = dh; qa.neox = m->neox ? 1 : 0;
         BLK_CUDA(launch_chain(qkv_post_kernel, dim3(n), dim3(256), 0, st, qa));
@@ -1089,29 +1127,15 @@ void prefill_chunk(blk_ctx* c, const int32_t* tokens, int n, const VerifyIo* ver
         pa.out = c->pf_ao; pa.T = n; pa.n_head = m->n_head; pa.n_head_kv = m->n_head_kv; pa.kv_dim = dkv; pa.scale = 1.0f / sqrtf((float)dh);
         launch_prefill_attn(c, pa, n, st);
         prof_mark(c, "flash_attn");
-        BLK_CUDA(prefill_gemm(L.wo, c->pf_ao, n, c->pf_x, d, nullptr, 1, st, before_gemm(4 * l + 1), false, &sk));
-        after_gemm(4 * l + 1);
-        prof_mark(c, "gemm_wo");
-        rmsnorm_bf16_launch(c->pf_x, L.ffn_norm, d, m->rms_eps, c->pf_xn, n, st, &pend);
-        BLK_CUDA(cudaGetLastError());
-        prof_mark(c, "rmsnorm_bf16");
-        BLK_CUDA(prefill_gemm_swiglu(L.gate, L.up, c->pf_xn, n, c->pf_h, ff, st, before_gemm(4 * l + 2), false, &sk));
-        after_gemm(4 * l + 2);
-        prof_mark(c, "gemm_gate_up_swiglu");
-        BLK_CUDA(prefill_gemm(L.down, c->pf_h, n, c->pf_x, d, nullptr, 1, st, before_gemm(4 * l + 3), false, (l + 1 < m->n_layer || verify) ? &sk : &sk_last));
-        after_gemm(4 * l + 3);
-        prof_mark(c, "gemm_down");
-        c->launches += 12;
-    }
+        c->launches += 6;      // (with the 6 run_layers counts: 12 per layer)
+    });
     BLK_CUDA(launch_pdl(advance_pos_kernel, dim3(1), dim3(32), 0, st, c->d_pos, n));
     c->launches++;
-    if (pend.ws && !verify) throw BlkError(BLK_ERR_CUDA, "prefill: a deferred split-K reduce was left unconsumed");      // (verify: the final RMSNorm below takes it)
     if (verify) {
         BLK_CUDA(cudaMemcpyAsync(c->pf_claimed, verify->claimed + (size_t)verify_row0 * 10, (size_t)n * 10 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
         BLK_CUDA(cudaMemcpyAsync(c->pf_nclaimed, verify->n_claimed + verify_row0, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
         rmsnorm_bf16_launch(c->pf_x, m->out_norm, d, m->rms_eps, c->pf_xn, n, st, &pend);
         BLK_CUDA(cudaGetLastError()); c->launches++;
-        __nv_bfloat16* head_panel = nullptr;
         if (sparse_head) {
             BLK_CUDA(prefill_claimed_logits(m->output, c->pf_xn, c->pf_claimed, c->pf_nclaimed, n, c->pf_gath, st));
             c->launches++;
@@ -1121,9 +1145,11 @@ void prefill_chunk(blk_ctx* c, const int32_t* tokens, int n, const VerifyIo* ver
             a.nseg = 1; a.seg[0] = {m->output, nullptr, 0, 0}; a.total_pairs = V / 2; a.out = c->logits;
             matvec<EPI_STORE>(c, a, c->pf_x + (size_t)(n - 1) * d, m->out_norm, c->act_d, "gemv_lm_head");
         }
+        GemmOp head{};
         for (int r0 = 0; r0 < n && !sparse_head; r0 += c->pf_logit_rows) {
             const int rows = std::min(c->pf_logit_rows, n - r0);
-            BLK_CUDA(prefill_gemm(m->output, c->pf_xn + (size_t)r0 * d, rows, c->pf_logits, V, nullptr, 0, st, r0 == 0 ? (head_panel = before_gemm(4 * m->n_layer)) : head_panel, false));
+            if (r0 == 0) head = sched.next(OP_HEAD);
+            BLK_CUDA(prefill_gemm(*head.part[0].W, c->pf_xn + (size_t)r0 * d, rows, c->pf_logits, V, nullptr, 0, st, head.panel));
             prof_mark(c, "gemm_lm_head");
             RowTopkArgs ta{};
             ta.logits = c->pf_logits; ta.ld = V; ta.n_vocab = V; ta.row0 = r0;
@@ -1214,6 +1240,14 @@ void step(blk_ctx* c, int32_t tok, bool with_head) {
 
 } // namespace
 
+extern "C" int64_t blk_model_panel_bytes(blk_model* m, int32_t* n_resident, int32_t* n_matrices) {
+    if (!m) return 0;
+    std::lock_guard<std::mutex> lk(m->panels.mu);
+    if (n_resident) *n_resident = m->panels.n_resident;
+    if (n_matrices) *n_matrices = n_gemm_ops(m);
+    return (int64_t)m->panels.bytes;
+}
+
 extern "C" blk_ctx* blk_ctx_create(blk_model* m, int32_t n_ctx, int32_t n_batch) {
     if (!m) { fail(BLK_ERR_ARG, "null model"); return nullptr; }
     if (m->vocab_only) { fail(BLK_ERR_ARG, "Failed to create context: the model was loaded vocabulary-only"); return nullptr; }
@@ -1250,7 +1284,6 @@ extern "C" blk_ctx* blk_ctx_create(blk_model* m, int32_t n_ctx, int32_t n_batch)
         c->x = dalloc<float>(c.get(), d); c->qbuf = dalloc<float>(c.get(), dq); c->hbuf = dalloc<float>(c.get(), ff);
         c->rope_cs = dalloc<float2>(c.get(), dh / 2);
         c->act_d = make_act(c.get(), d); c->act_q = make_act(c.get(), dq); c->act_q2 = make_act(c.get(), dq); c->act_ff = make_act(c.get(), ff);
-        BLK_CUDA(cudaDeviceGetAttribute(&c->n_sms, cudaDevAttrMultiProcessorCount, m->device));
         {   // single-kernel cluster attention when one CTA's share of the scores fits in shared memory
             const int gq = m->n_head / m->n_head_kv;
             c->attn_cluster = 8;
@@ -1536,7 +1569,7 @@ extern "C" blk_status blk_decode_batch(blk_ctx* ws, blk_ctx* const* ctxs, const 
     return guarded([&] {
         blk_model* m = ws->m;
         BLK_CUDA(cudaSetDevice(m->device));
-        const int d = m->n_embd, dh = m->d_head, dq = m->n_head * dh, dkv = m->n_head_kv * dh, ff = m->n_ff, V = m->n_vocab;
+        const int d = m->n_embd, dh = m->d_head, dq = m->n_head * dh, dkv = m->n_head_kv * dh, V = m->n_vocab;
         for (int i = 0; i < n; i++) {
             blk_ctx* c = ctxs[i];
             if (!c || c->m != m) throw BlkError(BLK_ERR_ARG, "blk_decode_batch: every context must belong to the workspace's model");
@@ -1571,21 +1604,14 @@ extern "C" blk_status blk_decode_batch(blk_ctx* ws, blk_ctx* const* ctxs, const 
         BLK_CUDA(cudaMemcpyAsync(ws->bd_dev, ws->bd_host, sizeof(BatchDesc), cudaMemcpyHostToDevice, st));
         embed_rows_kernel<<<n, 256, 0, st>>>(m->tok_embd, dv->tokens, dv->rpos, ws->pf_x, ws->pf_rope, dh / 2, m->theta_scale, m->rope_freqs);
         BLK_CUDA(cudaGetLastError()); ws->launches++;
-        const long long ldq = dq + 2 * dkv;
         const ChainPdl chain_scope(n);
-        PendingReduce pend;      // split-K reduce of Wo / down folded into the RMSNorm that follows
-        const SplitKWs sk{ws->pf_splitk, ws->pf_splitk_elems, &pend};
         // matrices with a resident bf16 panel (model cache) take the TMA-fed GEMM: the step then streams the panels at HBM speed
-        // instead of waiting for the de-quantising producers of the fused form
-        const std::vector<__nv_bfloat16*>& res = model_panels(ws);
-        auto res_op = [&](int i) -> __nv_bfloat16* { return i < (int)res.size() ? res[i] : nullptr; };
-        for (int l = 0; l < m->n_layer; l++) {
-            const LayerWeights& L = m->layers[l];
-            rmsnorm_bf16_launch(ws->pf_x, L.attn_norm, d, m->rms_eps, ws->pf_xn, n, st, &pend);
-            const GemmPart qkv_parts[3] = {{&L.wq, L.bq, 0}, {&L.wk, L.bk, dq}, {&L.wv, L.bv, dq + dkv}};
-            BLK_CUDA(prefill_gemm_multi(qkv_parts, 3, ws->pf_xn, n, ws->pf_qkv, ldq, st, res_op(4 * l), false, &sk));
+        // instead of waiting for the de-quantising producers of the fused form (BATCH_MAX rows are below the default panel_min)
+        GemmSchedule sched(ws, n, n_gemm_ops(m));
+        PendingReduce pend;
+        run_layers(ws, n, sched, pend, true, [&](int l) {
             QkvPostBatchArgs qa{};
-            qa.base.qkv = ws->pf_qkv; qa.base.ld = ldq; qa.base.rope_cs = ws->pf_rope; qa.base.q_out = ws->pf_q;
+            qa.base.qkv = ws->pf_qkv; qa.base.ld = dq + 2 * dkv; qa.base.rope_cs = ws->pf_rope; qa.base.q_out = ws->pf_q;
             qa.base.dq = dq; qa.base.dkv = dkv; qa.base.d_head = dh; qa.base.neox = m->neox ? 1 : 0;
             qa.pos = dv->pos; qa.page_table = dv->page_table; qa.k_pools = dv->k_pools; qa.v_pools = dv->v_pools; qa.layer = l;
             BLK_CUDA(launch_chain(qkv_post_batch_kernel, dim3(n), dim3(256), 0, st, qa));
@@ -1595,14 +1621,11 @@ extern "C" blk_status blk_decode_batch(blk_ctx* ws, blk_ctx* const* ctxs, const 
             if (dh == 128) BLK_CUDA(launch_chain(decode_attn_batch_kernel<128>, dim3(m->n_head_kv, n), dim3(256), 0, st, aa));
             else BLK_CUDA(launch_chain(decode_attn_batch_kernel<64>, dim3(m->n_head_kv, n), dim3(256), 0, st, aa));
             BLK_CUDA(cudaGetLastError());
-            BLK_CUDA(prefill_gemm(L.wo, ws->pf_ao, n, ws->pf_x, d, nullptr, 1, st, res_op(4 * l + 1), false, &sk));
-            rmsnorm_bf16_launch(ws->pf_x, L.ffn_norm, d, m->rms_eps, ws->pf_xn, n, st, &pend);
-            BLK_CUDA(prefill_gemm_swiglu(L.gate, L.up, ws->pf_xn, n, ws->pf_h, ff, st, res_op(4 * l + 2), false, &sk));
-            BLK_CUDA(prefill_gemm(L.down, ws->pf_h, n, ws->pf_x, d, nullptr, 1, st, res_op(4 * l + 3), false, &sk));
-            ws->launches += 8;
-        }
+            ws->launches += 2;
+        });
         rmsnorm_bf16_launch(ws->pf_x, m->out_norm, d, m->rms_eps, ws->pf_xn, n, st, &pend);
-        BLK_CUDA(prefill_gemm(m->output, ws->pf_xn, n, ws->pf_logits, V, nullptr, 0, st, res_op(4 * m->n_layer), false));
+        const GemmOp head = sched.next(OP_HEAD);
+        BLK_CUDA(prefill_gemm(*head.part[0].W, ws->pf_xn, n, ws->pf_logits, V, nullptr, 0, st, head.panel));
         ws->launches += 2;
         // threshold top-64 of every row (the selector of the batch-1 path, blockIdx.y = row): two launches for the whole batch
         {
@@ -1956,7 +1979,6 @@ extern "C" blk_status blk_test_gemv(int32_t device, int32_t type, const void* bl
         BLK_CUDA(cudaMemcpyAsync(d_x, x, k * 4, cudaMemcpyHostToDevice, c.stream));
         GemvArgs a{};
         a.nseg = 1; a.seg[0] = {tm.W, nullptr, 0, 0}; a.total_pairs = (int)(rows / 2); a.out = d_y;
-        BLK_CUDA(cudaDeviceGetAttribute(&c.n_sms, cudaDevAttrMultiProcessorCount, device));
         matvec<EPI_STORE>(&c, a, d_x, nullptr, act, "test");
         BLK_CUDA(cudaMemcpyAsync(y, d_y, rows * 4, cudaMemcpyDeviceToHost, c.stream));
         BLK_CUDA(cudaStreamSynchronize(c.stream));
@@ -1975,7 +1997,11 @@ extern "C" blk_status blk_test_gemm(int32_t device, int32_t type, const void* bl
         BLK_CUDA(cudaMemcpyAsync(d_x, x, (size_t)n_tok * k * 4, cudaMemcpyHostToDevice, c.stream));
         BLK_CUDA(convert_f32_to_bf16(d_x, d_xb, (size_t)n_tok * k, c.stream));
         __nv_bfloat16* panel = nullptr;        // BLK_TEST_PANEL=1: the two-pass form (dequantise to a bf16 panel, TMA-fed GEMM)
-        { const char* tp = getenv("BLK_TEST_PANEL"); if (tp && tp[0] == '1' && type != GT_F32 && type != GT_F16) panel = dalloc<__nv_bfloat16>(&c, prefill_panel_rows((int)rows) * (size_t)k); }
+        const GemmPart part{&tm.W, nullptr, 0};
+        { const char* tp = getenv("BLK_TEST_PANEL"); if (tp && tp[0] == '1' && type != GT_F32 && type != GT_F16) panel = dalloc<__nv_bfloat16>(&c, prefill_panel_elems(&part, 1, false)); }
+        cudaError_t err = cudaSuccess;
+        if (panel && !prefill_panel_fill(&part, 1, false, panel, c.stream, &err)) panel = nullptr;
+        BLK_CUDA(err);
         BLK_CUDA(prefill_gemm(tm.W, d_xb, (int)n_tok, d_y, rows, nullptr, 0, c.stream, panel));
         BLK_CUDA(cudaMemcpyAsync(y, d_y, (size_t)n_tok * rows * 4, cudaMemcpyDeviceToHost, c.stream));
         BLK_CUDA(cudaStreamSynchronize(c.stream));
@@ -1993,10 +2019,17 @@ extern "C" blk_status blk_bench_gemm(int32_t device, int32_t type, const void* b
         float* d_y = dalloc<float>(&c, (size_t)n_tok * rows);
         BLK_CUDA(cudaMemsetAsync(d_xb, 0x3c, (size_t)n_tok * k * 2, c.stream));
         __nv_bfloat16* panel = nullptr;        // BLK_TEST_PANEL=1: time the two-pass form (dequantisation pass included)
-        { const char* tp = getenv("BLK_TEST_PANEL"); if (tp && tp[0] == '1') panel = dalloc<__nv_bfloat16>(&c, prefill_panel_rows((int)rows) * (size_t)k); }
-        for (int i = 0; i < 3; i++) BLK_CUDA(prefill_gemm(tm.W, d_xb, (int)n_tok, d_y, rows, nullptr, 0, c.stream, panel));
+        const GemmPart part{&tm.W, nullptr, 0};
+        { const char* tp = getenv("BLK_TEST_PANEL"); if (tp && tp[0] == '1') panel = dalloc<__nv_bfloat16>(&c, prefill_panel_elems(&part, 1, false)); }
+        auto run = [&] {
+            cudaError_t err = cudaSuccess;
+            const bool filled = panel && prefill_panel_fill(&part, 1, false, panel, c.stream, &err);
+            BLK_CUDA(err);
+            BLK_CUDA(prefill_gemm(tm.W, d_xb, (int)n_tok, d_y, rows, nullptr, 0, c.stream, filled ? panel : nullptr));
+        };
+        for (int i = 0; i < 3; i++) run();
         BLK_CUDA(cudaEventRecord(c.ev0, c.stream));
-        for (int i = 0; i < iters; i++) BLK_CUDA(prefill_gemm(tm.W, d_xb, (int)n_tok, d_y, rows, nullptr, 0, c.stream, panel));
+        for (int i = 0; i < iters; i++) run();
         BLK_CUDA(cudaEventRecord(c.ev1, c.stream));
         BLK_CUDA(cudaEventSynchronize(c.ev1));
         float ms = 0.0f;
@@ -2086,12 +2119,13 @@ extern "C" blk_status blk_test_qkv_post(int32_t device, const float* qkv, int32_
 
 // Causal prefill attention of T query rows at positions pos0 .. over a cache of pos0 + T keys: q [T][n_head*dh], k / v [pos0+T][n_head_kv*dh]
 // (rounded to f16 on the way in, like the cache); out [T][n_head*dh] = the kernel's bf16 output as f32.  *used_tc = 1 when the tcgen05
-// kernel ran (d_head 128), 0 for the mma.sync fallbacks.
+// kernel ran (d_head 128), 0 for the mma.sync kernels (d_head 64).  A d_head 128 shape the tcgen05 kernel does not cover is BLK_ERR_ARG.
 extern "C" blk_status blk_test_prefill_attn(int32_t device, const float* q, const float* k, const float* v, int32_t T, int32_t pos0, int32_t n_head,
                                             int32_t n_head_kv, int32_t d_head, float* out, int32_t* used_tc) {
     return guarded([&] {
         if (blk_init() != BLK_OK) throw BlkError(BLK_ERR_NO_DEVICE, g_last_error);
         if (T <= 0 || pos0 < 0 || (d_head != 64 && d_head != 128) || n_head <= 0 || n_head_kv <= 0 || n_head % n_head_kv) throw BlkError(BLK_ERR_ARG, "blk_test_prefill_attn: bad shape");
+        if (d_head == 128 && !prefill_attn_tc_supported(d_head, n_head, n_head_kv)) throw BlkError(BLK_ERR_ARG, "blk_test_prefill_attn: no kernel for this shape");
         BLK_CUDA(cudaSetDevice(device));
         const int dq = n_head * d_head, dkv = n_head_kv * d_head, n_keys = pos0 + T;
         blk_model mm; mm.device = device; mm.n_head = n_head; mm.n_head_kv = n_head_kv; mm.d_head = d_head;
@@ -2116,9 +2150,8 @@ extern "C" blk_status blk_test_prefill_attn(int32_t device, const float* q, cons
         BLK_CUDA(cudaStreamSynchronize(c.stream));
         BLK_CUDA(cudaMemcpyAsync(fkv, v, (size_t)n_keys * dkv * 4, cudaMemcpyHostToDevice, c.stream));
         f32_to_f16_kernel<<<grid_of((size_t)n_keys * dkv), 256, 0, c.stream>>>(fkv, vp, (size_t)n_keys * dkv);
-        const bool tc = prefill_attn_tc_supported(d_head, n_head, n_head_kv);
+        const bool tc = d_head == 128;
         if (tc) { c.pf_vt_pad = (c.n_pages * KV_PAGE + 127) / 128 * 128; c.pf_vt = dalloc<__half>(&c, (size_t)n_head_kv * 128 * c.pf_vt_pad); }
-        BLK_CUDA(cudaFuncSetAttribute(prefill_attn_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, 3 * 64 * (128 + 8) * 2));
         BLK_CUDA(cudaFuncSetAttribute(prefill_attn_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, 3 * 64 * (64 + 8) * 2));
         PrefillAttnArgs pa{};
         pa.q = q16; pa.k_pool = kp; pa.v_pool = vp; pa.page_table = c.page_table; pa.pos0 = c.d_pos; pa.out = o; pa.T = T;

@@ -76,11 +76,10 @@ struct blk_model {
     std::map<std::string, std::string> meta;
     int64_t weight_bytes_per_token = 0;
     int act_fmt = blk::ACT_F32;       // activation format of the layer mat-vecs
-    int act_fmt_out = blk::ACT_F32;   // ... of the lm_head
     // Resident bf16 copies ("panels") of the layer matrices for the TMA-fed tcgen05 GEMMs of the multi-token paths (prompt prefill,
     // verify, batched decode): B200 has 180 GB, an 8B model's panels are 14 GB.  Filled once, by the first multi-token pass that
-    // wants them, into whatever device memory is free beyond a reserve (BLK_PANEL_CACHE_GB caps it, 0 = off); op index
-    // 4 l + {0 QKV, 1 Wo, 2 gate+up, 3 down}, 4 n_layer = lm_head; nullptr = not resident (streamed through the per-context panels).
+    // wants them, into whatever device memory is free beyond a reserve (BLK_PANEL_CACHE_GB caps it, 0 = off); indexed by GEMM op
+    // (gemm_op in engine.cu); nullptr = not resident (streamed through the per-context panels).
     struct PanelCache { std::mutex mu; bool built = false; std::vector<__nv_bfloat16*> op; std::vector<void*> allocs; size_t bytes = 0; int n_resident = 0; } panels;
     ~blk_model();
 };
@@ -116,7 +115,6 @@ struct blk_ctx {
     float* hbuf = nullptr;                // [n_ff]
     float2* rope_cs = nullptr;            // [d_head/2]
     blk::ActBuf act_d, act_q, act_q2, act_ff;
-    int n_sms = 148;
     int attn_cluster = 0, attn_cap = 0;   // cluster size (0 = three-kernel fallback) and tokens per CTA
     float* part_o = nullptr; float* scores = nullptr;
     float* logits = nullptr;              // [n_vocab] of the last decoded token
@@ -136,7 +134,7 @@ struct blk_ctx {
     int pf_cap = 0, pf_logit_rows = 0;
     int32_t* pf_tokens = nullptr; float2* pf_rope = nullptr;
     float* pf_x = nullptr; __nv_bfloat16* pf_xn = nullptr; float* pf_qkv = nullptr; __half* pf_q = nullptr;
-    __nv_bfloat16* pf_ao = nullptr; float* pf_g = nullptr; float* pf_u = nullptr; __nv_bfloat16* pf_h = nullptr;
+    __nv_bfloat16* pf_ao = nullptr; __nv_bfloat16* pf_h = nullptr;
     float* pf_logits = nullptr;
     __half* pf_vt = nullptr; int pf_vt_pad = 0;           // transposed V of one layer for the tcgen05 prefill attention
     float* pf_splitk = nullptr; size_t pf_splitk_elems = 0;               // partial sums of the split-K prefill GEMMs (few-token batches)

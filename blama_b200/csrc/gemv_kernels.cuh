@@ -11,7 +11,6 @@ constexpr int KV_PAGE = 64;          // tokens per KV page
 constexpr int GEMV_THREADS = 256;    // 8 warps per CTA
 constexpr int MAX_GQ = 8;            // query heads per KV head (70B: 8, Qwen2.5-7B: 7)
 constexpr int TOPK_MAX = 64;
-constexpr int TOPK_CHUNK = 1024;     // logits per CTA in the first top-k stage
 
 // activations prepared for a quantised mat-vec
 struct ActBuf {

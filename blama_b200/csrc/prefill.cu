@@ -46,7 +46,7 @@ cudaError_t convert_f32_to_bf16(const float* x, __nv_bfloat16* y, size_t n, cuda
 }
 
 namespace {
-using GemmKernel = void (*)(const CUtensorMap, const CUtensorMap, const PrefillGemmArgs);
+using GemmKernel = void (*)(const CUtensorMap, const PrefillGemmArgs);
 
 GemmKernel pick_kernel(int ta, int tb) {
 #define BLK_K(A, B) if (ta == A && tb == B) return prefill_gemm_kernel<A, B>;
@@ -56,15 +56,15 @@ GemmKernel pick_kernel(int ta, int tb) {
     return nullptr;
 }
 
-// panel: nullptr for the fused (in-kernel dequantisation) form, else the bf16 panel [panel_rows][K] the B tiles are read from
-cudaError_t launch_gemm(PrefillGemmArgs& a, int ta, int tb, const __nv_bfloat16* X, cudaStream_t st, const __nv_bfloat16* panel = nullptr, long long panel_rows = 0,
+// panel: nullptr for the fused (in-kernel dequantisation) form, else the bf16 panel (panel_layout) the B tiles are read from
+cudaError_t launch_gemm(PrefillGemmArgs& a, int ta, int tb, const __nv_bfloat16* X, cudaStream_t st, const __nv_bfloat16* panel = nullptr,
                         const SplitKWs* sk = nullptr) {
     EncodeTiledFn enc = encode_tiled();
     if (!enc) return cudaErrorNotSupported;
     if (a.K % PG_BK || a.T <= 0 || a.n_tiles <= 0) return cudaErrorInvalidValue;
     GemmKernel kernel = panel ? pick_kernel(QT_PANEL, QT_PANEL) : pick_kernel(ta, tb);
     if (!kernel) return cudaErrorInvalidValue;
-    CUtensorMap tmap, tmap_w;
+    CUtensorMap tmap;
     const cuuint64_t gdim[2] = {(cuuint64_t)a.K, (cuuint64_t)a.T};
     const cuuint64_t gstride[1] = {(cuuint64_t)a.K * sizeof(__nv_bfloat16)};
     const cuuint32_t box[2] = {(cuuint32_t)PG_BK, 128u};
@@ -73,9 +73,7 @@ cudaError_t launch_gemm(PrefillGemmArgs& a, int ta, int tb, const __nv_bfloat16*
                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return cudaErrorInvalidValue;
-    tmap_w = tmap;
     a.panel = reinterpret_cast<const unsigned char*>(panel);      // tile images, fetched with plain bulk copies (no tensor map)
-    (void)panel_rows;
     int dev = 0, sms = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e != cudaSuccess) return e;
@@ -100,7 +98,7 @@ cudaError_t launch_gemm(PrefillGemmArgs& a, int ta, int tb, const __nv_bfloat16*
     }
     const int items = a.n_whole + (tiles - a.n_whole) * a.k_splits;
     const int grid = items < sms ? items : sms;
-    e = launch_chain(kernel, dim3((unsigned)grid), dim3(PG_THREADS), PG_SMEM_BYTES, st, tmap, tmap_w, a);
+    e = launch_chain(kernel, dim3((unsigned)grid), dim3(PG_THREADS), PG_SMEM_BYTES, st, tmap, a);
     if (e == cudaSuccess) e = cudaGetLastError();
     if (e != cudaSuccess || a.k_splits == 1) return e;
     if (sk && sk->defer && a.mode == PG_ACCUM && a.n_whole == 0 && a.nseg == 1 && a.seg[0].col0 == 0 && !a.seg[0].bias &&
@@ -130,103 +128,86 @@ cudaError_t panel_dequant(const QMat& W, __nv_bfloat16* panel, long long row0, c
     return cudaGetLastError();
 }
 bool panel_type_ok(int t) { return t == QT_Q4_K || t == QT_Q5_K || t == QT_Q6_K || t == QT_Q8_0; }
+
+// The bf16 panel layout of the two-pass form: part i's rows start at panel row row0[i] (if row0 is given); returns the rows the
+// panel holds.  The parts of one GEMM take whole 256-row tiles one after another.  A SwiGLU tile pairs 128 gate rows with the
+// matching 128 up rows, so there up starts at the first 128-aligned row after gate.
+long long panel_layout(const GemmPart* parts, int n_parts, bool swiglu, long long* row0 = nullptr) {
+    const int align = swiglu ? 128 : PG_BN;
+    long long rows = 0;
+    for (int i = 0; i < n_parts; i++) {
+        if (row0) row0[i] = rows;
+        rows += (long long)((parts[i].W->N + align - 1) / align) * align;
+    }
+    return rows;
+}
 } // namespace
 
 cudaError_t prefill_gemm(const QMat& W, const __nv_bfloat16* X, int T, float* C, long long ldc, const float* bias, int mode, cudaStream_t st,
-                         __nv_bfloat16* panel, bool panel_fill, const SplitKWs* sk) {
+                         const __nv_bfloat16* panel, const SplitKWs* sk) {
     PrefillGemmArgs a{};
     a.nseg = 1; a.seg[0] = {W, bias, 0, 0};
     a.C = C; a.ldc = ldc; a.T = T; a.K = W.K; a.mode = mode;
     a.n_tiles = (W.N + PG_BN - 1) / PG_BN;
-    if (panel && panel_type_ok(W.type) && W.K % 64 == 0) {
-        if (panel_fill) { cudaError_t e = panel_dequant(W, panel, 0, st); if (e != cudaSuccess) return e; }
-        return launch_gemm(a, W.type, W.type, X, st, panel, (long long)a.n_tiles * PG_BN, (W.N % 4 == 0 && ldc % 4 == 0) ? sk : nullptr);
-    }
-    return launch_gemm(a, W.type, W.type, X, st, nullptr, 0, (W.N % 4 == 0 && ldc % 4 == 0) ? sk : nullptr);
+    const bool use_panel = panel && panel_type_ok(W.type) && W.K % 64 == 0;
+    return launch_gemm(a, W.type, W.type, X, st, use_panel ? panel : nullptr, (W.N % 4 == 0 && ldc % 4 == 0) ? sk : nullptr);
 }
-// the dequantisation passes alone (same panel layout as the GEMM entry points above use), so that a caller can run them on a
-// second stream one GEMM ahead; false = this combination takes the fused form (the GEMM call must then get panel = nullptr)
-bool prefill_panel_fill(const GemmPart* parts, int n_parts, __nv_bfloat16* panel, cudaStream_t st, cudaError_t* err) {
+// the dequantisation passes alone, so that a caller can run them on a second stream one GEMM ahead; false = this combination takes
+// the fused form (the GEMM call must then get panel = nullptr)
+bool prefill_panel_fill(const GemmPart* parts, int n_parts, bool swiglu, __nv_bfloat16* panel, cudaStream_t st, cudaError_t* err) {
     *err = cudaSuccess;
-    if (!panel || n_parts < 1 || n_parts > 3) return false;
+    if (!panel || n_parts < 1 || n_parts > 3 || (swiglu && (n_parts != 2 || parts[1].W->type != parts[0].W->type))) return false;
     for (int i = 0; i < n_parts; i++) if (!panel_type_ok(parts[i].W->type) || parts[i].W->K != parts[0].W->K || parts[i].col0 % 4 || parts[i].W->K % 64) return false;
-    int tile0 = 0;
+    long long row0[3];
+    panel_layout(parts, n_parts, swiglu, row0);
     for (int i = 0; i < n_parts; i++) {
-        *err = panel_dequant(*parts[i].W, panel, (long long)tile0 * PG_BN, st);
+        *err = panel_dequant(*parts[i].W, panel, row0[i], st);
         if (*err != cudaSuccess) return true;
-        tile0 += (parts[i].W->N + PG_BN - 1) / PG_BN;
     }
     return true;
 }
-bool prefill_panel_fill_swiglu(const QMat& gate, const QMat& up, __nv_bfloat16* panel, cudaStream_t st, cudaError_t* err) {
-    *err = cudaSuccess;
-    if (!panel || gate.type != up.type || !panel_type_ok(gate.type) || gate.K % 64) return false;
-    const long long up0 = (long long)((gate.N + 127) / 128) * 128;
-    *err = panel_dequant(gate, panel, 0, st);
-    if (*err == cudaSuccess) *err = panel_dequant(up, panel, up0, st);
-    return true;
+size_t prefill_panel_elems(const GemmPart* parts, int n_parts, bool swiglu) {
+    return (size_t)panel_layout(parts, n_parts, swiglu) * (size_t)parts[0].W->K;
 }
-size_t prefill_panel_rows(int N) { return (size_t)((N + PG_BN - 1) / PG_BN) * PG_BN; }
 
 cudaError_t prefill_gemm_multi(const GemmPart* parts, int n_parts, const __nv_bfloat16* X, int T, float* C, long long ldc, cudaStream_t st,
-                               __nv_bfloat16* panel, bool panel_fill, const SplitKWs* sk) {
+                               const __nv_bfloat16* panel, const SplitKWs* sk) {
     bool all_panel = panel != nullptr && n_parts >= 1 && n_parts <= 3;
     for (int i = 0; i < n_parts && all_panel; i++) all_panel = panel_type_ok(parts[i].W->type) && parts[i].W->K == parts[0].W->K && parts[i].col0 % 4 == 0;
     bool fuse = n_parts >= 2 && n_parts <= 3 && parts[0].W->type == parts[1].W->type;
     for (int i = 0; i < n_parts && fuse; i++) fuse = (parts[i].col0 % 4 == 0) && parts[i].W->K == parts[0].W->K;
     if (fuse && n_parts == 3 && !pick_kernel(parts[0].W->type, parts[2].W->type)) fuse = false;
-    if (all_panel) {      // any mix of weight types: every segment is dequantised to its tile-aligned rows of the panel
-        PrefillGemmArgs a{};
-        a.nseg = n_parts; a.C = C; a.ldc = ldc; a.T = T; a.K = parts[0].W->K; a.mode = PG_STORE;
-        int tile0 = 0;
+    if (!all_panel && !fuse) {
         for (int i = 0; i < n_parts; i++) {
-            a.seg[i] = {*parts[i].W, parts[i].bias, parts[i].col0, tile0};
-            if (panel_fill) { cudaError_t e = panel_dequant(*parts[i].W, panel, (long long)tile0 * PG_BN, st); if (e != cudaSuccess) return e; }
-            tile0 += (parts[i].W->N + PG_BN - 1) / PG_BN;
-        }
-        a.n_tiles = tile0;
-        bool sk_ok = ldc % 4 == 0;
-        for (int i = 0; i < n_parts; i++) sk_ok = sk_ok && parts[i].W->N % 4 == 0;
-        return launch_gemm(a, QT_PANEL, QT_PANEL, X, st, panel, (long long)tile0 * PG_BN, sk_ok ? sk : nullptr);
-    }
-    if (!fuse) {
-        for (int i = 0; i < n_parts; i++) {
-            cudaError_t e = prefill_gemm(*parts[i].W, X, T, C + parts[i].col0, ldc, parts[i].bias, 0, st, nullptr, false, nullptr);     // (column-offset C: no split-K)
+            cudaError_t e = prefill_gemm(*parts[i].W, X, T, C + parts[i].col0, ldc, parts[i].bias, 0, st, nullptr, nullptr);     // (column-offset C: no split-K)
             if (e != cudaSuccess) return e;
         }
         return cudaSuccess;
     }
+    // one launch over every segment; the panel form takes any mix of weight types (each segment is dequantised to its own rows)
     PrefillGemmArgs a{};
     a.nseg = n_parts; a.C = C; a.ldc = ldc; a.T = T; a.K = parts[0].W->K; a.mode = PG_STORE;
-    int tile0 = 0;
-    for (int i = 0; i < n_parts; i++) {
-        a.seg[i] = {*parts[i].W, parts[i].bias, parts[i].col0, tile0};
-        tile0 += (parts[i].W->N + PG_BN - 1) / PG_BN;
-    }
-    a.n_tiles = tile0;
+    long long row0[3];
+    a.n_tiles = (int)(panel_layout(parts, n_parts, false, row0) / PG_BN);
+    for (int i = 0; i < n_parts; i++) a.seg[i] = {*parts[i].W, parts[i].bias, parts[i].col0, (int)(row0[i] / PG_BN)};
     bool sk_ok = ldc % 4 == 0;
     for (int i = 0; i < n_parts; i++) sk_ok = sk_ok && parts[i].W->N % 4 == 0;
-    return launch_gemm(a, parts[0].W->type, n_parts == 3 ? parts[2].W->type : parts[0].W->type, X, st, nullptr, 0, sk_ok ? sk : nullptr);
+    return launch_gemm(a, parts[0].W->type, n_parts == 3 ? parts[2].W->type : parts[0].W->type, X, st, all_panel ? panel : nullptr, sk_ok ? sk : nullptr);
 }
 
 cudaError_t prefill_gemm_swiglu(const QMat& gate, const QMat& up, const __nv_bfloat16* X, int T, __nv_bfloat16* H, long long ldh, cudaStream_t st,
-                                __nv_bfloat16* panel, bool panel_fill, const SplitKWs* sk) {
+                                const __nv_bfloat16* panel, const SplitKWs* sk) {
     if (gate.type != up.type || gate.N != up.N || gate.K != up.K || ldh % 8) return cudaErrorInvalidValue;
     PrefillGemmArgs a{};
     a.nseg = 2; a.seg[0] = {gate, nullptr, 0, 0}; a.seg[1] = {up, nullptr, 0, 0};
     a.H = H; a.ldh = ldh; a.T = T; a.K = gate.K; a.mode = PG_SWIGLU;
     a.n_tiles = (gate.N + 127) / 128;
-    if (panel && panel_type_ok(gate.type) && gate.K % 64 == 0) {
-        a.panel_up_row0 = a.n_tiles * 128;                         // gate rows, then (tile-aligned) the up rows
-        if (panel_fill) {
-            cudaError_t e = panel_dequant(gate, panel, 0, st);
-            if (e != cudaSuccess) return e;
-            e = panel_dequant(up, panel, a.panel_up_row0, st);
-            if (e != cudaSuccess) return e;
-        }
-        return launch_gemm(a, gate.type, gate.type, X, st, panel, 2LL * a.panel_up_row0, sk);
-    }
-    return launch_gemm(a, gate.type, gate.type, X, st, nullptr, 0, sk);
+    if (!(panel && panel_type_ok(gate.type) && gate.K % 64 == 0)) return launch_gemm(a, gate.type, gate.type, X, st, nullptr, sk);
+    const GemmPart parts[2] = {{&gate, nullptr, 0}, {&up, nullptr, 0}};
+    long long row0[2];
+    panel_layout(parts, 2, true, row0);
+    a.panel_up_row0 = (int)row0[1];
+    return launch_gemm(a, gate.type, gate.type, X, st, panel, sk);
 }
 
 namespace {

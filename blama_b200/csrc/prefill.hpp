@@ -10,8 +10,8 @@ namespace blk {
 
 // C[T][N] (f32, row stride ldc) = or += X[T][K] (bf16, row-major, device) . W^T  through the tcgen05 GEMM
 // mode: 0 store (+bias), 1 accumulate into C.  Returns a CUDA error (cudaErrorNotSupported if the driver lacks TMA).
-// panel != nullptr selects the two-pass form: W is dequantised once into the bf16 panel (panel_fill) and the GEMM reads its B
-// tiles from there by TMA -- for many-token batches, where the fused form would dequantise every weight tile T / 256 times.
+// panel != nullptr selects the two-pass form: W was dequantised once into the bf16 panel (prefill_panel_fill) and the GEMM reads
+// its B tiles from there -- for many-token batches, where the fused form would dequantise every weight tile T / 256 times.
 // sk != nullptr: workspace for the deterministic split-K of the last, partial wave of tiles (all tiles when the batch has fewer
 // tiles than SMs); n_sm * 65536 floats always suffice (split tiles * splits never exceeds the SM count)
 // a split-K ACCUMULATE (C += X W^T over the residual stream, every tile split) whose partial sums are still in the workspace: the RMSNorm
@@ -19,23 +19,23 @@ namespace blk {
 struct PendingReduce { const float* ws = nullptr; int S = 0, m_tiles = 0; };
 struct SplitKWs { float* ws; size_t elems; PendingReduce* defer = nullptr; };
 cudaError_t prefill_gemm(const QMat& W, const __nv_bfloat16* X, int T, float* C, long long ldc, const float* bias, int mode, cudaStream_t st,
-                         __nv_bfloat16* panel = nullptr, bool panel_fill = true, const SplitKWs* sk = nullptr);
-// rows a matrix of N rows occupies in a panel (tile aligned)
-size_t prefill_panel_rows(int N);
+                         const __nv_bfloat16* panel = nullptr, const SplitKWs* sk = nullptr);
 
 // several matrices with the same K in one launch: C[:, col0_s : col0_s + N_s] = X . W_s^T (+bias_s).  Matrices 0 and 1 must share
 // a weight type.  Falls back to one launch per matrix when a column offset is not 4-element aligned.
 struct GemmPart { const QMat* W; const float* bias; int col0; };
 cudaError_t prefill_gemm_multi(const GemmPart* parts, int n_parts, const __nv_bfloat16* X, int T, float* C, long long ldc, cudaStream_t st,
-                               __nv_bfloat16* panel = nullptr, bool panel_fill = true, const SplitKWs* sk = nullptr);
+                               const __nv_bfloat16* panel = nullptr, const SplitKWs* sk = nullptr);
 
 // H[T][ff] (bf16) = silu(X . Wgate^T) * (X . Wup^T), one launch, SwiGLU in the GEMM epilogue
 cudaError_t prefill_gemm_swiglu(const QMat& gate, const QMat& up, const __nv_bfloat16* X, int T, __nv_bfloat16* H, long long ldh, cudaStream_t st,
-                                __nv_bfloat16* panel = nullptr, bool panel_fill = true, const SplitKWs* sk = nullptr);
-// The dequantisation passes alone (same panel layout), so that a caller can run them on a second stream one GEMM ahead.
+                                const __nv_bfloat16* panel = nullptr, const SplitKWs* sk = nullptr);
+// The dequantisation passes of the two-pass form: the panel of one GEMM over parts (prefill_gemm, prefill_gemm_multi), or with
+// swiglu = true over {gate, up} (prefill_gemm_swiglu).  A caller can run them on a second stream one GEMM ahead.
 // Return false when the combination takes the fused form (the GEMM call must then get panel = nullptr).
-bool prefill_panel_fill(const GemmPart* parts, int n_parts, __nv_bfloat16* panel, cudaStream_t st, cudaError_t* err);
-bool prefill_panel_fill_swiglu(const QMat& gate, const QMat& up, __nv_bfloat16* panel, cudaStream_t st, cudaError_t* err);
+bool prefill_panel_fill(const GemmPart* parts, int n_parts, bool swiglu, __nv_bfloat16* panel, cudaStream_t st, cudaError_t* err);
+// bf16 elements of that panel
+size_t prefill_panel_elems(const GemmPart* parts, int n_parts, bool swiglu);
 
 // Causal attention of a prefill chunk on tcgen05 (prefill_attn_tc.cuh): d_head = 128, GQA ratio 1 .. 8.
 //   q [T][n_head*128] f16 (post-RoPE), paged f16 K / V pools of the layer, out [T][n_head*128] bf16;

@@ -339,7 +339,7 @@ __device__ __forceinline__ PgItem pg_item(int item, int n_whole, int n_split, in
 }
 
 template <int TA, int TB>
-__global__ void __launch_bounds__(PG_THREADS, 1) prefill_gemm_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__ CUtensorMap tmap_w, const PrefillGemmArgs a) {
+__global__ void __launch_bounds__(PG_THREADS, 1) prefill_gemm_kernel(const __grid_constant__ CUtensorMap tmap_x, const PrefillGemmArgs a) {
     constexpr bool PANEL = (TA == QT_PANEL);
     // The tiles need 1024-byte alignment (SWIZZLE_128B atoms).  The dynamic shared memory of a kernel without static shared memory
     // starts 1024-aligned on this part; it is checked, not assumed, and NOT re-aligned through an integer cast -- that hides the

@@ -149,20 +149,6 @@ __global__ void __launch_bounds__(256) qkv_post_kernel(const QkvPostArgs a) {
     qkv_post_row(a, blockIdx.x, a.pos0[0] + (int)blockIdx.x, a.k_pool, a.v_pool, a.page_table);
 }
 
-// ---- SwiGLU: h = silu(g) * u -> bf16 ------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) swiglu_bf16_kernel(const float* __restrict__ g, const float* __restrict__ u, size_t n, __nv_bfloat16* __restrict__ h) {
-    const size_t i = ((size_t)blockIdx.x * 256 + threadIdx.x) * 4;
-    if (i + 3 < n) {
-        const float4 a = *reinterpret_cast<const float4*>(g + i), b = *reinterpret_cast<const float4*>(u + i);
-        __nv_bfloat162 p0 = __floats2bfloat162_rn((a.x / (1.0f + expf(-a.x))) * b.x, (a.y / (1.0f + expf(-a.y))) * b.y);
-        __nv_bfloat162 p1 = __floats2bfloat162_rn((a.z / (1.0f + expf(-a.z))) * b.z, (a.w / (1.0f + expf(-a.w))) * b.w);
-        uint2 o; o.x = *reinterpret_cast<uint32_t*>(&p0); o.y = *reinterpret_cast<uint32_t*>(&p1);
-        *reinterpret_cast<uint2*>(h + i) = o;
-    } else {
-        for (size_t j = i; j < n; j++) h[j] = __float2bfloat16_rn((g[j] / (1.0f + expf(-g[j]))) * u[j]);
-    }
-}
-
 // ---- causal flash attention over the paged KV cache (mma.sync m16n8k16 f16, f32 accumulate) -------------------------------------
 // grid = (ceil(T/64), n_head); block = 128 (4 warps x 16 query rows).  Keys 0 .. pos0+T-1 (the chunk's own K/V are already
 // in the cache).  Output bf16 [T][n_head*DH].

@@ -111,3 +111,16 @@ def test_prefill_attention(n_head, n_head_kv, d_head, T, pos0, scores):
     # bf16 output (half ulp 2^-9 of the value) + f16 probabilities (2^-11 each, averaged over the row): bounded by 1e-3 of the row's
     # largest value beside the output rounding
     assert np.all(err <= BF16_ULP * 0.51 * np.abs(ref) + 1e-3 * scale), rel
+
+
+def test_prefill_attention_rejects_a_shape_without_a_kernel():
+    """d_head 128 runs only on the tcgen05 kernel, which covers GQA ratios up to 8: a ratio of 16 is an argument error, not a launch."""
+    from blama_b200 import capi
+
+    capi.init()
+    T = 16
+    q = np.zeros((T, 16 * 128), dtype=np.float32)
+    kv = np.zeros((T, 128), dtype=np.float32)
+    with pytest.raises(capi.BlkError) as e:
+        capi.test_prefill_attn(q, kv, kv, 0, 16, 1, 128)
+    assert e.value.code == 4      # BLK_ERR_ARG
