@@ -89,6 +89,8 @@ SYMBOLS = {
     "blk_test_rmsnorm": (_i32, [_i32, _vp, _vp, _i32, _i32, C.c_float, _vp]),
     "blk_test_qkv_post": (_i32, [_i32, _vp, _i32, _i32, _i32, _i32, _i32, _i32, C.c_float, _vp, _vp, _vp, _vp]),
     "blk_test_prefill_attn": (_i32, [_i32, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp, C.POINTER(_i32)]),
+    "blk_test_decode_attn": (_i32, [_i32, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i64, _vp, C.POINTER(_i32)]),
+    "blk_test_decode_attn_batch": (_i32, [_i32, _i32, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i64, _vp]),
 }
 
 _lib: Optional[C.CDLL] = None
@@ -154,7 +156,33 @@ def test_prefill_attn(q: np.ndarray, k: np.ndarray, v: np.ndarray, pos0: int, n_
     return out, bool(tc.value)
 
 
+def test_decode_attn(q: np.ndarray, k: np.ndarray, v: np.ndarray, n_ctx: int, n_head: int, n_head_kv: int, d_head: int, form: int = -1,
+                     seed: int = 0, device: int = 0):
+    """Decode attention of q [n_head*d_head] over the n_kv = len(k) cells of a context of n_ctx cells.  form: -1 the engine's plan,
+    0 the split form, 1 the cluster form.  Returns (out [n_head*d_head] f32, True when the cluster form ran)."""
+    q = np.ascontiguousarray(q, dtype=np.float32).reshape(-1)
+    k = np.ascontiguousarray(k, dtype=np.float32); v = np.ascontiguousarray(v, dtype=np.float32)
+    out = np.zeros_like(q)
+    used = _i32(-1)
+    _check(lib().blk_test_decode_attn(device, _p(q), _p(k), _p(v), k.shape[0], n_ctx, n_head, n_head_kv, d_head, form, seed, _p(out), C.byref(used)))
+    return out, bool(used.value)
+
+
+def test_decode_attn_batch(q: np.ndarray, k: np.ndarray, v: np.ndarray, n_kv: Sequence[int], n_head: int, n_head_kv: int, d_head: int,
+                           seed: int = 0, device: int = 0) -> np.ndarray:
+    """Batched decode attention: row b of q [n][n_head*d_head] over its own n_kv[b] cells, whose keys / values are rows
+    sum(n_kv[:b]) .. of k / v.  Returns the bf16 output [n][n_head*d_head] as f32."""
+    q = np.ascontiguousarray(q, dtype=np.float32)
+    k = np.ascontiguousarray(k, dtype=np.float32); v = np.ascontiguousarray(v, dtype=np.float32)
+    nk = np.ascontiguousarray(n_kv, dtype=np.int32)
+    assert q.shape[0] == nk.shape[0] and k.shape[0] == v.shape[0] == int(nk.sum())
+    out = np.zeros_like(q)
+    _check(lib().blk_test_decode_attn_batch(device, q.shape[0], _p(q), _p(k), _p(v), _p(nk), n_head, n_head_kv, d_head, seed, _p(out)))
+    return out
+
+
 test_rmsnorm.__test__ = test_qkv_post.__test__ = test_prefill_attn.__test__ = False      # (not pytest tests)
+test_decode_attn.__test__ = test_decode_attn_batch.__test__ = False
 
 
 def decode_batch(ws: "Ctx", ctxs: Sequence["Ctx"], tokens: Sequence[int], k: int = 40) -> np.ndarray:

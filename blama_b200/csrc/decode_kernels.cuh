@@ -266,6 +266,7 @@ struct AttnClusterArgs {
 };
 
 constexpr int ATTN_THREADS = 512;
+constexpr int ATTN_CLUSTER_PAGES = 512;      // KV pages one CTA's token slice may span (s_page below)
 
 template <int DH, int GQ>      // GQ = compile-time bound on query heads per KV head (4 or 8)
 __global__ void __launch_bounds__(ATTN_THREADS) attn_cluster_kernel(const AttnClusterArgs a) {
@@ -281,7 +282,10 @@ __global__ void __launch_bounds__(ATTN_THREADS) attn_cluster_kernel(const AttnCl
     __shared__ float s_M[GQ], s_inv[GQ];
     __shared__ float red_f[GQ][NW];
     __shared__ double red_d[GQ][NW];
-    __shared__ int s_page[512];
+    // The slice's physical page numbers.  Nothing here checks the slice length: the host plan (plan_decode_attn in engine.cu) picks
+    // this kernel only when cap tokens starting anywhere inside a page span at most ATTN_CLUSTER_PAGES pages, i.e.
+    // cap <= (ATTN_CLUSTER_PAGES - 1) * KV_PAGE + 1.  Longer slices (MHA models at contexts above ~262k cells) take the split form.
+    __shared__ int s_page[ATTN_CLUSTER_PAGES];
 
     const int CS = (int)cluster.num_blocks(), r = (int)cluster.block_rank();
     const int hk = blockIdx.x / CS, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
@@ -295,7 +299,7 @@ __global__ void __launch_bounds__(ATTN_THREADS) attn_cluster_kernel(const AttnCl
     // physical pages of this CTA's token slice (removes a dependent global load from every K / V row address)
     const int pg0 = t0 / KV_PAGE;
     const int npg = nt > 0 ? (t1 - 1) / KV_PAGE - pg0 + 1 : 0;
-    for (int i = tid; i < npg && i < 512; i += ATTN_THREADS) s_page[i] = a.page_table[pg0 + i];
+    for (int i = tid; i < npg && i < ATTN_CLUSTER_PAGES; i += ATTN_THREADS) s_page[i] = a.page_table[pg0 + i];
     __syncthreads();
     auto row_off = [&](int t) -> size_t { return ((size_t)s_page[t / KV_PAGE - pg0] * KV_PAGE + (t % KV_PAGE)) * a.kv_dim + (size_t)hk * DH; };
 

@@ -16,6 +16,7 @@
 #include <cstdio>
 #include <cstring>
 #include <mutex>
+#include <random>
 #include <tuple>
 
 using namespace blk;
@@ -612,6 +613,72 @@ TopkArgs own_topk_args(const blk_ctx* c) {
     return tk;
 }
 
+// The per-op decode attention form of a context of c->n_pages KV pages (decode_kernels.cuh): the single-kernel cluster form when
+// one CTA's share of the scores fits in shared memory and its token slice spans at most ATTN_CLUSTER_PAGES pages, else the
+// three-kernel split form.  A slice of cap tokens starting anywhere inside a page spans at most (cap + KV_PAGE - 2) / KV_PAGE + 1
+// pages, hence the bound on cap.  form: -1 = that rule, 0 = the split form, 1 = the cluster form (BLK_ERR_ARG when the rule does
+// not allow it).  Sets attn_cluster, attn_cap, n_split and the cluster kernels' shared-memory attribute.
+void plan_decode_attn(blk_ctx* c, int form = -1) {
+    const blk_model* m = c->m;
+    const int gq = m->n_head / m->n_head_kv;
+    const int cs = 8;
+    c->attn_cap = (c->n_pages * KV_PAGE + cs - 1) / cs;
+    const size_t smem = (size_t)gq * (c->attn_cap + (ATTN_THREADS / 32) * m->d_head) * sizeof(float);
+    const bool fits = smem <= 160 * 1024 && c->attn_cap <= (ATTN_CLUSTER_PAGES - 1) * KV_PAGE + 1;
+    if (form == 1 && !fits) throw BlkError(BLK_ERR_ARG, "the cluster attention form does not cover this context");
+    c->attn_cluster = (form == -1 ? fits : form == 1) ? cs : 0;
+    if (c->attn_cluster) {
+        BLK_CUDA(cudaFuncSetAttribute(attn_cluster_kernel<128, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 164 * 1024));
+        BLK_CUDA(cudaFuncSetAttribute(attn_cluster_kernel<128, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 164 * 1024));
+        BLK_CUDA(cudaFuncSetAttribute(attn_cluster_kernel<64, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 164 * 1024));
+        BLK_CUDA(cudaFuncSetAttribute(attn_cluster_kernel<64, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 164 * 1024));
+    }
+    c->n_split = std::max(1, std::min(32, (2 * 148) / m->n_head_kv));
+}
+
+// decode attention of layer l (c->qbuf over the cache at c->d_pos -> c->act_q.f32) in the form plan_decode_attn chose
+void launch_decode_attn(blk_ctx* c, int l) {
+    const blk_model* m = c->m;
+    const int dh = m->d_head, dq = m->n_head * dh, dkv = m->n_head_kv * dh;
+    if (c->attn_cluster > 0) {
+        AttnClusterArgs ac{};
+        ac.q = c->qbuf; ac.k_pool = c->k_pool[l]; ac.v_pool = c->v_pool[l]; ac.page_table = c->page_table; ac.pos = c->d_pos;
+        ac.n_head = m->n_head; ac.n_head_kv = m->n_head_kv; ac.kv_dim = dkv; ac.cap = c->attn_cap;
+        ac.scale = 1.0f / sqrtf((float)dh); ac.out = c->act_q.f32;
+        const size_t smem = (size_t)(m->n_head / m->n_head_kv) * (c->attn_cap + (ATTN_THREADS / 32) * dh) * sizeof(float);
+        const dim3 grid(m->n_head_kv * c->attn_cluster), block(ATTN_THREADS);
+        const bool g4 = (m->n_head / m->n_head_kv) <= 4;
+        if (dh == 128 && g4) BLK_CUDA(launch_pdl_cluster(attn_cluster_kernel<128, 4>, grid, block, smem, c->attn_cluster, c->stream, ac));
+        else if (dh == 128) BLK_CUDA(launch_pdl_cluster(attn_cluster_kernel<128, 8>, grid, block, smem, c->attn_cluster, c->stream, ac));
+        else if (g4) BLK_CUDA(launch_pdl_cluster(attn_cluster_kernel<64, 4>, grid, block, smem, c->attn_cluster, c->stream, ac));
+        else BLK_CUDA(launch_pdl_cluster(attn_cluster_kernel<64, 8>, grid, block, smem, c->attn_cluster, c->stream, ac));
+        c->launches++;
+        prof_mark(c, "attn_cluster");
+        return;
+    }
+    AttnArgs at{};
+    at.q = c->qbuf; at.k_pool = c->k_pool[l]; at.v_pool = c->v_pool[l]; at.page_table = c->page_table; at.pos = c->d_pos;
+    at.n_head = m->n_head; at.n_head_kv = m->n_head_kv; at.d_head = dh; at.kv_dim = dkv; at.n_split = c->n_split;
+    at.scale = 1.0f / sqrtf((float)dh); at.scores = c->scores; at.score_stride = c->n_pages * KV_PAGE; at.part_o = c->part_o;
+    dim3 grid(m->n_head_kv, c->n_split);
+    if (dh == 128) {
+        BLK_CUDA(launch_pdl(attn_scores_kernel<128>, grid, dim3(128), 0, c->stream, at));
+        prof_mark(c, "attn_scores");
+        BLK_CUDA(launch_pdl(attn_pv_kernel<128>, grid, dim3(128), 0, c->stream, at));
+        prof_mark(c, "attn_pv");
+    } else {
+        BLK_CUDA(launch_pdl(attn_scores_kernel<64>, grid, dim3(64), 0, c->stream, at));
+        prof_mark(c, "attn_scores");
+        BLK_CUDA(launch_pdl(attn_pv_kernel<64>, grid, dim3(64), 0, c->stream, at));
+        prof_mark(c, "attn_pv");
+    }
+    c->launches += 2;
+    // one CTA per 256 outputs: model widths are multiples of 256; blk_test_decode_attn pads part_o / act_q for narrower shapes
+    BLK_CUDA(launch_pdl(attn_combine_kernel, dim3((dq + 255) / 256), dim3(256), 0, c->stream, c->part_o, dh, c->n_split, (int)ACT_F32, c->act_q));
+    c->launches++;
+    prof_mark(c, "attn_combine");
+}
+
 // one decode step on c->stream: token id in c->d_tok, position in c->d_pos.
 // Per layer: QKV mat-vec (RMSNorm prologue; +bias, RoPE, KV-page write) | attention | Wo mat-vec (+residual) |
 // gate/up mat-vec (RMSNorm prologue; SwiGLU) | down mat-vec (+residual); then final norm + lm_head mat-vec + top-k.
@@ -658,44 +725,7 @@ void enqueue_step(blk_ctx* c, bool with_head, bool feedback = false) {
             a.k_pool = c->k_pool[l]; a.v_pool = c->v_pool[l]; a.page_table = c->page_table; a.kv_dim = dkv;
             matvec<EPI_QKV>(c, a, c->x, L.attn_norm, c->act_d, "gemv_qkv");
         }
-        {
-            if (c->attn_cluster > 0) {
-                AttnClusterArgs ac{};
-                ac.q = c->qbuf; ac.k_pool = c->k_pool[l]; ac.v_pool = c->v_pool[l]; ac.page_table = c->page_table; ac.pos = c->d_pos;
-                ac.n_head = m->n_head; ac.n_head_kv = m->n_head_kv; ac.kv_dim = dkv; ac.cap = c->attn_cap;
-                ac.scale = 1.0f / sqrtf((float)dh); ac.out = c->act_q.f32;
-                const size_t smem = (size_t)(m->n_head / m->n_head_kv) * (c->attn_cap + (ATTN_THREADS / 32) * dh) * sizeof(float);
-                const dim3 grid(m->n_head_kv * c->attn_cluster), block(ATTN_THREADS);
-                const bool g4 = (m->n_head / m->n_head_kv) <= 4;
-                if (dh == 128 && g4) BLK_CUDA(launch_pdl_cluster(attn_cluster_kernel<128, 4>, grid, block, smem, c->attn_cluster, c->stream, ac));
-                else if (dh == 128) BLK_CUDA(launch_pdl_cluster(attn_cluster_kernel<128, 8>, grid, block, smem, c->attn_cluster, c->stream, ac));
-                else if (g4) BLK_CUDA(launch_pdl_cluster(attn_cluster_kernel<64, 4>, grid, block, smem, c->attn_cluster, c->stream, ac));
-                else BLK_CUDA(launch_pdl_cluster(attn_cluster_kernel<64, 8>, grid, block, smem, c->attn_cluster, c->stream, ac));
-                c->launches++;
-                prof_mark(c, "attn_cluster");
-            } else {
-            AttnArgs at{};
-            at.q = c->qbuf; at.k_pool = c->k_pool[l]; at.v_pool = c->v_pool[l]; at.page_table = c->page_table; at.pos = c->d_pos;
-            at.n_head = m->n_head; at.n_head_kv = m->n_head_kv; at.d_head = dh; at.kv_dim = dkv; at.n_split = c->n_split;
-            at.scale = 1.0f / sqrtf((float)dh); at.scores = c->scores; at.score_stride = c->n_pages * KV_PAGE; at.part_o = c->part_o;
-            dim3 grid(m->n_head_kv, c->n_split);
-            if (dh == 128) {
-                BLK_CUDA(launch_pdl(attn_scores_kernel<128>, grid, dim3(128), 0, c->stream, at));
-                prof_mark(c, "attn_scores");
-                BLK_CUDA(launch_pdl(attn_pv_kernel<128>, grid, dim3(128), 0, c->stream, at));
-                prof_mark(c, "attn_pv");
-            } else {
-                BLK_CUDA(launch_pdl(attn_scores_kernel<64>, grid, dim3(64), 0, c->stream, at));
-                prof_mark(c, "attn_scores");
-                BLK_CUDA(launch_pdl(attn_pv_kernel<64>, grid, dim3(64), 0, c->stream, at));
-                prof_mark(c, "attn_pv");
-            }
-            c->launches += 2;
-            BLK_CUDA(launch_pdl(attn_combine_kernel, dim3(dq / 256), dim3(256), 0, c->stream, c->part_o, dh, c->n_split, (int)ACT_F32, c->act_q));
-            c->launches++;
-            prof_mark(c, "attn_combine");
-            }
-        }
+        launch_decode_attn(c, l);
         {
             GemvArgs a{};
             a.nseg = 1; a.seg[0] = {L.wo, nullptr, 0, 0}; a.total_pairs = d / 2; a.out = c->x;
@@ -1284,20 +1314,7 @@ extern "C" blk_ctx* blk_ctx_create(blk_model* m, int32_t n_ctx, int32_t n_batch)
         c->x = dalloc<float>(c.get(), d); c->qbuf = dalloc<float>(c.get(), dq); c->hbuf = dalloc<float>(c.get(), ff);
         c->rope_cs = dalloc<float2>(c.get(), dh / 2);
         c->act_d = make_act(c.get(), d); c->act_q = make_act(c.get(), dq); c->act_q2 = make_act(c.get(), dq); c->act_ff = make_act(c.get(), ff);
-        {   // single-kernel cluster attention when one CTA's share of the scores fits in shared memory
-            const int gq = m->n_head / m->n_head_kv;
-            c->attn_cluster = 8;
-            c->attn_cap = (c->n_pages * KV_PAGE + c->attn_cluster - 1) / c->attn_cluster;
-            const size_t smem = (size_t)gq * (c->attn_cap + (ATTN_THREADS / 32) * m->d_head) * sizeof(float);
-            if (smem > 160 * 1024) c->attn_cluster = 0;
-            else {
-                BLK_CUDA(cudaFuncSetAttribute(attn_cluster_kernel<128, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 164 * 1024));
-                BLK_CUDA(cudaFuncSetAttribute(attn_cluster_kernel<128, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 164 * 1024));
-                BLK_CUDA(cudaFuncSetAttribute(attn_cluster_kernel<64, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 164 * 1024));
-                BLK_CUDA(cudaFuncSetAttribute(attn_cluster_kernel<64, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 164 * 1024));
-            }
-        }
-        c->n_split = std::max(1, std::min(32, (2 * 148) / m->n_head_kv));
+        plan_decode_attn(c.get());
         c->part_o = dalloc<float>(c.get(), (size_t)m->n_head * c->n_split * dh);
         c->scores = dalloc<float>(c.get(), (size_t)m->n_head * c->n_pages * KV_PAGE);
         c->logits = dalloc<float>(c.get(), m->n_vocab);
@@ -2052,6 +2069,30 @@ __global__ void rope_rows_kernel(float2* rope_cs, int half_rot, int pos0, float 
     rope_table_fill(rope_cs + (size_t)blockIdx.x * half_rot, half_rot, pos0 + (int)blockIdx.x, theta_scale, ff);
 }
 unsigned grid_of(size_t n) { return (unsigned)((n + 255) / 256); }
+// rows [n][dkv] f32 -> f16 cache cells 0 .. n - 1 of a paged pool, through the page table
+__global__ void scatter_cells_kernel(const float* x, __half* pool, const int32_t* page_table, int n, int dkv) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)n * dkv) return;
+    const int t = (int)(i / dkv), e = (int)(i % dkv);
+    pool[((size_t)page_table[t / KV_PAGE] * KV_PAGE + (t % KV_PAGE)) * dkv + e] = __float2half_rn(x[i]);
+}
+// A page table of n_pages entries over a pool of about 1.5 times as many pages: the first n_pages of a seeded random permutation.
+// Returns the pool size in pages.
+int random_page_table(std::mt19937_64& rng, int n_pages, std::vector<int32_t>& pt) {
+    const int pool_pages = n_pages + n_pages / 2 + 1;
+    std::vector<int32_t> perm(pool_pages);
+    for (int i = 0; i < pool_pages; i++) perm[i] = i;
+    std::shuffle(perm.begin(), perm.end(), rng);
+    pt.assign(perm.begin(), perm.begin() + n_pages);
+    return pool_pages;
+}
+// Fill a pool with f16 NaN (0xffff), then write rows [n][dkv] into cells 0 .. n - 1 through the table: a read through the wrong
+// page, of a cell past n, or of the wrong pool gives NaN.
+void fill_pool(__half* pool, size_t pool_elems, const float* staging, const int32_t* d_pt, int n, int dkv, cudaStream_t st) {
+    BLK_CUDA(cudaMemsetAsync(pool, 0xff, pool_elems * sizeof(__half), st));
+    scatter_cells_kernel<<<grid_of((size_t)n * dkv), 256, 0, st>>>(staging, pool, d_pt, n, dkv);
+    BLK_CUDA(cudaGetLastError());
+}
 } // namespace
 
 // y[t][:] = bf16(rms_norm(x[t][:]) * w) through rmsnorm_bf16_kernel; out as f32 (exactly the bf16 values)
@@ -2162,5 +2203,134 @@ extern "C" blk_status blk_test_prefill_attn(int32_t device, const float* q, cons
         BLK_CUDA(cudaMemcpyAsync(out, fo, (size_t)T * dq * 4, cudaMemcpyDeviceToHost, c.stream));
         BLK_CUDA(cudaStreamSynchronize(c.stream));
         if (used_tc) *used_tc = tc ? 1 : 0;
+    });
+}
+
+// Decode attention of one query row q [n_head*dh] (f32, the kernels round it to f16) over the cache cells 0 .. n_kv - 1 of a context of
+// n_ctx cells, through plan_decode_attn / launch_decode_attn: k / v [n_kv][n_head_kv*dh] are rounded to f16 into a NaN-filled pool
+// behind a seeded random page table.  form: -1 = the plan's choice, 0 / 1 = force the split / cluster form (BLK_ERR_ARG, without a
+// launch, when the plan does not allow the cluster form).  out [n_head*dh] f32; *used_form = 1 when the cluster form ran.
+extern "C" blk_status blk_test_decode_attn(int32_t device, const float* q, const float* k, const float* v, int32_t n_kv, int32_t n_ctx,
+                                           int32_t n_head, int32_t n_head_kv, int32_t d_head, int32_t form, int64_t seed, float* out,
+                                           int32_t* used_form) {
+    return guarded([&] {
+        if (blk_init() != BLK_OK) throw BlkError(BLK_ERR_NO_DEVICE, g_last_error);
+        if (n_kv <= 0 || n_ctx < n_kv || (d_head != 64 && d_head != 128) || n_head <= 0 || n_head_kv <= 0 || n_head % n_head_kv ||
+            n_head / n_head_kv > MAX_GQ || form < -1 || form > 1)
+            throw BlkError(BLK_ERR_ARG, "blk_test_decode_attn: bad shape");
+        BLK_CUDA(cudaSetDevice(device));
+        const int dq = n_head * d_head, dkv = n_head_kv * d_head;
+        const int dq_pad = (dq + 255) / 256 * 256;          // attn_combine_kernel writes whole 256-output blocks
+        blk_model mm; mm.device = device; mm.n_head = n_head; mm.n_head_kv = n_head_kv; mm.d_head = d_head;
+        blk_ctx c; c.m = &mm;
+        c.n_ctx = n_ctx; c.n_pages = (n_ctx + KV_PAGE - 1) / KV_PAGE;
+        plan_decode_attn(&c, form);
+        BLK_CUDA(cudaStreamCreateWithFlags(&c.stream, cudaStreamNonBlocking));
+        std::mt19937_64 rng((uint64_t)seed);
+        std::vector<int32_t> hpt;
+        const int pool_pages = random_page_table(rng, c.n_pages, hpt);
+        const size_t pool = (size_t)pool_pages * KV_PAGE * dkv;
+        c.k_pool = {dalloc<__half>(&c, pool)}; c.v_pool = {dalloc<__half>(&c, pool)};
+        c.page_table = dalloc<int32_t>(&c, c.n_pages); c.d_pos = dalloc<int32_t>(&c, 2);
+        c.qbuf = dalloc<float>(&c, dq); c.act_q.f32 = dalloc<float>(&c, dq_pad);
+        c.part_o = dalloc<float>(&c, (size_t)dq_pad * c.n_split);
+        BLK_CUDA(cudaMemsetAsync(c.part_o, 0, (size_t)dq_pad * c.n_split * 4, c.stream));
+        c.scores = dalloc<float>(&c, (size_t)n_head * c.n_pages * KV_PAGE);
+        float* staging = dalloc<float>(&c, (size_t)n_kv * dkv);
+        const int32_t hpos[2] = {n_kv - 1, 0};
+        BLK_CUDA(cudaMemcpyAsync(c.page_table, hpt.data(), (size_t)c.n_pages * 4, cudaMemcpyHostToDevice, c.stream));
+        BLK_CUDA(cudaMemcpyAsync(c.d_pos, hpos, sizeof(hpos), cudaMemcpyHostToDevice, c.stream));
+        BLK_CUDA(cudaMemcpyAsync(c.qbuf, q, (size_t)dq * 4, cudaMemcpyHostToDevice, c.stream));
+        BLK_CUDA(cudaMemcpyAsync(staging, k, (size_t)n_kv * dkv * 4, cudaMemcpyHostToDevice, c.stream));
+        fill_pool(c.k_pool[0], pool, staging, c.page_table, n_kv, dkv, c.stream);
+        BLK_CUDA(cudaMemcpyAsync(staging, v, (size_t)n_kv * dkv * 4, cudaMemcpyHostToDevice, c.stream));
+        fill_pool(c.v_pool[0], pool, staging, c.page_table, n_kv, dkv, c.stream);
+        BLK_CUDA(cudaMemsetAsync(c.act_q.f32, 0xff, (size_t)dq * 4, c.stream));
+        launch_decode_attn(&c, 0);
+        BLK_CUDA(cudaGetLastError());
+        BLK_CUDA(cudaMemcpyAsync(out, c.act_q.f32, (size_t)dq * 4, cudaMemcpyDeviceToHost, c.stream));
+        BLK_CUDA(cudaStreamSynchronize(c.stream));
+        if (used_form) *used_form = c.attn_cluster > 0 ? 1 : 0;
+    });
+}
+
+// decode_attn_batch_kernel over n <= BATCH_MAX rows in one launch: row b attends with q [b][n_head*dh] (rounded to f16 like the batch
+// step's q) over its own n_kv[b] cells; k / v hold the rows' keys / values one after another ([sum n_kv][n_head_kv*dh], rounded to
+// f16).  Every row has its own seeded random page table and two-layer K / V pools, all NaN except the cells 0 .. n_kv[b] - 1 of
+// layer 1, which the kernel reads.  out [n][n_head*dh] = the kernel's bf16 output as f32.
+extern "C" blk_status blk_test_decode_attn_batch(int32_t device, int32_t n, const float* q, const float* k, const float* v, const int32_t* n_kv,
+                                                 int32_t n_head, int32_t n_head_kv, int32_t d_head, int64_t seed, float* out) {
+    return guarded([&] {
+        if (blk_init() != BLK_OK) throw BlkError(BLK_ERR_NO_DEVICE, g_last_error);
+        if (n <= 0 || n > BATCH_MAX || !n_kv || (d_head != 64 && d_head != 128) || n_head <= 0 || n_head_kv <= 0 || n_head % n_head_kv ||
+            n_head / n_head_kv > MAX_GQ)
+            throw BlkError(BLK_ERR_ARG, "blk_test_decode_attn_batch: bad shape");
+        for (int b = 0; b < n; b++) if (n_kv[b] <= 0) throw BlkError(BLK_ERR_ARG, "blk_test_decode_attn_batch: bad n_kv");
+        BLK_CUDA(cudaSetDevice(device));
+        constexpr int N_LAYER = 2, LAYER = 1;
+        const int dq = n_head * d_head, dkv = n_head_kv * d_head;
+        std::mt19937_64 rng((uint64_t)seed);
+        // per row: its page table, its pool size in pages, where both start, where its keys start
+        std::vector<int32_t> pt_all, pos(n);
+        std::vector<size_t> pt_off(n), page_off(n), row_off(n);
+        size_t total_pages = 0, total_rows = 0;
+        for (int b = 0; b < n; b++) {
+            std::vector<int32_t> pt;
+            const int pool_pages = random_page_table(rng, (n_kv[b] + KV_PAGE - 1) / KV_PAGE, pt);
+            pt_off[b] = pt_all.size(); page_off[b] = total_pages; row_off[b] = total_rows;
+            pt_all.insert(pt_all.end(), pt.begin(), pt.end());
+            total_pages += pool_pages; total_rows += n_kv[b]; pos[b] = n_kv[b] - 1;
+        }
+        const size_t layer_elems = total_pages * KV_PAGE * dkv;
+        Scratch sc;
+        __half* kar = sc.get<__half>(N_LAYER * layer_elems); __half* var = sc.get<__half>(N_LAYER * layer_elems);
+        int32_t* d_pt = sc.get<int32_t>(pt_all.size()); int32_t* d_pos = sc.get<int32_t>(n);
+        float* staging = sc.get<float>(std::max(total_rows * dkv, (size_t)n * dq));
+        __half* q16 = sc.get<__half>((size_t)n * dq);
+        __nv_bfloat16* o = sc.get<__nv_bfloat16>((size_t)n * dq); float* fo = sc.get<float>((size_t)n * dq);
+        // device pointer tables: [b] -> page table, [b] -> [layer] -> pool
+        std::vector<const int32_t*> h_pts(n);
+        std::vector<__half*> h_kl((size_t)n * N_LAYER), h_vl((size_t)n * N_LAYER);
+        const int32_t** d_pts = sc.get<const int32_t*>(n);
+        __half** d_kl = sc.get<__half*>((size_t)n * N_LAYER); __half** d_vl = sc.get<__half*>((size_t)n * N_LAYER);
+        std::vector<__half* const*> h_kp(n), h_vp(n);
+        __half* const** d_kp = sc.get<__half* const*>(n); __half* const** d_vp = sc.get<__half* const*>(n);
+        for (int b = 0; b < n; b++) {
+            h_pts[b] = d_pt + pt_off[b];
+            for (int l = 0; l < N_LAYER; l++) {
+                h_kl[(size_t)b * N_LAYER + l] = kar + l * layer_elems + page_off[b] * KV_PAGE * dkv;
+                h_vl[(size_t)b * N_LAYER + l] = var + l * layer_elems + page_off[b] * KV_PAGE * dkv;
+            }
+            h_kp[b] = d_kl + (size_t)b * N_LAYER; h_vp[b] = d_vl + (size_t)b * N_LAYER;
+        }
+        BLK_CUDA(cudaMemcpy(d_pt, pt_all.data(), pt_all.size() * 4, cudaMemcpyHostToDevice));
+        BLK_CUDA(cudaMemcpy(d_pos, pos.data(), (size_t)n * 4, cudaMemcpyHostToDevice));
+        BLK_CUDA(cudaMemcpy(d_pts, h_pts.data(), (size_t)n * sizeof(void*), cudaMemcpyHostToDevice));
+        BLK_CUDA(cudaMemcpy(d_kl, h_kl.data(), h_kl.size() * sizeof(void*), cudaMemcpyHostToDevice));
+        BLK_CUDA(cudaMemcpy(d_vl, h_vl.data(), h_vl.size() * sizeof(void*), cudaMemcpyHostToDevice));
+        BLK_CUDA(cudaMemcpy(d_kp, h_kp.data(), (size_t)n * sizeof(void*), cudaMemcpyHostToDevice));
+        BLK_CUDA(cudaMemcpy(d_vp, h_vp.data(), (size_t)n * sizeof(void*), cudaMemcpyHostToDevice));
+        BLK_CUDA(cudaMemset(kar, 0xff, N_LAYER * layer_elems * sizeof(__half)));
+        BLK_CUDA(cudaMemset(var, 0xff, N_LAYER * layer_elems * sizeof(__half)));
+        for (int kv = 0; kv < 2; kv++) {
+            BLK_CUDA(cudaMemcpy(staging, kv ? v : k, total_rows * dkv * 4, cudaMemcpyHostToDevice));
+            for (int b = 0; b < n; b++)
+                scatter_cells_kernel<<<grid_of((size_t)n_kv[b] * dkv), 256>>>(staging + row_off[b] * dkv, (kv ? h_vl : h_kl)[(size_t)b * N_LAYER + LAYER],
+                                                                             d_pt + pt_off[b], n_kv[b], dkv);
+            BLK_CUDA(cudaGetLastError());
+            BLK_CUDA(cudaDeviceSynchronize());
+        }
+        BLK_CUDA(cudaMemcpy(staging, q, (size_t)n * dq * 4, cudaMemcpyHostToDevice));
+        f32_to_f16_kernel<<<grid_of((size_t)n * dq), 256>>>(staging, q16, (size_t)n * dq);
+        BLK_CUDA(cudaMemset(o, 0xff, (size_t)n * dq * sizeof(__nv_bfloat16)));
+        BatchAttnArgs aa{};
+        aa.q = q16; aa.pos = d_pos; aa.page_table = d_pts; aa.k_pools = d_kp; aa.v_pools = d_vp; aa.out = o;
+        aa.layer = LAYER; aa.n_head = n_head; aa.n_head_kv = n_head_kv; aa.kv_dim = dkv; aa.scale = 1.0f / sqrtf((float)d_head);
+        if (d_head == 128) decode_attn_batch_kernel<128><<<dim3(n_head_kv, n), 256>>>(aa);
+        else decode_attn_batch_kernel<64><<<dim3(n_head_kv, n), 256>>>(aa);
+        BLK_CUDA(cudaGetLastError());
+        bf16_to_f32_kernel<<<grid_of((size_t)n * dq), 256>>>(o, fo, (size_t)n * dq);
+        BLK_CUDA(cudaGetLastError());
+        BLK_CUDA(cudaMemcpy(out, fo, (size_t)n * dq * 4, cudaMemcpyDeviceToHost));
     });
 }

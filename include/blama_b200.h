@@ -212,6 +212,16 @@ BLK_API blk_status blk_test_qkv_post(int32_t device, const float* qkv, int32_t T
                                      int32_t pos0, float rope_theta, const float* freq_factors, float* q_out, float* k_out, float* v_out);
 BLK_API blk_status blk_test_prefill_attn(int32_t device, const float* q, const float* k, const float* v, int32_t T, int32_t pos0, int32_t n_head,
                                          int32_t n_head_kv, int32_t d_head, float* out, int32_t* used_tc);
+/* The decode attention kernels over a paged f16 cache behind a seeded random page table (pages and cells nothing should read hold NaN).
+ * blk_test_decode_attn: one query row q [n_head*d_head] over cells 0 .. n_kv - 1 of a context of n_ctx cells (k / v [n_kv][n_head_kv*d_head]),
+ * through the per-op decode step's form plan and launch; form -1 = the plan's choice, 0 = the three-kernel split form, 1 = the cluster form
+ * (BLK_ERR_ARG without a launch when the plan does not allow it); *used_form = 1 when the cluster form ran.
+ * blk_test_decode_attn_batch: the batched decode step's attention over n rows of their own lengths n_kv[n] in one launch (k / v: the
+ * rows' keys / values one after another); out [n][n_head*d_head] = the bf16 output as f32. */
+BLK_API blk_status blk_test_decode_attn(int32_t device, const float* q, const float* k, const float* v, int32_t n_kv, int32_t n_ctx, int32_t n_head,
+                                        int32_t n_head_kv, int32_t d_head, int32_t form, int64_t seed, float* out, int32_t* used_form);
+BLK_API blk_status blk_test_decode_attn_batch(int32_t device, int32_t n, const float* q, const float* k, const float* v, const int32_t* n_kv,
+                                              int32_t n_head, int32_t n_head_kv, int32_t d_head, int64_t seed, float* out);
 /* dequantise through the device re-tile + dequant kernels */
 BLK_API blk_status blk_test_dequant(int32_t device, int32_t type, const void* w_blocks, int64_t rows, int64_t k, float* out);
 
