@@ -765,71 +765,107 @@ void enqueue_step(blk_ctx* c, bool with_head, bool feedback = false) {
 } // namespace
 
 // ------------------------------------------------------------------------------------------------------------------
-// cell positions other than the cell index (Self-Extend: llama_kv_self_seq_add / seq_div, reference Session.cpp:348-368)
+// KV cell bookkeeping: the cells in use (n_past), their rotary positions (Self-Extend: llama_kv_self_seq_add / seq_div,
+// reference Session.cpp:348-368) and the device copy d_pos
 // ------------------------------------------------------------------------------------------------------------------
 namespace {
-// K rows of cells [cell0, cell0 + n) of every layer rotated IN PLACE by each cell's own position delta (llama.cpp's K-shift after
-// llama_kv_self_seq_add / seq_div: ggml rope on the F16 cache).  grid = (n, n_layer), block = 128.
-__global__ void __launch_bounds__(128) kv_rerope_kernel(__half* const* __restrict__ k_pools, const int32_t* __restrict__ page_table, int kv_dim, int d_head,
-                                                        int neox, int cell0, const int32_t* __restrict__ delta, float theta_scale,
+// K rows of cells [src0, src0 + n) of every layer re-rotated by a position delta and written to cells [dst0, dst0 + n), the way
+// llama.cpp's K-shift does it (ggml rope on the F16 cache: f16 -> f32, rotate by theta_i = delta * theta_scale^i / freq_factor_i,
+// f32 -> f16).  The delta is `deltas[cell]` of the source cell when `deltas` is given, else `delta`.  V rows are copied when the
+// cells move.  The two ranges are the same (in place) or do not overlap.  grid = (n, n_layer), block = 128.
+__global__ void __launch_bounds__(128) kv_rerope_kernel(__half* const* __restrict__ k_pools, __half* const* __restrict__ v_pools,
+                                                        const int32_t* __restrict__ page_table, int kv_dim, int d_head, int neox, int src0,
+                                                        int dst0, int delta, const int32_t* __restrict__ deltas, float theta_scale,
                                                         const float* __restrict__ freq_factors) {
     __shared__ float2 cs[64];
-    const int cell = cell0 + (int)blockIdx.x;
-    const int dl = delta[cell];
-    if (dl == 0) return;
+    const int ts = src0 + (int)blockIdx.x, td = dst0 + (int)blockIdx.x;
+    const int dl = deltas ? deltas[ts] : delta;
+    if (dl == 0 && ts == td) return;
     const int half_rot = d_head / 2;
     rope_table_fill(cs, half_rot, dl, theta_scale, freq_factors);
     __syncthreads();
-    __half* k = k_pools[blockIdx.y] + ((size_t)page_table[cell / KV_PAGE] * KV_PAGE + (cell % KV_PAGE)) * kv_dim;
+    const size_t rs = ((size_t)page_table[ts / KV_PAGE] * KV_PAGE + (ts % KV_PAGE)) * kv_dim;
+    const size_t rd = ((size_t)page_table[td / KV_PAGE] * KV_PAGE + (td % KV_PAGE)) * kv_dim;
+    const __half* ks = k_pools[blockIdx.y] + rs; __half* kd = k_pools[blockIdx.y] + rd;
     for (int p = threadIdx.x; p < kv_dim / 2; p += blockDim.x) {
         const int h = p / half_rot, i = p - h * half_rot;
         const int e0 = neox ? h * d_head + i : h * d_head + 2 * i;
         const int e1 = neox ? e0 + half_rot : e0 + 1;
-        const float x0 = __half2float(k[e0]), x1 = __half2float(k[e1]);
+        const float x0 = __half2float(ks[e0]), x1 = __half2float(ks[e1]);
         const float2 c = cs[i];
-        k[e0] = __float2half_rn(__fsub_rn(__fmul_rn(x0, c.x), __fmul_rn(x1, c.y)));
-        k[e1] = __float2half_rn(__fadd_rn(__fmul_rn(x0, c.y), __fmul_rn(x1, c.x)));
+        kd[e0] = __float2half_rn(__fsub_rn(__fmul_rn(x0, c.x), __fmul_rn(x1, c.y)));
+        kd[e1] = __float2half_rn(__fadd_rn(__fmul_rn(x0, c.y), __fmul_rn(x1, c.x)));
     }
+    if (ts == td) return;
+    const __half* vs = v_pools[blockIdx.y] + rs; __half* vd = v_pools[blockIdx.y] + rd;
+    for (int e = threadIdx.x; e < kv_dim / 8; e += blockDim.x) reinterpret_cast<uint4*>(vd)[e] = reinterpret_cast<const uint4*>(vs)[e];
 }
 
-// positions of the cells as a host vector (created on the first Self-Extend call)
+void rerope_cells(blk_ctx* c, int src0, int dst0, int n, int delta, const int32_t* deltas) {
+    const blk_model* m = c->m;
+    kv_rerope_kernel<<<dim3((unsigned)n, (unsigned)m->n_layer), 128, 0, c->stream>>>(c->d_kpools, c->d_vpools, c->page_table, m->n_head_kv * m->d_head,
+                                                                                      m->d_head, m->neox ? 1 : 0, src0, dst0, delta, deltas,
+                                                                                      m->theta_scale, m->rope_freqs);
+    BLK_CUDA(cudaGetLastError());
+    c->launches++;
+}
+
+// d_pos from the host's {n_past, rope_off}; the kernels advance it themselves as they add cells
+void upload_pos(blk_ctx* c) {
+    const int32_t both[2] = {c->n_past, c->rope_off};
+    BLK_CUDA(cudaMemcpyAsync(c->d_pos, both, sizeof(both), cudaMemcpyHostToDevice, c->stream));
+    BLK_CUDA(cudaStreamSynchronize(c->stream));      // `both` is a stack variable
+}
+
+// n_past cells, every position its cell index, no logits
+void reset_cells(blk_ctx* c, int n_past) {
+    c->n_past = n_past; c->have_logits = false;
+    c->cell_pos.clear(); c->cell_shift.clear(); c->rope_off = 0; c->shift_pending = false;
+    upload_pos(c);
+}
+
+// the first Self-Extend call: every cell's position is its index and no shift is pending
 void materialise_positions(blk_ctx* c) {
-    if (!c->cell_pos.empty() || c->n_past == 0) { if (c->cell_pos.empty()) { c->cell_pos.assign((size_t)c->n_ctx, 0); c->cell_shift.assign((size_t)c->n_ctx, 0); } return; }
-    c->cell_pos.resize((size_t)c->n_ctx); c->cell_shift.assign((size_t)c->n_ctx, 0);
+    if (!c->cell_pos.empty()) return;
+    c->cell_pos.resize((size_t)c->n_ctx);
     for (int i = 0; i < c->n_ctx; i++) c->cell_pos[(size_t)i] = i;
+    c->cell_shift.assign((size_t)c->n_ctx, 0);
+    if (!c->d_cell_shift) c->d_cell_shift = dalloc<int32_t>(c, (size_t)c->n_ctx);
 }
 // after a position change: the next token's rotary position is one past the largest cell position (llama_batch_allocr, pos == nullptr)
 void refresh_rope_offset(blk_ctx* c) {
     int mx = -1;
     for (int i = 0; i < c->n_past; i++) mx = std::max(mx, c->cell_pos[(size_t)i]);
     c->rope_off = (mx + 1) - c->n_past;
-    const int32_t both[2] = {c->n_past, c->rope_off};
-    BLK_CUDA(cudaMemcpyAsync(c->d_pos, both, sizeof(both), cudaMemcpyHostToDevice, c->stream));
-    BLK_CUDA(cudaStreamSynchronize(c->stream));
-}
-// new cells [n_past, n_past + n) take the positions the kernels used for them
-void note_new_cells(blk_ctx* c, int n) {
-    if (c->cell_pos.empty()) return;
-    for (int i = 0; i < n; i++) { c->cell_pos[(size_t)(c->n_past + i)] = c->n_past + c->rope_off + i; c->cell_shift[(size_t)(c->n_past + i)] = 0; }
+    upload_pos(c);
 }
 // the accumulated position changes reach the K rows before anything reads them (llama.cpp applies its K-shift at the next decode)
 void flush_pos_shift(blk_ctx* c) {
     if (!c->shift_pending) return;
-    blk_model* m = c->m;
-    int32_t* d_delta = nullptr;
-    BLK_CUDA(cudaMalloc(&d_delta, (size_t)c->n_past * sizeof(int32_t)));
-    cudaError_t e = cudaMemcpyAsync(d_delta, c->cell_shift.data(), (size_t)c->n_past * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream);
-    if (e == cudaSuccess) {
-        kv_rerope_kernel<<<dim3((unsigned)c->n_past, (unsigned)m->n_layer), 128, 0, c->stream>>>(c->d_kpools, c->page_table, m->n_head_kv * m->d_head, m->d_head,
-                                                                                                   m->neox ? 1 : 0, 0, d_delta, m->theta_scale, m->rope_freqs);
-        e = cudaGetLastError();
-        c->launches++;
-    }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    cudaFree(d_delta);
-    BLK_CUDA(e);
+    BLK_CUDA(cudaMemcpyAsync(c->d_cell_shift, c->cell_shift.data(), (size_t)c->n_past * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
+    rerope_cells(c, 0, 0, c->n_past, 0, c->d_cell_shift);
+    BLK_CUDA(cudaStreamSynchronize(c->stream));      // cell_shift is cleared next
     std::fill(c->cell_shift.begin(), c->cell_shift.begin() + c->n_past, 0);
     c->shift_pending = false;
+}
+
+// the checks of begin_cells: the token ids index the embedding matrix, and the n new cells fit the context (callers that add cells
+// in several parts run it for all of them first)
+void check_cells(const blk_ctx* c, const int32_t* ids, int n_ids, int n) {
+    for (int i = 0; i < n_ids; i++) if (ids[i] < 0 || ids[i] >= c->m->n_vocab) throw BlkError(BLK_ERR_ARG, "token id out of range");
+    if (c->n_past + n > c->n_ctx) throw BlkError(BLK_ERR_CTX_FULL, "context is full");
+}
+// Every path that puts n tokens into the cache starts with begin_cells and ends with end_cells.  begin_cells checks the ids and
+// the room, applies pending re-rotations and records the positions the kernels use for the new cells [n_past, n_past + n).
+void begin_cells(blk_ctx* c, const int32_t* ids, int n_ids, int n) {
+    check_cells(c, ids, n_ids, n);
+    flush_pos_shift(c);
+    if (c->cell_pos.empty()) return;
+    for (int i = 0; i < n; i++) { c->cell_pos[(size_t)(c->n_past + i)] = c->n_past + c->rope_off + i; c->cell_shift[(size_t)(c->n_past + i)] = 0; }
+}
+void end_cells(blk_ctx* c, int n, bool have_logits) {
+    c->n_past += n;
+    c->have_logits = have_logits;
 }
 } // namespace
 
@@ -1131,8 +1167,7 @@ void prefill_chunk(blk_ctx* c, const int32_t* tokens, int n, const VerifyIo* ver
     blk_model* m = c->m;
     const int d = m->n_embd, dh = m->d_head, dq = m->n_head * dh, dkv = m->n_head_kv * dh, V = m->n_vocab;
     ensure_prefill_bufs(c, n);
-    flush_pos_shift(c);
-    note_new_cells(c, n);
+    begin_cells(c, tokens, n, n);
     cudaStream_t st = c->stream;
     const ChainPdl chain_scope(n);      // few-token passes: every kernel of the chain is a programmatic dependent of its predecessor
     BLK_CUDA(cudaMemcpyAsync(c->pf_tokens, tokens, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
@@ -1207,8 +1242,7 @@ void prefill_chunk(blk_ctx* c, const int32_t* tokens, int n, const VerifyIo* ver
         matvec<EPI_STORE>(c, a, c->pf_x + (size_t)(n - 1) * d, m->out_norm, c->act_d, "gemv_lm_head");
         topk_of_logits(c);
     }
-    c->n_past += n;
-    c->have_logits = true;
+    end_cells(c, n, true);
 }
 
 // tokens per chunk when n tokens do not fit one logical batch: equal chunks (rounded up to whole 64-token tiles) instead of full
@@ -1248,11 +1282,7 @@ void check_mega(blk_ctx* c) {
 }
 
 void step(blk_ctx* c, int32_t tok, bool with_head) {
-    blk_model* m = c->m;
-    if (tok < 0 || tok >= m->n_vocab) throw BlkError(BLK_ERR_ARG, "token id out of range");
-    if (c->n_past + 1 > c->n_ctx) throw BlkError(BLK_ERR_CTX_FULL, "context is full");
-    flush_pos_shift(c);
-    note_new_cells(c, 1);
+    begin_cells(c, &tok, 1, 1);
     // pinned ring of token slots: a slot is only rewritten after the stream has drained once per lap
     if (c->tok_slot == 0) BLK_CUDA(cudaStreamSynchronize(c->stream));
     int32_t* slot = c->h_tok + c->tok_slot;
@@ -1264,8 +1294,7 @@ void step(blk_ctx* c, int32_t tok, bool with_head) {
         BLK_CUDA(cudaGraphLaunch(with_head ? c->g_full : c->g_body, c->stream));
         c->launches += with_head ? c->launches_full : c->launches_body;
     }
-    c->n_past++;
-    c->have_logits = with_head;
+    end_cells(c, 1, with_head);
 }
 
 } // namespace
@@ -1309,7 +1338,7 @@ extern "C" blk_ctx* blk_ctx_create(blk_model* m, int32_t n_ctx, int32_t n_batch)
         BLK_CUDA(cudaMemcpy(c->d_kpools, c->k_pool.data(), m->n_layer * sizeof(__half*), cudaMemcpyHostToDevice));
         BLK_CUDA(cudaMemcpy(c->d_vpools, c->v_pool.data(), m->n_layer * sizeof(__half*), cudaMemcpyHostToDevice));
         c->d_tok = dalloc<int32_t>(c.get(), 1); c->d_pos = dalloc<int32_t>(c.get(), 2);
-        BLK_CUDA(cudaMemset(c->d_pos, 0, 2 * sizeof(int32_t)));
+        upload_pos(c.get());
         c->h_tok = halloc<int32_t>(c.get(), blk_ctx::TOK_RING);
         c->x = dalloc<float>(c.get(), d); c->qbuf = dalloc<float>(c.get(), dq); c->hbuf = dalloc<float>(c.get(), ff);
         c->rope_cs = dalloc<float2>(c.get(), dh / 2);
@@ -1375,7 +1404,7 @@ extern "C" blk_ctx* blk_ctx_create(blk_model* m, int32_t n_ctx, int32_t n_batch)
                 }
             }
             if (!c->mega_on) { enqueue_step(c.get(), true, false); BLK_CUDA(cudaStreamSynchronize(c->stream)); }
-            BLK_CUDA(cudaMemsetAsync(c->d_pos, 0, sizeof(int32_t), c->stream));
+            reset_cells(c.get(), 0);
             c->launches = 0;
         }
         if (!c->mega_on) build_graphs(c.get());
@@ -1400,9 +1429,7 @@ extern "C" blk_status blk_ctx_set_verify_mode(blk_ctx* c, int32_t mode) {
 extern "C" blk_status blk_kv_clear(blk_ctx* c) {
     return guarded([&] {
         BLK_CUDA(cudaSetDevice(c->m->device));
-        BLK_CUDA(cudaMemsetAsync(c->d_pos, 0, 2 * sizeof(int32_t), c->stream));
-        c->n_past = 0; c->have_logits = false;
-        c->cell_pos.clear(); c->cell_shift.clear(); c->rope_off = 0; c->shift_pending = false;
+        reset_cells(c, 0);
     });
 }
 extern "C" blk_status blk_sync(blk_ctx* c) {
@@ -1413,40 +1440,21 @@ extern "C" blk_status blk_sync(blk_ctx* c) {
 // context shift + state (reference Session.cpp:324-347 llama_kv_self_seq_rm / seq_add; :284-310 llama_state_get/set_data)
 // ------------------------------------------------------------------------------------------------------------------
 namespace {
-// Cache rows [src0, src0 + n) of every layer move to [dst0, dst0 + n) (the two ranges do not overlap within one launch).  K rows are
-// re-rotated by `delta` positions the way llama.cpp's K-shift does it (ggml rope on the F16 cache: f16 -> f32, rotate by
-// theta_i = delta * theta_scale^i / freq_factor_i, f32 -> f16); V rows are copied.  grid = (n, n_layer), block = 128.
-__global__ void __launch_bounds__(128) kv_shift_kernel(__half* const* __restrict__ k_pools, __half* const* __restrict__ v_pools,
-                                                       const int32_t* __restrict__ page_table, int kv_dim, int d_head, int neox, int src0, int dst0,
-                                                       int delta, float theta_scale, const float* __restrict__ freq_factors) {
-    __shared__ float2 cs[64];
-    const int half_rot = d_head / 2;
-    rope_table_fill(cs, half_rot, delta, theta_scale, freq_factors);
-    __syncthreads();
-    const int ts = src0 + (int)blockIdx.x, td = dst0 + (int)blockIdx.x;
-    const size_t rs = ((size_t)page_table[ts / KV_PAGE] * KV_PAGE + (ts % KV_PAGE)) * kv_dim;
-    const size_t rd = ((size_t)page_table[td / KV_PAGE] * KV_PAGE + (td % KV_PAGE)) * kv_dim;
-    const __half* ks = k_pools[blockIdx.y] + rs; __half* kd = k_pools[blockIdx.y] + rd;
-    const __half* vs = v_pools[blockIdx.y] + rs; __half* vd = v_pools[blockIdx.y] + rd;
-    for (int p = threadIdx.x; p < kv_dim / 2; p += blockDim.x) {
-        const int h = p / half_rot, i = p - h * half_rot;
-        const int e0 = neox ? h * d_head + i : h * d_head + 2 * i;
-        const int e1 = neox ? e0 + half_rot : e0 + 1;
-        const float x0 = __half2float(ks[e0]), x1 = __half2float(ks[e1]);
-        const float2 c = cs[i];
-        kd[e0] = __float2half_rn(__fsub_rn(__fmul_rn(x0, c.x), __fmul_rn(x1, c.y)));
-        kd[e1] = __float2half_rn(__fadd_rn(__fmul_rn(x0, c.y), __fmul_rn(x1, c.x)));
-    }
-    for (int e = threadIdx.x; e < kv_dim / 8; e += blockDim.x) reinterpret_cast<uint4*>(vd)[e] = reinterpret_cast<const uint4*>(vs)[e];
-}
-
 constexpr uint32_t STATE_MAGIC = 0x534B4C42u;      // "BLKS"
-struct StateHeader { uint32_t magic, version; int32_t n_layer, kv_dim, n_vocab, n_past, have_logits, reserved; };
+struct StateHeader { uint32_t magic, version; int32_t n_layer, kv_dim, n_vocab, n_past, have_logits, with_positions; };
 size_t state_bytes(const blk_ctx* c, int n_past, bool with_positions) {
     const blk_model* m = c->m;
     const size_t kv_dim = (size_t)m->n_head_kv * m->d_head;
     return sizeof(StateHeader) + (size_t)m->n_vocab * 4 + TOPK_MAX * 8 + (with_positions ? 4 + (size_t)n_past * 4 : 0) +
            2 * (size_t)m->n_layer * (size_t)n_past * kv_dim * 2;
+}
+// the K and V rows of cells [0, n_past) in state blob order: per layer K then V, one contiguous run per page
+template <class F> void for_each_kv_run(blk_ctx* c, int n_past, F&& f) {
+    const int kv_dim = c->m->n_head_kv * c->m->d_head;
+    for (int l = 0; l < c->m->n_layer; l++)
+        for (__half* pool : {c->k_pool[l], c->v_pool[l]})
+            for (int t0 = 0; t0 < n_past; t0 += KV_PAGE)
+                f(pool + (size_t)c->page_table_host[t0 / KV_PAGE] * KV_PAGE * kv_dim, (size_t)std::min(KV_PAGE, n_past - t0) * kv_dim * 2);
 }
 } // namespace
 
@@ -1456,20 +1464,12 @@ extern "C" blk_status blk_kv_shift(blk_ctx* c, int32_t p0, int32_t p1) {
         blk_model* m = c->m;
         BLK_CUDA(cudaSetDevice(m->device));
         if (!c->cell_pos.empty()) throw BlkError(BLK_ERR_ARG, "blk_kv_shift: not available once Self-Extend has moved cell positions (blk_kv_seq_add / blk_kv_seq_div)");
-        const int d = p1 - p0, dkv = m->n_head_kv * m->d_head;
+        const int d = p1 - p0;
         // front to back in chunks of at most d rows: a chunk's destination never overlaps its source, and what it overwrites has been
         // moved already
-        for (int t = p1; t < c->n_past; t += d) {
-            const int n = std::min(d, c->n_past - t);
-            kv_shift_kernel<<<dim3((unsigned)n, (unsigned)m->n_layer), 128, 0, c->stream>>>(c->d_kpools, c->d_vpools, c->page_table, dkv, m->d_head, m->neox ? 1 : 0,
-                                                                                                t, t - d, -d, m->theta_scale, m->rope_freqs);
-            BLK_CUDA(cudaGetLastError());
-            c->launches++;
-        }
+        for (int t = p1; t < c->n_past; t += d) rerope_cells(c, t, t - d, std::min(d, c->n_past - t), -d, nullptr);
         c->n_past -= d;
-        int32_t np = c->n_past;
-        BLK_CUDA(cudaMemcpyAsync(c->d_pos, &np, sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
-        BLK_CUDA(cudaStreamSynchronize(c->stream));      // np is a stack variable
+        upload_pos(c);
     });
 }
 
@@ -1498,14 +1498,7 @@ extern "C" blk_status blk_state_get(blk_ctx* c, void* dst, int64_t cap, int64_t*
             memcpy(out, &off, 4); out += 4;
             memcpy(out, c->cell_pos.data(), (size_t)c->n_past * 4); out += (size_t)c->n_past * 4;
         }
-        const size_t row = (size_t)kv_dim * 2;
-        for (int l = 0; l < m->n_layer; l++)
-            for (const __half* pool : {c->k_pool[l], c->v_pool[l]})
-                for (int t0 = 0; t0 < c->n_past; t0 += KV_PAGE) {
-                    const int n = std::min(KV_PAGE, c->n_past - t0);
-                    BLK_CUDA(cudaMemcpy(out, pool + (size_t)c->page_table_host[t0 / KV_PAGE] * KV_PAGE * kv_dim, n * row, cudaMemcpyDeviceToHost));
-                    out += n * row;
-                }
+        for_each_kv_run(c, c->n_past, [&](const __half* rows, size_t bytes) { BLK_CUDA(cudaMemcpy(out, rows, bytes, cudaMemcpyDeviceToHost)); out += bytes; });
         *written = (int64_t)need;
     });
 }
@@ -1522,32 +1515,22 @@ extern "C" blk_status blk_state_set(blk_ctx* c, const void* src, int64_t size) {
         if (h.magic != STATE_MAGIC || h.version != 1u) throw BlkError(BLK_ERR_FORMAT, "blk_state_set: not a state blob of this engine");
         if (h.n_layer != m->n_layer || h.kv_dim != kv_dim || h.n_vocab != m->n_vocab) throw BlkError(BLK_ERR_FORMAT, "blk_state_set: the state belongs to another model");
         if (h.n_past < 0 || h.n_past > c->n_ctx) throw BlkError(BLK_ERR_CTX_FULL, "blk_state_set: the state does not fit this context");
-        if ((size_t)size != state_bytes(c, h.n_past, h.reserved != 0)) throw BlkError(BLK_ERR_FORMAT, "blk_state_set: truncated state");
+        if ((size_t)size != state_bytes(c, h.n_past, h.with_positions != 0)) throw BlkError(BLK_ERR_FORMAT, "blk_state_set: truncated state");
         BLK_CUDA(cudaStreamSynchronize(c->stream));
+        reset_cells(c, h.n_past);
         BLK_CUDA(cudaMemcpy(c->logits, in, (size_t)m->n_vocab * 4, cudaMemcpyHostToDevice)); in += (size_t)m->n_vocab * 4;
         memcpy(c->h_top_ids, in, TOPK_MAX * 4); in += TOPK_MAX * 4;
         memcpy(c->h_top_logits, in, TOPK_MAX * 4); in += TOPK_MAX * 4;
         BLK_CUDA(cudaMemcpy(c->top_ids, c->h_top_ids, TOPK_MAX * 4, cudaMemcpyHostToDevice));
         BLK_CUDA(cudaMemcpy(c->top_logits, c->h_top_logits, TOPK_MAX * 4, cudaMemcpyHostToDevice));
-        c->cell_pos.clear(); c->cell_shift.clear(); c->rope_off = 0; c->shift_pending = false;
-        if (h.reserved != 0) {
-            int32_t off = 0;
-            memcpy(&off, in, 4); in += 4;
-            c->cell_pos.assign((size_t)c->n_ctx, 0); c->cell_shift.assign((size_t)c->n_ctx, 0);
+        if (h.with_positions != 0) {
+            materialise_positions(c);
+            memcpy(&c->rope_off, in, 4); in += 4;
             memcpy(c->cell_pos.data(), in, (size_t)h.n_past * 4); in += (size_t)h.n_past * 4;
-            c->rope_off = off;
+            upload_pos(c);
         }
-        const size_t row = (size_t)kv_dim * 2;
-        for (int l = 0; l < m->n_layer; l++)
-            for (__half* pool : {c->k_pool[l], c->v_pool[l]})
-                for (int t0 = 0; t0 < h.n_past; t0 += KV_PAGE) {
-                    const int n = std::min(KV_PAGE, h.n_past - t0);
-                    BLK_CUDA(cudaMemcpy(pool + (size_t)c->page_table_host[t0 / KV_PAGE] * KV_PAGE * kv_dim, in, n * row, cudaMemcpyHostToDevice));
-                    in += n * row;
-                }
-        c->n_past = h.n_past; c->have_logits = h.have_logits != 0;
-        const int32_t both[2] = {h.n_past, c->rope_off};
-        BLK_CUDA(cudaMemcpy(c->d_pos, both, sizeof(both), cudaMemcpyHostToDevice));
+        for_each_kv_run(c, h.n_past, [&](__half* rows, size_t bytes) { BLK_CUDA(cudaMemcpy(rows, in, bytes, cudaMemcpyHostToDevice)); in += bytes; });
+        c->have_logits = h.have_logits != 0;
     });
 }
 
@@ -1555,8 +1538,7 @@ extern "C" blk_status blk_decode(blk_ctx* c, const int32_t* tokens, int32_t n) {
     if (!c || !tokens || n <= 0) return fail(BLK_ERR_ARG, "blk_decode: bad arguments");
     return guarded([&] {
         BLK_CUDA(cudaSetDevice(c->m->device));
-        if (c->n_past + n > c->n_ctx) throw BlkError(BLK_ERR_CTX_FULL, "context is full");
-        for (int i = 0; i < n; i++) if (tokens[i] < 0 || tokens[i] >= c->m->n_vocab) throw BlkError(BLK_ERR_ARG, "token id out of range");
+        check_cells(c, tokens, n, n);
         if (n >= c->prefill_min) {
             const int per = balanced_chunk(n, c->n_batch);
             for (int off = 0; off < n; off += per) prefill_chunk(c, tokens + off, std::min(per, n - off), nullptr, 0);
@@ -1591,10 +1573,7 @@ extern "C" blk_status blk_decode_batch(blk_ctx* ws, blk_ctx* const* ctxs, const 
             blk_ctx* c = ctxs[i];
             if (!c || c->m != m) throw BlkError(BLK_ERR_ARG, "blk_decode_batch: every context must belong to the workspace's model");
             for (int j = 0; j < i; j++) if (ctxs[j] == c) throw BlkError(BLK_ERR_ARG, "blk_decode_batch: a context appears twice");
-            if (tokens[i] < 0 || tokens[i] >= V) throw BlkError(BLK_ERR_ARG, "token id out of range");
-            if (c->n_past + 1 > c->n_ctx) throw BlkError(BLK_ERR_CTX_FULL, "context is full");
-            BLK_CUDA(cudaStreamSynchronize(c->stream));          // its prompt prefill / previous step ran on its own stream
-            flush_pos_shift(c);
+            check_cells(c, tokens + i, 1, 1);
         }
         ensure_prefill_bufs(ws, n);
         if (!ws->bd_host) {
@@ -1614,9 +1593,11 @@ extern "C" blk_status blk_decode_batch(blk_ctx* ws, blk_ctx* const* ctxs, const 
         BatchDesc* h = reinterpret_cast<BatchDesc*>(ws->bd_host);
         const BatchDesc* dv = reinterpret_cast<const BatchDesc*>(ws->bd_dev);
         for (int i = 0; i < n; i++) {
-            h->tokens[i] = tokens[i]; h->pos[i] = ctxs[i]->n_past; h->rpos[i] = ctxs[i]->n_past + ctxs[i]->rope_off; h->page_table[i] = ctxs[i]->page_table;
-            note_new_cells(ctxs[i], 1);
-            h->k_pools[i] = ctxs[i]->d_kpools; h->v_pools[i] = ctxs[i]->d_vpools; h->pos_ptr[i] = ctxs[i]->d_pos;
+            blk_ctx* c = ctxs[i];
+            BLK_CUDA(cudaStreamSynchronize(c->stream));          // its prompt prefill / previous step ran on its own stream
+            begin_cells(c, tokens + i, 1, 1);
+            h->tokens[i] = tokens[i]; h->pos[i] = c->n_past; h->rpos[i] = c->n_past + c->rope_off; h->page_table[i] = c->page_table;
+            h->k_pools[i] = c->d_kpools; h->v_pools[i] = c->d_vpools; h->pos_ptr[i] = c->d_pos;
         }
         BLK_CUDA(cudaMemcpyAsync(ws->bd_dev, ws->bd_host, sizeof(BatchDesc), cudaMemcpyHostToDevice, st));
         embed_rows_kernel<<<n, 256, 0, st>>>(m->tok_embd, dv->tokens, dv->rpos, ws->pf_x, ws->pf_rope, dh / 2, m->theta_scale, m->rope_freqs);
@@ -1660,7 +1641,7 @@ extern "C" blk_status blk_decode_batch(blk_ctx* ws, blk_ctx* const* ctxs, const 
         BLK_CUDA(cudaMemcpyAsync(ws->bd_h_top_logits, ws->bd_top_logits, (size_t)n * TOPK_MAX * sizeof(float), cudaMemcpyDeviceToHost, st));
         BLK_CUDA(cudaStreamSynchronize(st));
         for (int i = 0; i < n; i++) {
-            ctxs[i]->n_past++; ctxs[i]->have_logits = false;
+            end_cells(ctxs[i], 1, false);
             for (int j = 0; j < k; j++) { out[(size_t)i * k + j].token = ws->bd_h_top_ids[i * TOPK_MAX + j]; out[(size_t)i * k + j].logit = ws->bd_h_top_logits[i * TOPK_MAX + j]; }
         }
     });
@@ -1671,10 +1652,7 @@ extern "C" blk_status blk_decode_loop(blk_ctx* c, int32_t first_token, int32_t n
     return guarded([&] {
         blk_model* m = c->m;
         BLK_CUDA(cudaSetDevice(m->device));
-        if (first_token < 0 || first_token >= m->n_vocab) throw BlkError(BLK_ERR_ARG, "token id out of range");
-        if (c->n_past + n_steps > c->n_ctx) throw BlkError(BLK_ERR_CTX_FULL, "context is full");
-        flush_pos_shift(c);
-        note_new_cells(c, n_steps);
+        begin_cells(c, &first_token, 1, n_steps);
         BLK_CUDA(cudaStreamSynchronize(c->stream));
         c->h_tok[0] = first_token; c->tok_slot = 1;
         BLK_CUDA(cudaMemcpyAsync(c->d_tok, c->h_tok, sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
@@ -1683,10 +1661,9 @@ extern "C" blk_status blk_decode_loop(blk_ctx* c, int32_t first_token, int32_t n
             for (int i = 0; i < n_steps; i++) BLK_CUDA(cudaGraphLaunch(c->g_loop, c->stream));
             c->launches += c->launches_loop * n_steps;
         }
-        c->n_past += n_steps;
+        end_cells(c, n_steps, true);
         BLK_CUDA(cudaMemcpyAsync(c->h_top_ids, c->top_ids, TOPK_MAX * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
         BLK_CUDA(cudaMemcpyAsync(c->h_top_logits, c->top_logits, TOPK_MAX * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-        c->have_logits = true;
         if (last_token) { BLK_CUDA(cudaStreamSynchronize(c->stream)); *last_token = c->h_top_ids[0]; }
     });
 }
@@ -1741,8 +1718,7 @@ extern "C" blk_status blk_verify_prefill(blk_ctx* c, const int32_t* tokens, int3
     if (!c || !tokens || n <= 0 || !claimed || !n_claimed || !gathered) return fail(BLK_ERR_ARG, "blk_verify_prefill: bad arguments");
     return guarded([&] {
         BLK_CUDA(cudaSetDevice(c->m->device));
-        if (c->n_past + n > c->n_ctx) throw BlkError(BLK_ERR_CTX_FULL, "context is full");
-        for (int i = 0; i < n; i++) if (tokens[i] < 0 || tokens[i] >= c->m->n_vocab) throw BlkError(BLK_ERR_ARG, "token id out of range");
+        check_cells(c, tokens, n, n);
         if (c->verify_mode == 0 && n >= c->prefill_min) {
             VerifyIo io{claimed, n_claimed, gathered, top};
             const int per = balanced_chunk(n, c->n_batch);
@@ -1857,8 +1833,7 @@ extern "C" blk_status blk_bench_kernel(blk_ctx* c, int32_t which, int32_t iters,
         BLK_CUDA(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
         *avg_ms = ms / (float)iters;
         *bytes_per_launch = bytes / iters;
-        BLK_CUDA(cudaMemsetAsync(c->d_pos, 0, sizeof(int32_t), c->stream));
-        c->n_past = 0; c->have_logits = false;
+        reset_cells(c, 0);
     });
 }
 
@@ -1890,7 +1865,7 @@ extern "C" blk_status blk_profile_step(blk_ctx* c, int32_t token, char* report, 
     if (!c || !report || cap <= 0) return fail(BLK_ERR_ARG, "blk_profile_step: bad arguments");
     return guarded([&] {
         BLK_CUDA(cudaSetDevice(c->m->device));
-        if (c->n_past + 1 > c->n_ctx) throw BlkError(BLK_ERR_CTX_FULL, "context is full");
+        begin_cells(c, &token, 1, 1);
         BLK_CUDA(cudaStreamSynchronize(c->stream));
         c->h_tok[0] = token; c->tok_slot = 1;
         BLK_CUDA(cudaMemcpyAsync(c->d_tok, c->h_tok, sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
@@ -1899,7 +1874,7 @@ extern "C" blk_status blk_profile_step(blk_ctx* c, int32_t token, char* report, 
         enqueue_step(c, true, false);
         c->profiling = false;
         BLK_CUDA(cudaStreamSynchronize(c->stream));
-        c->n_past++; c->have_logits = true;
+        end_cells(c, 1, true);
         prof_report(c, report, cap);
     });
 }

@@ -86,7 +86,7 @@ struct blk_model {
 
 struct blk_ctx {
     blk_model* m = nullptr;
-    int n_ctx = 0, n_batch = 0, n_past = 0;
+    int n_ctx = 0, n_batch = 0, n_past = 0;   // n_past: cells in the cache = cell index of the next token
     int n_pages = 0, n_split = 1;
     int verify_mode = 0;
     cudaStream_t stream = nullptr;
@@ -101,12 +101,15 @@ struct blk_ctx {
     std::vector<int32_t> page_table_host;                          // host copy of the page table (state save / restore)
     // decode-step state
     int32_t* d_tok = nullptr;
-    int32_t* d_pos = nullptr;             // device [2]: {cells in the cache = cell index of the next token, rotary position of the next token MINUS that}
+    // KV cell bookkeeping (engine.cu): every path that adds cells goes through begin_cells / end_cells, every reset through
+    // reset_cells, and only upload_pos writes d_pos from the host.
+    int32_t* d_pos = nullptr;             // device [2]: {n_past, rope_off}; the kernels that add cells advance word 0
     // Self-Extend (llama_kv_self_seq_add / seq_div, reference Session.cpp:348-368): cell positions other than the cell index.
     // Materialised on the first such call; empty = every cell's position is its index (the normal case, nothing is touched).
     std::vector<int32_t> cell_pos, cell_shift;      // position of every cell; rotation delta not yet applied to its K row
+    int32_t* d_cell_shift = nullptr;                // device [n_ctx]: cell_shift staged for the K re-rotation
     int rope_off = 0;                               // rotary position of the next token - n_past
-    bool shift_pending = false;
+    bool shift_pending = false;                     // some cell_shift is non-zero: applied to the K rows before the cache is read
     static constexpr int TOK_RING = 256;
     int32_t* h_tok = nullptr;             // pinned ring [TOK_RING]
     int tok_slot = 0;

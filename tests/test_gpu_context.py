@@ -221,3 +221,66 @@ def test_self_extend_session_follows_the_reference_schedule(gguf_path, oracle):
     print(f"\n[self-extend session] ga index {ga_i} after 120 tokens, max |dlogit| on the reported top-10 = {worst:.3g}")
     assert ga_i >= 3 * (W // F) and worst <= ps.FLIP_TOL, (ga_i, worst)
     oc.close(); om.close(); hm.close()
+
+
+@pytest.mark.parametrize("persistent", [True, False], ids=["persistent", "per-op"])
+def test_profile_step_adds_its_cell_like_decode(persistent, gguf_path, monkeypatch):
+    """blk_profile_step between Self-Extend regroupings: the pending K re-rotation is applied before the step and the new cell's
+    position is recorded for the next regrouping, exactly as blk_decode does it (BLK_MEGA=0: the eagerly enqueued per-op step)"""
+    from blama_b200 import capi
+
+    name, F, W = "small-llama-q4km", 2, 32
+    if not persistent:
+        monkeypatch.setenv("BLK_MEGA", "0")                  # read when the model is loaded
+    m = capi.Model(gguf_path(name))
+    monkeypatch.delenv("BLK_MEGA", raising=False)
+    a, b = capi.Ctx(m, 256), capi.Ctx(m, 256)
+    assert a.persistent_decode == persistent
+    toks = [int(t) for t in gs.synth_prompt(name, 69, 61)]
+    a.decode(toks[:40]); b.decode(toks[:40])
+    n_pos, ga_i, regroups = 40, 0, 0
+    for t in toks[40:68]:
+        before = ga_i
+        n_pos, ga_i = _regroup([a, b], n_pos, ga_i, F, W)
+        regroups += ga_i != before
+        a.profile_step(t); b.decode([t])
+        n_pos += 1
+        assert np.array_equal(a.logits(), b.logits())
+        assert a.n_past == b.n_past and a.next_pos == b.next_pos == n_pos
+    assert regroups >= 2
+    a.decode([toks[68]]); b.decode([toks[68]])
+    assert np.array_equal(a.logits(), b.logits())
+    a.close(); b.close(); m.close()
+
+
+def test_profile_step_rejects_a_bad_token(gguf_path):
+    from blama_b200 import capi
+
+    name = "small-llama-q4km"
+    m = capi.Model(gguf_path(name)); c = capi.Ctx(m, 64)
+    c.decode([int(t) for t in gs.synth_prompt(name, 5, 3)])
+    for bad in (m.n_vocab, -1):
+        with pytest.raises(capi.BlkError):
+            c.profile_step(bad)
+        assert c.n_past == 5
+    c.close(); m.close()
+
+
+def test_bench_kernel_resets_the_context(gguf_path, monkeypatch):
+    """the per-op kernel benchmark leaves an empty context behind, Self-Extend positions included"""
+    from blama_b200 import capi
+
+    name = "small-llama-q4km"
+    monkeypatch.setenv("BLK_MEGA", "0")                      # the kernels of the per-op step, as bench.py times them
+    m = capi.Model(gguf_path(name))
+    monkeypatch.delenv("BLK_MEGA", raising=False)
+    c, fresh = capi.Ctx(m, 256), capi.Ctx(m, 256)
+    toks = [int(t) for t in gs.synth_prompt(name, 52, 9)]
+    c.decode(toks[:40])
+    _regroup([c], 40, 0, 2, 32)
+    assert c.next_pos != c.n_past
+    c.bench_kernel(0, 4)
+    assert c.n_past == 0 and c.next_pos == 0
+    c.decode(toks[40:]); fresh.decode(toks[40:])
+    assert np.array_equal(c.logits(), fresh.logits())
+    c.close(); fresh.close(); m.close()
