@@ -71,6 +71,9 @@ SYMBOLS = {
     "blk_decode_topk": (_i32, [_vp, _i32, _i32, _vp]),
     "blk_decode_loop": (_i32, [_vp, _i32, _i32, C.POINTER(_i32)]),
     "blk_decode_batch": (_i32, [_vp, _vp, _vp, _i32, _i32, _vp]),
+    "blk_decode_topk_edited": (_i32, [_vp, _i32, _i32, _vp, _vp, _vp]),
+    "blk_topk_last_edited": (_i32, [_vp, _i32, _vp, _vp]),
+    "blk_decode_batch_edited": (_i32, [_vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp]),
     "blk_verify_prefill": (_i32, [_vp, _vp, _i32, _vp, _vp, _vp, _vp]),
     "blk_ctx_set_verify_mode": (_i32, [_vp, _i32]),
     "blk_timer_start": (_i32, [_vp]),
@@ -91,6 +94,7 @@ SYMBOLS = {
     "blk_test_prefill_attn": (_i32, [_i32, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp, C.POINTER(_i32)]),
     "blk_test_decode_attn": (_i32, [_i32, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i64, _vp, C.POINTER(_i32)]),
     "blk_test_decode_attn_batch": (_i32, [_i32, _i32, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i64, _vp]),
+    "blk_test_logit_edits": (_i32, [_i32, _vp, _i32, _i32, _vp, _i32, _vp]),
 }
 
 _lib: Optional[C.CDLL] = None
@@ -181,7 +185,39 @@ def test_decode_attn_batch(q: np.ndarray, k: np.ndarray, v: np.ndarray, n_kv: Se
     return out
 
 
+EDIT_DTYPE = np.dtype([("token", np.int32), ("count", np.int32), ("bias", np.float32)])     # blk_logit_edit
+
+
+class LogitEdits(C.Structure):
+    """blk_logit_edits: one row's (repeat, freq, present) and its edit list, ids ascending"""
+    _fields_ = [("repeat", C.c_float), ("freq", C.c_float), ("present", C.c_float), ("edits", C.c_void_p), ("n_edits", C.c_int32)]
+
+
+def logit_edits(edits=None, repeat: float = 1.0, freq: float = 0.0, present: float = 0.0):
+    """(LogitEdits, the array it points into) from [(token, count, bias), ...] or an EDIT_DTYPE array; keep both alive while in use"""
+    arr = np.zeros(0, dtype=EDIT_DTYPE) if edits is None else (np.ascontiguousarray(edits) if isinstance(edits, np.ndarray)
+                                                               else np.array([tuple(e) for e in edits], dtype=EDIT_DTYPE))
+    assert arr.dtype == EDIT_DTYPE
+    return LogitEdits(repeat, freq, present, arr.ctypes.data if len(arr) else None, len(arr)), arr
+
+
+def _edit_rows(per_row):
+    """[(edits, repeat, freq, present), ...] -> (LogitEdits array, arrays to keep alive)"""
+    made = [logit_edits(*r) for r in per_row]
+    return (LogitEdits * len(made))(*[m[0] for m in made]), [m[1] for m in made]
+
+
+def test_logit_edits(logits: np.ndarray, per_row, k: int = 64, device: int = 0) -> np.ndarray:
+    """edited top-k of every row of logits [n][V]; per_row[i] = (edits, repeat, freq, present) as logit_edits takes them"""
+    lg = np.ascontiguousarray(logits, dtype=np.float32).reshape(len(per_row), -1)
+    rows, keep = _edit_rows(per_row)
+    out = np.zeros((lg.shape[0], k), dtype=TD_DTYPE)
+    _check(lib().blk_test_logit_edits(device, _p(lg), lg.shape[0], lg.shape[1], C.cast(rows, C.c_void_p), k, _p(out)))
+    return out
+
+
 test_rmsnorm.__test__ = test_qkv_post.__test__ = test_prefill_attn.__test__ = False      # (not pytest tests)
+test_logit_edits.__test__ = False
 test_decode_attn.__test__ = test_decode_attn_batch.__test__ = False
 
 
@@ -193,6 +229,17 @@ def decode_batch(ws: "Ctx", ctxs: Sequence["Ctx"], tokens: Sequence[int], k: int
     out = np.zeros((n, k), dtype=TD_DTYPE)
     _check(lib().blk_decode_batch(ws.h, arr, _p(t), n, k, _p(out)))
     return out
+
+
+def decode_batch_edited(ws: "Ctx", ctxs: Sequence["Ctx"], tokens: Sequence[int], per_row, k: int = 64):
+    """blk_decode_batch_edited: (raw [n][k], edited [n][k]); per_row[i] = (edits, repeat, freq, present)"""
+    n = len(ctxs)
+    arr = (_vp * n)(*[c.h for c in ctxs])
+    t = np.ascontiguousarray(tokens, dtype=np.int32)
+    rows, keep = _edit_rows(per_row)
+    raw = np.zeros((n, k), dtype=TD_DTYPE); ed = np.zeros((n, k), dtype=TD_DTYPE)
+    _check(lib().blk_decode_batch_edited(ws.h, arr, _p(t), n, k, C.cast(rows, C.c_void_p), _p(raw), _p(ed)))
+    return raw, ed
 
 
 def device_count() -> int:
@@ -295,6 +342,19 @@ class Ctx:
     def decode_topk(self, token: int, k: int = 40) -> np.ndarray:
         out = np.zeros(k, dtype=TD_DTYPE)
         _check(lib().blk_decode_topk(self.h, int(token), k, _p(out)))
+        return out
+
+    def decode_topk_edited(self, token: int, edits=None, repeat: float = 1.0, freq: float = 0.0, present: float = 0.0, k: int = 64):
+        """blk_decode_topk_edited: (raw top-k, edited top-k)"""
+        e, keep = logit_edits(edits, repeat, freq, present)
+        raw = np.zeros(k, dtype=TD_DTYPE); ed = np.zeros(k, dtype=TD_DTYPE)
+        _check(lib().blk_decode_topk_edited(self.h, int(token), k, C.byref(e), _p(raw), _p(ed)))
+        return raw, ed
+
+    def topk_edited(self, edits=None, repeat: float = 1.0, freq: float = 0.0, present: float = 0.0, k: int = 64) -> np.ndarray:
+        e, keep = logit_edits(edits, repeat, freq, present)
+        out = np.zeros(k, dtype=TD_DTYPE)
+        _check(lib().blk_topk_last_edited(self.h, k, C.byref(e), _p(out)))
         return out
 
     def decode_loop(self, first_token: int, n_steps: int, wait: bool = True) -> int:

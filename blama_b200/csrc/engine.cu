@@ -9,6 +9,7 @@
 #include "prefill.hpp"
 #include "prefill_kernels.cuh"
 #include "batch_decode.cuh"
+#include "logit_edit.cuh"
 
 #include <algorithm>
 #include <atomic>
@@ -604,6 +605,13 @@ void matvec(blk_ctx* c, GemvArgs& a, const float* in, const float* norm_w, const
     prof_mark(c, name);
 }
 
+// vocabulary chunks of the threshold top-k: the smallest power of two >= 64 ids that leaves at most 256 chunks
+void set_chunking(blk_ctx* c, int n_vocab) {
+    c->chunk_shift = 6;
+    while (((n_vocab + (1 << c->chunk_shift) - 1) >> c->chunk_shift) > 256) c->chunk_shift++;
+    c->n_chunks = (n_vocab + (1 << c->chunk_shift) - 1) >> c->chunk_shift;
+}
+
 // the threshold top-k of the context's own logits row (c->logits -> c->top_ids / c->top_logits)
 TopkArgs own_topk_args(const blk_ctx* c) {
     TopkArgs tk{};
@@ -1092,6 +1100,108 @@ void topk_of_logits(blk_ctx* c) {
     BLK_CUDA(cudaMemcpyAsync(c->h_top_logits, c->top_logits, TOPK_MAX * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
 }
 
+// ---- logit edit pass (logit bias + repetition penalties, blk_*_edited) ----
+static_assert(sizeof(LogitEdit) == sizeof(blk_logit_edit) && offsetof(blk_logit_edit, bias) == offsetof(LogitEdit, bias));
+
+void dfree(blk_ctx* c, void* p) {
+    if (!p) return;
+    c->allocs.erase(std::remove(c->allocs.begin(), c->allocs.end(), p), c->allocs.end());
+    cudaFree(p);
+}
+void hfree(blk_ctx* c, void* p) {
+    if (!p) return;
+    c->host_allocs.erase(std::remove(c->host_allocs.begin(), c->host_allocs.end(), p), c->host_allocs.end());
+    cudaFreeHost(p);
+}
+
+// the edited rows and their top-k scratch for `rows` rows of n_vocab ids (grown, never shrunk; callers have synchronised)
+void ensure_edit_bufs(blk_ctx* c, int rows, int n_vocab) {
+    if (rows <= c->ed_rows) return;
+    for (void* p : {(void*)c->ed_logits, (void*)c->ed_chunk_max, (void*)c->ed_cand_l, (void*)c->ed_cand_i, (void*)c->ed_counters,
+                    (void*)c->ed_top_ids, (void*)c->ed_top_logits}) dfree(c, p);
+    hfree(c, c->ed_h_top_ids); hfree(c, c->ed_h_top_logits);
+    c->ed_rows = 0;
+    c->ed_logits = dalloc<float>(c, (size_t)rows * n_vocab);
+    c->ed_chunk_max = dalloc<int>(c, (size_t)rows * 256);
+    c->ed_cand_l = dalloc<float>(c, (size_t)rows * c->cand_cap); c->ed_cand_i = dalloc<int>(c, (size_t)rows * c->cand_cap);
+    c->ed_counters = dalloc<unsigned int>(c, 2 * (size_t)rows);
+    BLK_CUDA(cudaMemset(c->ed_counters, 0, 2 * (size_t)rows * sizeof(unsigned int)));
+    c->ed_top_ids = dalloc<int32_t>(c, (size_t)rows * TOPK_MAX); c->ed_top_logits = dalloc<float>(c, (size_t)rows * TOPK_MAX);
+    c->ed_h_top_ids = halloc<int32_t>(c, (size_t)rows * TOPK_MAX); c->ed_h_top_logits = halloc<float>(c, (size_t)rows * TOPK_MAX);
+    c->ed_rows = rows;
+}
+
+// Checks n rows of edit lists (they come from outside the library) and packs them into the pinned staging block as
+// [row][3] params | row_off[n + 1] | edits.  Runs before anything is launched, so a malformed list costs no launch.  Returns the
+// bytes to upload.  The staging block is reused: every caller has synchronised its previous upload.
+size_t pack_edits(blk_ctx* c, const blk_logit_edits* per_row, int n, int n_vocab) {
+    if (!per_row) throw BlkError(BLK_ERR_ARG, "logit edits: null edit list");
+    size_t total = 0;
+    for (int r = 0; r < n; r++) {
+        const blk_logit_edits& e = per_row[r];
+        if (!(std::isfinite(e.repeat) && e.repeat > 0.0f) || !std::isfinite(e.freq) || !std::isfinite(e.present))
+            throw BlkError(BLK_ERR_ARG, "logit edits: repeat must be finite and > 0, freq and present finite");
+        if (e.n_edits < 0 || (e.n_edits > 0 && !e.edits)) throw BlkError(BLK_ERR_ARG, "logit edits: bad edit count");
+        for (int i = 0; i < e.n_edits; i++) {
+            const blk_logit_edit& d = e.edits[i];
+            if (d.token < 0 || d.token >= n_vocab) throw BlkError(BLK_ERR_ARG, "logit edits: token id out of range");
+            if (i > 0 && d.token <= e.edits[i - 1].token) throw BlkError(BLK_ERR_ARG, "logit edits: token ids must be strictly ascending");
+            if (d.count < 0) throw BlkError(BLK_ERR_ARG, "logit edits: negative count");
+            if (std::isnan(d.bias) || d.bias == INFINITY) throw BlkError(BLK_ERR_ARG, "logit edits: bias is NaN or +inf");
+        }
+        total += (size_t)e.n_edits;
+    }
+    const size_t off_params = 0, off_rows = (size_t)n * 3 * sizeof(float), off_edits = off_rows + (size_t)(n + 1) * sizeof(int32_t);
+    const size_t bytes = off_edits + total * sizeof(blk_logit_edit);
+    if (bytes > c->ed_stage_cap) {
+        hfree(c, c->ed_stage_h); dfree(c, c->ed_stage_d);
+        c->ed_stage_h = nullptr; c->ed_stage_d = nullptr; c->ed_stage_cap = 0;
+        const size_t cap = std::max<size_t>(bytes * 2, 4096);
+        c->ed_stage_h = halloc<uint8_t>(c, cap); c->ed_stage_d = dalloc<uint8_t>(c, cap);
+        c->ed_stage_cap = cap;
+    }
+    float* params = reinterpret_cast<float*>(c->ed_stage_h + off_params);
+    int32_t* row_off = reinterpret_cast<int32_t*>(c->ed_stage_h + off_rows);
+    blk_logit_edit* edits = reinterpret_cast<blk_logit_edit*>(c->ed_stage_h + off_edits);
+    int32_t at = 0;
+    for (int r = 0; r < n; r++) {
+        const blk_logit_edits& e = per_row[r];
+        params[3 * r] = e.repeat; params[3 * r + 1] = e.freq; params[3 * r + 2] = e.present;
+        row_off[r] = at;
+        if (e.n_edits) memcpy(edits + at, e.edits, (size_t)e.n_edits * sizeof(blk_logit_edit));
+        at += e.n_edits;
+    }
+    row_off[n] = at;
+    return bytes;
+}
+
+// The edit pass over n rows of `logits` (ld floats apart) with the lists pack_edits staged: edited copies + their chunk maxima,
+// the threshold selector on them (blockIdx.y = row), the per-row top-64 copied to c->ed_h_top_* (the caller synchronises).
+void launch_edited_topk(blk_ctx* c, const float* logits, long long ld, int n, int n_vocab, size_t staged, cudaStream_t st) {
+    BLK_CUDA(cudaMemcpyAsync(c->ed_stage_d, c->ed_stage_h, staged, cudaMemcpyHostToDevice, st));
+    LogitEditArgs ea{};
+    ea.logits = logits; ea.ld = ld; ea.n = n_vocab;
+    ea.params = reinterpret_cast<const float*>(c->ed_stage_d);
+    ea.row_off = reinterpret_cast<const int32_t*>(c->ed_stage_d + (size_t)n * 3 * sizeof(float));
+    ea.edits = reinterpret_cast<const LogitEdit*>(c->ed_stage_d + (size_t)n * 3 * sizeof(float) + (size_t)(n + 1) * sizeof(int32_t));
+    ea.out = c->ed_logits; ea.chunk_max = c->ed_chunk_max; ea.chunk_shift = c->chunk_shift;
+    logit_edit_kernel<<<dim3(c->n_chunks, n), 256, (size_t)sizeof(float) << c->chunk_shift, st>>>(ea);
+    BLK_CUDA(cudaGetLastError());
+    TopkArgs tk{};
+    tk.logits = c->ed_logits; tk.n = n_vocab; tk.ld = n_vocab; tk.chunk_max = c->ed_chunk_max; tk.n_chunks = c->n_chunks;
+    tk.cand_l = c->ed_cand_l; tk.cand_i = c->ed_cand_i; tk.cap = c->cand_cap; tk.count = c->ed_counters; tk.done = c->ed_counters + 1;
+    tk.out_ids = c->ed_top_ids; tk.out_logits = c->ed_top_logits;
+    topk_select_kernel<<<dim3(16, n), 1024, 0, st>>>(tk);
+    BLK_CUDA(cudaGetLastError());
+    c->launches += 2;
+    BLK_CUDA(cudaMemcpyAsync(c->ed_h_top_ids, c->ed_top_ids, (size_t)n * TOPK_MAX * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    BLK_CUDA(cudaMemcpyAsync(c->ed_h_top_logits, c->ed_top_logits, (size_t)n * TOPK_MAX * sizeof(float), cudaMemcpyDeviceToHost, st));
+}
+
+void copy_edited_topk(const blk_ctx* c, int row, int k, blk_token_data* out) {
+    for (int j = 0; j < k; j++) { out[j].token = c->ed_h_top_ids[row * TOPK_MAX + j]; out[j].logit = c->ed_h_top_logits[row * TOPK_MAX + j]; }
+}
+
 // causal flash attention of a prefill chunk: the query heads of a KV head share a CTA when the GQA ratio is a power of two
 template <int DH, int GQ>
 void launch_attn_gqa(const PrefillAttnArgs& pa, int n, int n_head_kv, cudaStream_t st) {
@@ -1347,9 +1457,7 @@ extern "C" blk_ctx* blk_ctx_create(blk_model* m, int32_t n_ctx, int32_t n_batch)
         c->part_o = dalloc<float>(c.get(), (size_t)m->n_head * c->n_split * dh);
         c->scores = dalloc<float>(c.get(), (size_t)m->n_head * c->n_pages * KV_PAGE);
         c->logits = dalloc<float>(c.get(), m->n_vocab);
-        c->chunk_shift = 6;
-        while (((m->n_vocab + (1 << c->chunk_shift) - 1) >> c->chunk_shift) > 256) c->chunk_shift++;
-        c->n_chunks = (m->n_vocab + (1 << c->chunk_shift) - 1) >> c->chunk_shift;
+        set_chunking(c.get(), m->n_vocab);
         c->cand_l = dalloc<float>(c.get(), c->cand_cap); c->cand_i = dalloc<int>(c.get(), c->cand_cap);
         c->chunk_max = dalloc<int>(c.get(), 256);
         {
@@ -1563,88 +1671,109 @@ struct BatchDesc {       // layout of blk_ctx::bd_host / bd_dev
 };
 } // namespace
 
+namespace {
+// blk_decode_batch, and with per_row != nullptr blk_decode_batch_edited (edited[i * k ..] = row i's edited top-k)
+void decode_batch(blk_ctx* ws, blk_ctx* const* ctxs, const int32_t* tokens, int32_t n, int32_t k, blk_token_data* out,
+                  const blk_logit_edits* per_row, blk_token_data* edited) {
+    blk_model* m = ws->m;
+    BLK_CUDA(cudaSetDevice(m->device));
+    const int d = m->n_embd, dh = m->d_head, dq = m->n_head * dh, dkv = m->n_head_kv * dh, V = m->n_vocab;
+    for (int i = 0; i < n; i++) {
+        blk_ctx* c = ctxs[i];
+        if (!c || c->m != m) throw BlkError(BLK_ERR_ARG, "blk_decode_batch: every context must belong to the workspace's model");
+        for (int j = 0; j < i; j++) if (ctxs[j] == c) throw BlkError(BLK_ERR_ARG, "blk_decode_batch: a context appears twice");
+        check_cells(c, tokens + i, 1, 1);
+    }
+    size_t staged = 0;
+    if (per_row) {          // checked before anything is launched; the staging block is reused every step
+        BLK_CUDA(cudaStreamSynchronize(ws->stream));
+        staged = pack_edits(ws, per_row, n, V);
+        ensure_edit_bufs(ws, n, V);
+    }
+    ensure_prefill_bufs(ws, n);
+    if (!ws->bd_host) {
+        ws->bd_host = reinterpret_cast<uint8_t*>(halloc<BatchDesc>(ws, 1));
+        ws->bd_dev = reinterpret_cast<uint8_t*>(dalloc<BatchDesc>(ws, 1));
+        ws->bd_top_ids = dalloc<int32_t>(ws, BATCH_MAX * TOPK_MAX); ws->bd_top_logits = dalloc<float>(ws, BATCH_MAX * TOPK_MAX);
+        ws->bd_h_top_ids = halloc<int32_t>(ws, BATCH_MAX * TOPK_MAX); ws->bd_h_top_logits = halloc<float>(ws, BATCH_MAX * TOPK_MAX);
+        // per-row scratch of the batched threshold selector
+        ws->bd_chunk_max = dalloc<int>(ws, BATCH_MAX * 256);
+        { std::vector<int> init(BATCH_MAX * 256, (int)0x80000000); BLK_CUDA(cudaMemcpy(ws->bd_chunk_max, init.data(), init.size() * sizeof(int), cudaMemcpyHostToDevice)); }
+        ws->bd_cand_l = dalloc<float>(ws, (size_t)BATCH_MAX * ws->cand_cap); ws->bd_cand_i = dalloc<int>(ws, (size_t)BATCH_MAX * ws->cand_cap);
+        ws->bd_counters = dalloc<unsigned int>(ws, 2 * BATCH_MAX);
+        BLK_CUDA(cudaMemset(ws->bd_counters, 0, 2 * BATCH_MAX * sizeof(unsigned int)));
+    }
+    cudaStream_t st = ws->stream;
+    BLK_CUDA(cudaStreamSynchronize(st));                      // the staging block is reused every step
+    BatchDesc* h = reinterpret_cast<BatchDesc*>(ws->bd_host);
+    const BatchDesc* dv = reinterpret_cast<const BatchDesc*>(ws->bd_dev);
+    for (int i = 0; i < n; i++) {
+        blk_ctx* c = ctxs[i];
+        BLK_CUDA(cudaStreamSynchronize(c->stream));          // its prompt prefill / previous step ran on its own stream
+        begin_cells(c, tokens + i, 1, 1);
+        h->tokens[i] = tokens[i]; h->pos[i] = c->n_past; h->rpos[i] = c->n_past + c->rope_off; h->page_table[i] = c->page_table;
+        h->k_pools[i] = c->d_kpools; h->v_pools[i] = c->d_vpools; h->pos_ptr[i] = c->d_pos;
+    }
+    BLK_CUDA(cudaMemcpyAsync(ws->bd_dev, ws->bd_host, sizeof(BatchDesc), cudaMemcpyHostToDevice, st));
+    embed_rows_kernel<<<n, 256, 0, st>>>(m->tok_embd, dv->tokens, dv->rpos, ws->pf_x, ws->pf_rope, dh / 2, m->theta_scale, m->rope_freqs);
+    BLK_CUDA(cudaGetLastError()); ws->launches++;
+    const ChainPdl chain_scope(n);
+    // matrices with a resident bf16 panel (model cache) take the TMA-fed GEMM: the step then streams the panels at HBM speed
+    // instead of waiting for the de-quantising producers of the fused form (BATCH_MAX rows are below the default panel_min)
+    GemmSchedule sched(ws, n, n_gemm_ops(m));
+    PendingReduce pend;
+    run_layers(ws, n, sched, pend, true, [&](int l) {
+        QkvPostBatchArgs qa{};
+        qa.base.qkv = ws->pf_qkv; qa.base.ld = dq + 2 * dkv; qa.base.rope_cs = ws->pf_rope; qa.base.q_out = ws->pf_q;
+        qa.base.dq = dq; qa.base.dkv = dkv; qa.base.d_head = dh; qa.base.neox = m->neox ? 1 : 0;
+        qa.pos = dv->pos; qa.page_table = dv->page_table; qa.k_pools = dv->k_pools; qa.v_pools = dv->v_pools; qa.layer = l;
+        BLK_CUDA(launch_chain(qkv_post_batch_kernel, dim3(n), dim3(256), 0, st, qa));
+        BatchAttnArgs aa{};
+        aa.q = ws->pf_q; aa.pos = dv->pos; aa.page_table = dv->page_table; aa.k_pools = dv->k_pools; aa.v_pools = dv->v_pools; aa.out = ws->pf_ao;
+        aa.layer = l; aa.n_head = m->n_head; aa.n_head_kv = m->n_head_kv; aa.kv_dim = dkv; aa.scale = 1.0f / sqrtf((float)dh);
+        if (dh == 128) BLK_CUDA(launch_chain(decode_attn_batch_kernel<128>, dim3(m->n_head_kv, n), dim3(256), 0, st, aa));
+        else BLK_CUDA(launch_chain(decode_attn_batch_kernel<64>, dim3(m->n_head_kv, n), dim3(256), 0, st, aa));
+        BLK_CUDA(cudaGetLastError());
+        ws->launches += 2;
+    });
+    rmsnorm_bf16_launch(ws->pf_x, m->out_norm, d, m->rms_eps, ws->pf_xn, n, st, &pend);
+    const GemmOp head = sched.next(OP_HEAD);
+    BLK_CUDA(prefill_gemm(*head.part[0].W, ws->pf_xn, n, ws->pf_logits, V, nullptr, 0, st, head.panel));
+    ws->launches += 2;
+    // threshold top-64 of every row (the selector of the batch-1 path, blockIdx.y = row): two launches for the whole batch
+    {
+        chunk_max_kernel<<<dim3(ws->n_chunks, n), 256, 0, st>>>(ws->pf_logits, V, ws->chunk_shift, ws->bd_chunk_max, (long long)V);
+        TopkArgs tk{};
+        tk.logits = ws->pf_logits; tk.n = V; tk.ld = V; tk.chunk_max = ws->bd_chunk_max; tk.n_chunks = ws->n_chunks;
+        tk.cand_l = ws->bd_cand_l; tk.cand_i = ws->bd_cand_i; tk.cap = ws->cand_cap; tk.count = ws->bd_counters; tk.done = ws->bd_counters + 1;
+        tk.out_ids = ws->bd_top_ids; tk.out_logits = ws->bd_top_logits;
+        topk_select_kernel<<<dim3(16, n), 1024, 0, st>>>(tk);
+        BLK_CUDA(cudaGetLastError()); ws->launches += 2;
+    }
+    if (per_row) launch_edited_topk(ws, ws->pf_logits, V, n, V, staged, st);
+    advance_many_kernel<<<1, BATCH_MAX, 0, st>>>(dv->pos_ptr, n);
+    BLK_CUDA(cudaGetLastError()); ws->launches++;
+    BLK_CUDA(cudaMemcpyAsync(ws->bd_h_top_ids, ws->bd_top_ids, (size_t)n * TOPK_MAX * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    BLK_CUDA(cudaMemcpyAsync(ws->bd_h_top_logits, ws->bd_top_logits, (size_t)n * TOPK_MAX * sizeof(float), cudaMemcpyDeviceToHost, st));
+    BLK_CUDA(cudaStreamSynchronize(st));
+    for (int i = 0; i < n; i++) {
+        end_cells(ctxs[i], 1, false);
+        for (int j = 0; j < k; j++) { out[(size_t)i * k + j].token = ws->bd_h_top_ids[i * TOPK_MAX + j]; out[(size_t)i * k + j].logit = ws->bd_h_top_logits[i * TOPK_MAX + j]; }
+        if (per_row) copy_edited_topk(ws, i, k, edited + (size_t)i * k);
+    }
+}
+} // namespace
+
 extern "C" blk_status blk_decode_batch(blk_ctx* ws, blk_ctx* const* ctxs, const int32_t* tokens, int32_t n, int32_t k, blk_token_data* out) {
     if (!ws || !ctxs || !tokens || !out || n <= 0 || n > BATCH_MAX || k <= 0 || k > TOPK_MAX) return fail(BLK_ERR_ARG, "blk_decode_batch: bad arguments");
-    return guarded([&] {
-        blk_model* m = ws->m;
-        BLK_CUDA(cudaSetDevice(m->device));
-        const int d = m->n_embd, dh = m->d_head, dq = m->n_head * dh, dkv = m->n_head_kv * dh, V = m->n_vocab;
-        for (int i = 0; i < n; i++) {
-            blk_ctx* c = ctxs[i];
-            if (!c || c->m != m) throw BlkError(BLK_ERR_ARG, "blk_decode_batch: every context must belong to the workspace's model");
-            for (int j = 0; j < i; j++) if (ctxs[j] == c) throw BlkError(BLK_ERR_ARG, "blk_decode_batch: a context appears twice");
-            check_cells(c, tokens + i, 1, 1);
-        }
-        ensure_prefill_bufs(ws, n);
-        if (!ws->bd_host) {
-            ws->bd_host = reinterpret_cast<uint8_t*>(halloc<BatchDesc>(ws, 1));
-            ws->bd_dev = reinterpret_cast<uint8_t*>(dalloc<BatchDesc>(ws, 1));
-            ws->bd_top_ids = dalloc<int32_t>(ws, BATCH_MAX * TOPK_MAX); ws->bd_top_logits = dalloc<float>(ws, BATCH_MAX * TOPK_MAX);
-            ws->bd_h_top_ids = halloc<int32_t>(ws, BATCH_MAX * TOPK_MAX); ws->bd_h_top_logits = halloc<float>(ws, BATCH_MAX * TOPK_MAX);
-            // per-row scratch of the batched threshold selector
-            ws->bd_chunk_max = dalloc<int>(ws, BATCH_MAX * 256);
-            { std::vector<int> init(BATCH_MAX * 256, (int)0x80000000); BLK_CUDA(cudaMemcpy(ws->bd_chunk_max, init.data(), init.size() * sizeof(int), cudaMemcpyHostToDevice)); }
-            ws->bd_cand_l = dalloc<float>(ws, (size_t)BATCH_MAX * ws->cand_cap); ws->bd_cand_i = dalloc<int>(ws, (size_t)BATCH_MAX * ws->cand_cap);
-            ws->bd_counters = dalloc<unsigned int>(ws, 2 * BATCH_MAX);
-            BLK_CUDA(cudaMemset(ws->bd_counters, 0, 2 * BATCH_MAX * sizeof(unsigned int)));
-        }
-        cudaStream_t st = ws->stream;
-        BLK_CUDA(cudaStreamSynchronize(st));                      // the staging block is reused every step
-        BatchDesc* h = reinterpret_cast<BatchDesc*>(ws->bd_host);
-        const BatchDesc* dv = reinterpret_cast<const BatchDesc*>(ws->bd_dev);
-        for (int i = 0; i < n; i++) {
-            blk_ctx* c = ctxs[i];
-            BLK_CUDA(cudaStreamSynchronize(c->stream));          // its prompt prefill / previous step ran on its own stream
-            begin_cells(c, tokens + i, 1, 1);
-            h->tokens[i] = tokens[i]; h->pos[i] = c->n_past; h->rpos[i] = c->n_past + c->rope_off; h->page_table[i] = c->page_table;
-            h->k_pools[i] = c->d_kpools; h->v_pools[i] = c->d_vpools; h->pos_ptr[i] = c->d_pos;
-        }
-        BLK_CUDA(cudaMemcpyAsync(ws->bd_dev, ws->bd_host, sizeof(BatchDesc), cudaMemcpyHostToDevice, st));
-        embed_rows_kernel<<<n, 256, 0, st>>>(m->tok_embd, dv->tokens, dv->rpos, ws->pf_x, ws->pf_rope, dh / 2, m->theta_scale, m->rope_freqs);
-        BLK_CUDA(cudaGetLastError()); ws->launches++;
-        const ChainPdl chain_scope(n);
-        // matrices with a resident bf16 panel (model cache) take the TMA-fed GEMM: the step then streams the panels at HBM speed
-        // instead of waiting for the de-quantising producers of the fused form (BATCH_MAX rows are below the default panel_min)
-        GemmSchedule sched(ws, n, n_gemm_ops(m));
-        PendingReduce pend;
-        run_layers(ws, n, sched, pend, true, [&](int l) {
-            QkvPostBatchArgs qa{};
-            qa.base.qkv = ws->pf_qkv; qa.base.ld = dq + 2 * dkv; qa.base.rope_cs = ws->pf_rope; qa.base.q_out = ws->pf_q;
-            qa.base.dq = dq; qa.base.dkv = dkv; qa.base.d_head = dh; qa.base.neox = m->neox ? 1 : 0;
-            qa.pos = dv->pos; qa.page_table = dv->page_table; qa.k_pools = dv->k_pools; qa.v_pools = dv->v_pools; qa.layer = l;
-            BLK_CUDA(launch_chain(qkv_post_batch_kernel, dim3(n), dim3(256), 0, st, qa));
-            BatchAttnArgs aa{};
-            aa.q = ws->pf_q; aa.pos = dv->pos; aa.page_table = dv->page_table; aa.k_pools = dv->k_pools; aa.v_pools = dv->v_pools; aa.out = ws->pf_ao;
-            aa.layer = l; aa.n_head = m->n_head; aa.n_head_kv = m->n_head_kv; aa.kv_dim = dkv; aa.scale = 1.0f / sqrtf((float)dh);
-            if (dh == 128) BLK_CUDA(launch_chain(decode_attn_batch_kernel<128>, dim3(m->n_head_kv, n), dim3(256), 0, st, aa));
-            else BLK_CUDA(launch_chain(decode_attn_batch_kernel<64>, dim3(m->n_head_kv, n), dim3(256), 0, st, aa));
-            BLK_CUDA(cudaGetLastError());
-            ws->launches += 2;
-        });
-        rmsnorm_bf16_launch(ws->pf_x, m->out_norm, d, m->rms_eps, ws->pf_xn, n, st, &pend);
-        const GemmOp head = sched.next(OP_HEAD);
-        BLK_CUDA(prefill_gemm(*head.part[0].W, ws->pf_xn, n, ws->pf_logits, V, nullptr, 0, st, head.panel));
-        ws->launches += 2;
-        // threshold top-64 of every row (the selector of the batch-1 path, blockIdx.y = row): two launches for the whole batch
-        {
-            chunk_max_kernel<<<dim3(ws->n_chunks, n), 256, 0, st>>>(ws->pf_logits, V, ws->chunk_shift, ws->bd_chunk_max, (long long)V);
-            TopkArgs tk{};
-            tk.logits = ws->pf_logits; tk.n = V; tk.ld = V; tk.chunk_max = ws->bd_chunk_max; tk.n_chunks = ws->n_chunks;
-            tk.cand_l = ws->bd_cand_l; tk.cand_i = ws->bd_cand_i; tk.cap = ws->cand_cap; tk.count = ws->bd_counters; tk.done = ws->bd_counters + 1;
-            tk.out_ids = ws->bd_top_ids; tk.out_logits = ws->bd_top_logits;
-            topk_select_kernel<<<dim3(16, n), 1024, 0, st>>>(tk);
-            BLK_CUDA(cudaGetLastError()); ws->launches += 2;
-        }
-        advance_many_kernel<<<1, BATCH_MAX, 0, st>>>(dv->pos_ptr, n);
-        BLK_CUDA(cudaGetLastError()); ws->launches++;
-        BLK_CUDA(cudaMemcpyAsync(ws->bd_h_top_ids, ws->bd_top_ids, (size_t)n * TOPK_MAX * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        BLK_CUDA(cudaMemcpyAsync(ws->bd_h_top_logits, ws->bd_top_logits, (size_t)n * TOPK_MAX * sizeof(float), cudaMemcpyDeviceToHost, st));
-        BLK_CUDA(cudaStreamSynchronize(st));
-        for (int i = 0; i < n; i++) {
-            end_cells(ctxs[i], 1, false);
-            for (int j = 0; j < k; j++) { out[(size_t)i * k + j].token = ws->bd_h_top_ids[i * TOPK_MAX + j]; out[(size_t)i * k + j].logit = ws->bd_h_top_logits[i * TOPK_MAX + j]; }
-        }
-    });
+    return guarded([&] { decode_batch(ws, ctxs, tokens, n, k, out, nullptr, nullptr); });
+}
+
+extern "C" blk_status blk_decode_batch_edited(blk_ctx* ws, blk_ctx* const* ctxs, const int32_t* tokens, int32_t n, int32_t k,
+                                              const blk_logit_edits* per_row, blk_token_data* raw, blk_token_data* edited) {
+    if (!ws || !ctxs || !tokens || !per_row || !raw || !edited || n <= 0 || n > BATCH_MAX || k <= 0 || k > TOPK_MAX)
+        return fail(BLK_ERR_ARG, "blk_decode_batch_edited: bad arguments");
+    return guarded([&] { decode_batch(ws, ctxs, tokens, n, k, raw, per_row, edited); });
 }
 
 extern "C" blk_status blk_decode_loop(blk_ctx* c, int32_t first_token, int32_t n_steps, int32_t* last_token) {
@@ -1676,6 +1805,41 @@ extern "C" blk_status blk_topk_last(blk_ctx* c, int32_t k, blk_token_data* out) 
         BLK_CUDA(cudaStreamSynchronize(c->stream));
         check_mega(c);
         for (int i = 0; i < k; i++) { out[i].token = c->h_top_ids[i]; out[i].logit = c->h_top_logits[i]; }
+    });
+}
+
+extern "C" blk_status blk_topk_last_edited(blk_ctx* c, int32_t k, const blk_logit_edits* edits, blk_token_data* edited) {
+    if (!c || !edits || !edited || k <= 0 || k > TOPK_MAX) return fail(BLK_ERR_ARG, "blk_topk_last_edited: bad arguments");
+    return guarded([&] {
+        if (!c->have_logits) throw BlkError(BLK_ERR_ARG, "no logits available: decode first");
+        BLK_CUDA(cudaSetDevice(c->m->device));
+        BLK_CUDA(cudaStreamSynchronize(c->stream));
+        check_mega(c);
+        const int V = c->m->n_vocab;
+        const size_t staged = pack_edits(c, edits, 1, V);
+        ensure_edit_bufs(c, 1, V);
+        launch_edited_topk(c, c->logits, V, 1, V, staged, c->stream);
+        BLK_CUDA(cudaStreamSynchronize(c->stream));
+        copy_edited_topk(c, 0, k, edited);
+    });
+}
+
+extern "C" blk_status blk_decode_topk_edited(blk_ctx* c, int32_t token, int32_t k, const blk_logit_edits* edits, blk_token_data* raw,
+                                             blk_token_data* edited) {
+    if (!c || !edits || !raw || !edited || k <= 0 || k > TOPK_MAX) return fail(BLK_ERR_ARG, "blk_decode_topk_edited: bad arguments");
+    return guarded([&] {
+        BLK_CUDA(cudaSetDevice(c->m->device));
+        BLK_CUDA(cudaStreamSynchronize(c->stream));            // the edit staging block is reused every call
+        const int V = c->m->n_vocab;
+        const size_t staged = pack_edits(c, edits, 1, V);
+        ensure_edit_bufs(c, 1, V);
+        step(c, token, true);
+        // after the step's own selection (persistent kernel) or graph replay (per-op path), eagerly on the same stream
+        launch_edited_topk(c, c->logits, V, 1, V, staged, c->stream);
+        BLK_CUDA(cudaStreamSynchronize(c->stream));
+        check_mega(c);
+        for (int i = 0; i < k; i++) { raw[i].token = c->h_top_ids[i]; raw[i].logit = c->h_top_logits[i]; }
+        copy_edited_topk(c, 0, k, edited);
     });
 }
 
@@ -1947,6 +2111,27 @@ void test_upload(TestMat& tm, int device, int type, const void* blocks, int64_t 
 }
 __global__ void test_dequant_kernel(QMat W, float* out) { dequant_row_cta(W, blockIdx.x, out + (size_t)blockIdx.x * W.K); }
 } // namespace
+
+extern "C" blk_status blk_test_logit_edits(int32_t device, const float* logits, int32_t n_rows, int32_t n_vocab, const blk_logit_edits* per_row,
+                                           int32_t k, blk_token_data* out) {
+    if (!logits || !out || n_rows <= 0 || n_rows > BATCH_MAX || n_vocab <= 0 || n_vocab % 2 || k <= 0 || k > TOPK_MAX)
+        return fail(BLK_ERR_ARG, "blk_test_logit_edits: bad arguments");
+    return guarded([&] {
+        if (blk_init() != BLK_OK) throw BlkError(BLK_ERR_NO_DEVICE, g_last_error);
+        blk_model holder; holder.device = device;
+        blk_ctx c; c.m = &holder;
+        BLK_CUDA(cudaSetDevice(device));
+        set_chunking(&c, n_vocab);
+        const size_t staged = pack_edits(&c, per_row, n_rows, n_vocab);
+        BLK_CUDA(cudaStreamCreateWithFlags(&c.stream, cudaStreamNonBlocking));
+        ensure_edit_bufs(&c, n_rows, n_vocab);
+        float* d_logits = dalloc<float>(&c, (size_t)n_rows * n_vocab);
+        BLK_CUDA(cudaMemcpyAsync(d_logits, logits, (size_t)n_rows * n_vocab * sizeof(float), cudaMemcpyHostToDevice, c.stream));
+        launch_edited_topk(&c, d_logits, n_vocab, n_rows, n_vocab, staged, c.stream);
+        BLK_CUDA(cudaStreamSynchronize(c.stream));
+        for (int r = 0; r < n_rows; r++) copy_edited_topk(&c, r, k, out + (size_t)r * k);
+    });
+}
 
 extern "C" blk_status blk_test_dequant(int32_t device, int32_t type, const void* blocks, int64_t rows, int64_t k, float* out) {
     return guarded([&] {

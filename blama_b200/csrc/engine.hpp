@@ -155,6 +155,12 @@ struct blk_ctx {
     uint8_t* bd_host = nullptr; uint8_t* bd_dev = nullptr;
     int32_t* bd_top_ids = nullptr; float* bd_top_logits = nullptr; int32_t* bd_h_top_ids = nullptr; float* bd_h_top_logits = nullptr;
     int* bd_chunk_max = nullptr; float* bd_cand_l = nullptr; int* bd_cand_i = nullptr; unsigned int* bd_counters = nullptr;      // [row][...] scratch of the batched top-k
+    // logit edit pass (blk_*_edited, logit_edit.cuh), allocated on first use for ed_rows rows: the edited copies and a top-k scratch
+    // of their own (the raw selection's scratch and results stay untouched), plus the packed edit lists (pinned staging + device copy)
+    int ed_rows = 0;
+    float* ed_logits = nullptr; int* ed_chunk_max = nullptr; float* ed_cand_l = nullptr; int* ed_cand_i = nullptr; unsigned int* ed_counters = nullptr;
+    int32_t* ed_top_ids = nullptr; float* ed_top_logits = nullptr; int32_t* ed_h_top_ids = nullptr; float* ed_h_top_logits = nullptr;
+    uint8_t* ed_stage_h = nullptr; uint8_t* ed_stage_d = nullptr; size_t ed_stage_cap = 0;
     // persistent decode kernel (one cooperative launch per token instead of the per-op graph)
     bool mega_on = false;
     blk::MegaParams mega_params{};

@@ -92,6 +92,16 @@ server::Server::CompleteReponse responseOf(const int32_t* toks, int n, const blk
     }
     return resp;
 }
+// the logit-bias and repetition-penalty stages of a Sampler::Params from C arrays
+void setStages(Sampler::Params& sp, int32_t last_n, float repeat, float freq, float present, const int32_t* bias_ids, const float* bias_vals, int n_bias) {
+    sp.repetitionPenalty = {last_n, repeat, freq, present};
+    for (int i = 0; i < n_bias; ++i) sp.logitBias[bias_ids[i]] = bias_vals[i];
+}
+void writeEdits(const Sampler::LogitEdits& e, blk_logit_edit* out, int cap, int32_t* n, float* out3) {
+    *n = int32_t(e.edits.size());
+    for (size_t j = 0; j < e.edits.size() && int(j) < cap; ++j) out[j] = {e.edits[j].token, e.edits[j].count, e.edits[j].bias};
+    out3[0] = e.repeat; out3[1] = e.freq; out3[2] = e.present;
+}
 } // namespace
 
 extern "C" {
@@ -237,6 +247,28 @@ BLK_API int blh_session_start_ex(void* i, uint32_t seed, float temp, float top_p
     });
 }
 
+// Session::resetSampler with the reference's chain plus logit bias / repetition penalties (bias_ids / bias_vals: n_bias map entries)
+BLK_API int blh_session_reset_sampler(void* i, uint32_t seed, float temp, float top_p, int32_t last_n, float repeat, float freq, float present,
+                                      const int32_t* bias_ids, const float* bias_vals, int n_bias) {
+    return guard([&] {
+        Sampler::Params sp; sp.rngSeed = seed; sp.temp = temp; sp.topP = top_p;
+        setStages(sp, last_n, repeat, freq, present, bias_ids, bias_vals, n_bias);
+        static_cast<InstanceBox*>(i)->session->resetSampler(sp);
+    });
+}
+// the session sampler's current edit list (Session::logitEdits): *n entries (at most cap written), out3 = repeat, freq, present
+BLK_API int blh_session_logit_edits(void* i, blk_logit_edit* out, int cap, int32_t* n, float* out3) {
+    return guard([&] { writeEdits(static_cast<InstanceBox*>(i)->session->logitEdits(), out, cap, n, out3); });
+}
+// Session::samplingCandidates: *n entries, at most cap written
+BLK_API int blh_session_candidates(void* i, blk_token_data* out, int cap, int32_t* n) {
+    return guard([&] {
+        const auto c = static_cast<InstanceBox*>(i)->session->samplingCandidates();
+        *n = int32_t(c.size());
+        for (size_t j = 0; j < c.size() && int(j) < cap; ++j) out[j] = {c[j].token, c[j].logit};
+    });
+}
+
 // ---- verdict -------------------------------------------------------------------------------------------------------
 BLK_API void blh_lc_compare(const blk_token_data* a, int32_t na, const blk_token_data* b, int32_t nb, float* out3) {
     auto m = compareChecked(toVec(a, na < 0 ? 0 : na), toVec(b, nb < 0 ? 0 : nb));
@@ -262,6 +294,51 @@ BLK_API int blh_sampler_draw(uint32_t seed, float temp, float top_p, int32_t top
         Sampler s(*none, sp);
         auto v = toVec(cand, n_cand);
         for (int32_t i = 0; i < n_draws; ++i) out[i] = s.sample(v, sorted != 0);
+    });
+}
+
+// The full-row path with logit bias and penalties: accepts `history`, then n_draws times edits a copy of the row (n_vocab logits)
+// with the window so far, draws from it (unsorted, as Session does with the whole vocabulary) and accepts the draw.
+BLK_API int blh_sampler_draw_penalized(uint32_t seed, float temp, float top_p, int32_t top_k, float min_p, int32_t min_keep,
+                                       int32_t last_n, float repeat, float freq, float present, const int32_t* bias_ids, const float* bias_vals, int n_bias,
+                                       const int32_t* history, int32_t n_history, const float* logits, int32_t n_vocab, int32_t n_draws, int32_t* out) {
+    return guard([&] {
+        Sampler::Params sp; sp.rngSeed = seed; sp.temp = temp; sp.topP = top_p; sp.topK = top_k; sp.minP = min_p; sp.minKeep = min_keep;
+        setStages(sp, last_n, repeat, freq, present, bias_ids, bias_vals, n_bias);
+        Model* none = nullptr;
+        Sampler s(*none, sp);
+        for (int32_t i = 0; i < n_history; ++i) s.accept(history[i], false);
+        std::vector<float> row(static_cast<size_t>(n_vocab));
+        TokenDataVector all(static_cast<size_t>(n_vocab));
+        for (int32_t d = 0; d < n_draws; ++d) {
+            row.assign(logits, logits + n_vocab);
+            s.applyEdits(row);
+            for (int32_t t = 0; t < n_vocab; ++t) all[size_t(t)] = {t, row[size_t(t)]};
+            out[d] = s.sample(all, false);
+            s.accept(out[d], true);
+        }
+    });
+}
+// constructs a Sampler with the given mirostat version / grammar (the stages this build refuses): 0 when it is accepted
+BLK_API int blh_sampler_check(int32_t mirostat, const char* grammar) {
+    return guard([&] {
+        Sampler::Params sp; sp.mirostat.ver = mirostat; sp.grammar = grammar ? grammar : "";
+        Model* none = nullptr;
+        Sampler s(*none, sp);
+    });
+}
+// Sampler::logitEdits after accepting `history` (and a reset() afterwards when reset_after != 0)
+BLK_API int blh_sampler_logit_edits(int32_t last_n, float repeat, float freq, float present, const int32_t* bias_ids, const float* bias_vals, int n_bias,
+                                    const int32_t* history, int32_t n_history, int32_t reset_after, int32_t n_vocab,
+                                    blk_logit_edit* out, int cap, int32_t* n, float* out3) {
+    return guard([&] {
+        Sampler::Params sp;
+        setStages(sp, last_n, repeat, freq, present, bias_ids, bias_vals, n_bias);
+        Model* none = nullptr;
+        Sampler s(*none, sp);
+        for (int32_t i = 0; i < n_history; ++i) s.accept(history[i], false);
+        if (reset_after) s.reset();
+        writeEdits(s.logitEdits(n_vocab), out, cap, n, out3);
     });
 }
 
@@ -303,6 +380,21 @@ BLK_API int blh_server_submit_complete(void* s, const int32_t* prompt, int n_pro
         auto* box = static_cast<ServerBox*>(s);
         auto [id, t] = box->open();
         server::Server::CompleteRequestParams p; p.maxTokens = max_tokens; p.seed = seed; p.temperature = temp; p.topP = top_p;
+        box->srv->completeTokens(std::vector<int32_t>(prompt, prompt + n_prompt), std::move(p),
+                                 [box, t = t](server::Server::CompleteReponse r) { t->response = std::move(r); box->finish(t); });
+        *ticket = id;
+    });
+}
+// the same with the request's logit bias / repetition penalties (CompleteRequestParams extension)
+BLK_API int blh_server_submit_complete_ex(void* s, const int32_t* prompt, int n_prompt, uint32_t max_tokens, uint32_t seed, float temp, float top_p,
+                                          int32_t last_n, float repeat, float freq, float present, const int32_t* bias_ids, const float* bias_vals,
+                                          int n_bias, int64_t* ticket) {
+    return guard([&] {
+        auto* box = static_cast<ServerBox*>(s);
+        server::Server::CompleteRequestParams p; p.maxTokens = max_tokens; p.seed = seed; p.temperature = temp; p.topP = top_p;
+        p.repetitionPenalty = {last_n, repeat, freq, present};
+        for (int i = 0; i < n_bias; ++i) p.logitBias[bias_ids[i]] = bias_vals[i];
+        auto [id, t] = box->open();
         box->srv->completeTokens(std::vector<int32_t>(prompt, prompt + n_prompt), std::move(p),
                                  [box, t = t](server::Server::CompleteReponse r) { t->response = std::move(r); box->finish(t); });
         *ticket = id;

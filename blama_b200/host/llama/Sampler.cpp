@@ -10,16 +10,22 @@
 namespace bl::llama {
 
 Sampler::Sampler(Model& /*model*/, const Params& params) : m_params(params), m_rng(params.rngSeed) {
-    // stages that need every logit of the vocabulary or a grammar engine are outside the hot path this build covers
+    // stages that need a grammar engine or adapt to the draws are outside the hot path this build covers
     if (!params.grammar.empty()) Raise{} << "grammar-constrained sampling is not supported by this build";
-    if (!params.logitBias.empty()) Raise{} << "logit bias is not supported by this build";
     if (params.mirostat.ver != 0) {
         if (params.mirostat.ver > 2) throw std::runtime_error("Unsupported mirostat version");
         Raise{} << "mirostat sampling is not supported by this build";
     }
+    // -inf bans an id; NaN and +inf would poison the row (the reference passes them through unchecked)
+    for (const auto& [id, bias] : params.logitBias)
+        if (std::isnan(bias) || bias == INFINITY) Raise{} << "logit bias of token " << id << " must not be NaN or +inf";
     const auto& rp = params.repetitionPenalty;
-    if (!(rp.numTokens == 0 || (rp.repeat == 1.0f && rp.freq == 0.0f && rp.present == 0.0f)))
-        Raise{} << "repetition penalties are not supported by this build";
+    if (!(rp.repeat == 1.0f && rp.freq == 0.0f && rp.present == 0.0f)) {
+        // whether llama_sampler_init_penalties clamps a negative window to 0 could not be confirmed, so it is refused
+        if (rp.numTokens < 0) Raise{} << "repetition penalty window must not be negative, got " << rp.numTokens;
+        if (!(std::isfinite(rp.repeat) && rp.repeat > 0.0f) || !std::isfinite(rp.freq) || !std::isfinite(rp.present))
+            Raise{} << "repetition penalties must be finite, and the repeat penalty > 0";
+    }
     for (auto t : params.samplerSequence)
         if (t == SamplingType::XTC || t == SamplingType::Infill) throw std::runtime_error("Unsupported sampler type");
     if (params.typicalP < 1.0f) Raise{} << "typical sampling is not supported by this build";
@@ -28,10 +34,64 @@ Sampler::Sampler(Model& /*model*/, const Params& params) : m_params(params), m_r
 
 Sampler::~Sampler() = default;
 
-void Sampler::reset() { m_rng.seed(m_params.rngSeed); }
+void Sampler::reset() {
+    m_rng.seed(m_params.rngSeed);
+    m_prev.clear();
+    m_counts.clear();
+}
 
-void Sampler::accept(Token, bool) {
-    // with the supported parameter set (no penalties, no grammar) accepting a token changes no sampler state
+void Sampler::accept(Token id, bool) {
+    const int32_t window = m_params.repetitionPenalty.numTokens;
+    if (window <= 0) return;
+    m_counts[id]++;
+    if (m_prev.size() >= size_t(window)) {
+        const Token old = m_prev.front();
+        m_prev.pop_front();
+        if (--m_counts[old] == 0) m_counts.erase(old);
+    }
+    m_prev.push_back(id);
+}
+
+bool Sampler::penaltiesActive() const noexcept {
+    const auto& rp = m_params.repetitionPenalty;
+    return rp.numTokens > 0 && !(rp.repeat == 1.0f && rp.freq == 0.0f && rp.present == 0.0f);
+}
+
+Sampler::LogitEdits Sampler::logitEdits(int32_t nVocab) const {
+    LogitEdits out;
+    const bool penalties = penaltiesActive();
+    if (penalties) {
+        out.repeat = m_params.repetitionPenalty.repeat;
+        out.freq = m_params.repetitionPenalty.freq;
+        out.present = m_params.repetitionPenalty.present;
+    }
+    // both maps are ordered by id: merge them
+    auto b = m_params.logitBias.lower_bound(0);
+    auto c = penalties ? m_counts.lower_bound(0) : m_counts.end();
+    const auto bEnd = m_params.logitBias.lower_bound(nVocab);
+    const auto cEnd = penalties ? m_counts.lower_bound(nVocab) : m_counts.end();
+    while (b != bEnd || c != cEnd) {
+        const Token id = (c == cEnd || (b != bEnd && b->first < c->first)) ? b->first : c->first;
+        LogitEdit e{id, 0, 0.0f};
+        if (b != bEnd && b->first == id) { e.bias = b->second; ++b; }
+        if (c != cEnd && c->first == id) { e.count = c->second; ++c; }
+        if (e.bias != 0.0f || e.count > 0) out.edits.push_back(e);
+    }
+    return out;
+}
+
+float Sampler::editLogit(float logit, int32_t count, float bias, float repeat, float freq, float present) {
+    if (bias != 0.0f) logit += bias;
+    if (count > 0) {
+        logit = logit <= 0.0f ? logit * repeat : logit / repeat;
+        logit -= float(count) * freq + present;
+    }
+    return logit;
+}
+
+void Sampler::applyEdits(std::span<float> row) const {
+    const LogitEdits e = logitEdits(int32_t(row.size()));
+    for (const auto& d : e.edits) row[size_t(d.token)] = editLogit(row[size_t(d.token)], d.count, d.bias, e.repeat, e.freq, e.present);
 }
 
 int32_t Sampler::candidatesNeeded() const noexcept {

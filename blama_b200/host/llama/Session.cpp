@@ -93,12 +93,14 @@ TokenPrediction Session::getToken() {
     // sample from the distribution left by the last decode; the chain only ever looks at its top-k
     const int32_t need = m_sampler->candidatesNeeded();
     if (need > 0) {
-        m_currToken = m_sampler->sample({m_candidates.data(), std::min<size_t>(m_candidates.size(), size_t(need))}, true);
+        const auto cands = samplingCandidates();
+        m_currToken = m_sampler->sample(cands.first(std::min<size_t>(cands.size(), size_t(need))), true);
     } else {
         // top-k disabled or wider than the device list: the whole row is needed (reference behaviour, slow path)
         const int32_t nVocab = blk_model_n_vocab(m_instance.model().lmodel());
         std::vector<float> row(static_cast<size_t>(nVocab));
         throwIfFailed(blk_get_logits_last(m_ctx, row.data()), "get logits");
+        m_sampler->applyEdits(row);
         TokenDataVector all(static_cast<size_t>(nVocab));
         for (int32_t i = 0; i < nVocab; ++i) all[size_t(i)] = {i, row[size_t(i)]};
         m_currToken = m_sampler->sample(all, false);
@@ -162,7 +164,6 @@ std::vector<TokenPrediction> Session::fillCtx(std::span<TokenPrediction> tokens)
     std::vector<int32_t> claimed(n * 10, 0), nClaimed(n, 0);
     for (size_t i = 0; i < n; ++i) {
         ids[i] = tokens[i].token;
-        m_sampler->accept(ids[i], false);
         // distinct claimed ids in ascending order: what the reference's vocabulary walk would visit (:271-275)
         std::vector<Token> uniq;
         for (const auto& td : tokens[i].logits) uniq.push_back(td.token);
@@ -173,12 +174,15 @@ std::vector<TokenPrediction> Session::fillCtx(std::span<TokenPrediction> tokens)
         nClaimed[i] = int32_t(uniq.size());
         std::copy(uniq.begin(), uniq.end(), claimed.begin() + long(i * 10));
     }
+    // the reference pushes every response token as a prompt of its own (reset, then accept): its last one is what remains
+    m_sampler->accept(ids.back(), false);
     std::vector<float> gathered(n * 10, 0.0f);
     throwIfFailed(blk_ctx_set_verify_mode(m_ctx, m_params.sequentialVerify ? 1 : 0), "verify mode");
     // the per-position top-10 of the verifier is not needed here (only the claimed ids are compared): nullptr skips that pass
     const int st = blk_verify_prefill(m_ctx, ids.data(), int32_t(n), claimed.data(), nClaimed.data(), gathered.data(), nullptr);
     if (st != BLK_OK) Raise{} << "Failed to decode tokens";
     m_numPast += uint32_t(n);
+    m_haveRow = true;
 
     for (size_t i = 0; i < n; ++i) {
         TokenDataVector v(size_t(nClaimed[i]));
@@ -212,11 +216,12 @@ std::vector<TokenPrediction> Session::setInitialPromptAndFill(std::span<const To
     std::vector<Token> ids(np + n);
     std::vector<int32_t> claimed((np + n) * 10, 0), nClaimed(np + n, 0);
     for (size_t i = 0; i < np; ++i) { ids[i] = prompt[i]; m_sampler->accept(prompt[i], false); }
-    m_sampler->reset();                                   // pushPrompt: previous inputs must not influence the generation
+    // fillCtx pushes every response token as a prompt of its own (reset, then accept): only the last one remains
+    m_sampler->reset();
+    m_sampler->accept(tokens[n - 1].token, false);
     const int32_t nVocab = blk_model_n_vocab(m_instance.model().lmodel());
     for (size_t i = 0; i < n; ++i) {
         ids[np + i] = tokens[i].token;
-        m_sampler->accept(tokens[i].token, false);
         std::vector<Token> uniq;
         for (const auto& td : tokens[i].logits) uniq.push_back(td.token);
         std::sort(uniq.begin(), uniq.end());
@@ -230,6 +235,7 @@ std::vector<TokenPrediction> Session::setInitialPromptAndFill(std::span<const To
     if (blk_verify_prefill(m_ctx, ids.data(), int32_t(np + n), claimed.data(), nClaimed.data(), gathered.data(), nullptr) != BLK_OK)
         Raise{} << "Failed to decode tokens";
     m_numPast += uint32_t(np + n);
+    m_haveRow = true;
     m_phase = Phase::Generating;
     std::vector<TokenPrediction> result;
     result.reserve(n);
@@ -248,16 +254,20 @@ Token Session::sampleNext() {
     flushPendingState();
     const int32_t need = m_sampler->candidatesNeeded();
     if (need <= 0) Raise{} << "batched decoding needs a sampler chain that starts with top-k (the device returns the top " << Sampler::MaxDeviceCandidates << ")";
-    const Token t = m_sampler->sample({m_candidates.data(), std::min<size_t>(m_candidates.size(), size_t(need))}, true);
+    const auto cands = samplingCandidates();
+    const Token t = m_sampler->sample(cands.first(std::min<size_t>(cands.size(), size_t(need))), true);
     if (m_instance.model().vocab().isEog(t)) return Token_Invalid;
     ensureRoom(1);
+    m_sampler->accept(t, true);
     return t;
 }
 
-TokenPrediction Session::acceptDecoded(Token token, std::span<const TokenData> candidates) {
-    m_sampler->accept(token, true);
+TokenPrediction Session::acceptDecoded(Token token, std::span<const TokenData> candidates, std::span<const TokenData> edited) {
     m_numPast += 1;
     m_candidates.assign(candidates.begin(), candidates.end());
+    m_edited.assign(edited.begin(), edited.end());
+    m_useEdited = !edited.empty();
+    m_haveRow = false;
     TokenPrediction out;
     out.token = token;
     out.logits.assign(m_candidates.begin(), m_candidates.begin() + std::min<size_t>(m_candidates.size(), size_t(kReportedTop)));
@@ -268,7 +278,25 @@ void Session::refreshCandidates() {
     m_candidates.resize(size_t(Sampler::MaxDeviceCandidates));
     static_assert(sizeof(TokenData) == sizeof(blk_token_data));
     throwIfFailed(blk_topk_last(m_ctx, Sampler::MaxDeviceCandidates, reinterpret_cast<blk_token_data*>(m_candidates.data())), "top-k");
+    refreshEdited();
 }
+
+// the edited top-k of the kept row for the current sampler (nothing to do, and no launch, when it has no edits)
+void Session::refreshEdited() {
+    const Sampler::LogitEdits edits = logitEdits();
+    m_useEdited = !edits.edits.empty();
+    if (!m_useEdited) return;
+    if (!m_haveRow) Raise{} << "logit bias and repetition penalties need the last logits row, which a batched decode step does not keep";
+    const blk_logit_edits e = abiEdits(edits);
+    m_edited.resize(size_t(Sampler::MaxDeviceCandidates));
+    throwIfFailed(blk_topk_last_edited(m_ctx, Sampler::MaxDeviceCandidates, &e, reinterpret_cast<blk_token_data*>(m_edited.data())), "edited top-k");
+}
+
+std::span<const TokenData> Session::samplingCandidates() const { return m_useEdited ? m_edited : m_candidates; }
+
+Sampler::LogitEdits Session::logitEdits() const { return m_sampler->logitEdits(nVocab()); }
+
+int32_t Session::nVocab() const { return blk_model_n_vocab(m_instance.model().lmodel()); }
 
 TokenDataVector Session::getLogitsFromCtx(int32_t topK) {
     requireStarted(true);
@@ -320,6 +348,7 @@ bool Session::setState(std::span<uint8_t> state) {
     // llama.cpp keeps the positions inside its context; here the session's counters follow the restored cache
     m_numPast = uint32_t(blk_ctx_next_pos(m_ctx));
     m_numKeep = std::min(m_numPast, m_maxTokens);
+    m_haveRow = true;
     refreshCandidates();
     m_phase = Phase::Generating;
     return true;
@@ -372,9 +401,21 @@ void Session::doDecode(std::span<const Token> tokens, Source src) {
 
     if (tokens.size() == 1) {
         m_candidates.resize(size_t(Sampler::MaxDeviceCandidates));
-        const int st = blk_decode_topk(m_ctx, tokens[0], Sampler::MaxDeviceCandidates, reinterpret_cast<blk_token_data*>(m_candidates.data()));
+        auto* raw = reinterpret_cast<blk_token_data*>(m_candidates.data());
+        // the edits of the history that now ends with this token: with none, exactly the plain decode
+        const Sampler::LogitEdits edits = logitEdits();
+        m_useEdited = !edits.edits.empty();
+        int st;
+        if (!m_useEdited) {
+            st = blk_decode_topk(m_ctx, tokens[0], Sampler::MaxDeviceCandidates, raw);
+        } else {
+            const blk_logit_edits e = abiEdits(edits);
+            m_edited.resize(size_t(Sampler::MaxDeviceCandidates));
+            st = blk_decode_topk_edited(m_ctx, tokens[0], Sampler::MaxDeviceCandidates, &e, raw, reinterpret_cast<blk_token_data*>(m_edited.data()));
+        }
         if (st != BLK_OK) Raise{} << "Failed to decode tokens";
         m_numPast += 1;
+        m_haveRow = true;
         return;
     }
     const auto batchSize = size_t(blk_ctx_n_batch(m_ctx));
@@ -384,6 +425,7 @@ void Session::doDecode(std::span<const Token> tokens, Source src) {
         if (blk_decode(m_ctx, batch.data(), int32_t(batch.size())) != BLK_OK) Raise{} << "Failed to decode tokens";
         m_numPast += uint32_t(batch.size());
     }
+    m_haveRow = true;
     refreshCandidates();
 }
 
@@ -395,7 +437,11 @@ void Session::flushPendingState() {
     }
 }
 
-void Session::resetSampler(const Sampler::Params& params) { m_sampler.reset(new Sampler(m_instance.model(), params)); }
+void Session::resetSampler(const Sampler::Params& params) {
+    m_sampler.reset(new Sampler(m_instance.model(), params));
+    if (m_phase == Phase::Initial) return;      // no row yet: the first decode selects with the new sampler's edits
+    refreshEdited();
+}
 
 TokenPrediction Session::StreamGenerator::complete() {
     if (m_session.m_phase != Session::Phase::Streaming || m_status != Status::InProgress) return {Token_Invalid, {}};

@@ -7,16 +7,22 @@
 #include "Sampler.hpp"
 #include "Token.hpp"
 
+#include <blama_b200.h>
+
 #include <memory>
 #include <span>
 #include <string>
 #include <vector>
 
-struct blk_ctx;
-
 namespace bl::llama {
 
 class Instance;
+
+// a sampler's edit list as the C ABI takes it (valid while `e` lives)
+inline blk_logit_edits abiEdits(const Sampler::LogitEdits& e) {
+    static_assert(sizeof(Sampler::LogitEdit) == sizeof(blk_logit_edit));
+    return {e.repeat, e.freq, e.present, reinterpret_cast<const blk_logit_edit*>(e.edits.data()), int32_t(e.edits.size())};
+}
 
 struct TokenPrediction {
     Token token;
@@ -91,10 +97,17 @@ public:
     // for several sessions at once (blk_decode_batch).  sampleNext() draws from the current distribution (Token_Invalid at an
     // end-of-generation token; shifts the context first when it is full, like doDecode); acceptDecoded() records that `token` has
     // been decoded into this session's cache and installs the new distribution's top-k.  Returns what getToken() would have.
+    // sampleNext() also accepts the drawn token into the sampler (as the reference does right before decoding it), so that
+    // logitEdits() then describes the edits of the row the decode produces: with logit bias or penalties active the batch runs
+    // blk_decode_batch_edited and acceptDecoded receives that row's edited top-k as well (empty = the raw list is sampled).
     Token sampleNext();
-    TokenPrediction acceptDecoded(Token token, std::span<const TokenData> candidates);
+    TokenPrediction acceptDecoded(Token token, std::span<const TokenData> candidates, std::span<const TokenData> edited = {});
+    Sampler::LogitEdits logitEdits() const;
+    // what the next draw samples from: the device top-k of the current row after the sampler's edits (the raw top-k without any)
+    std::span<const TokenData> samplingCandidates() const;
     std::vector<uint8_t> getState();
-    // New sampler chain for the rest of the session (Session.cpp:403-405); the KV cache is kept.
+    // New sampler chain for the rest of the session (Session.cpp:403-405); the KV cache is kept.  With logit bias active the edited
+    // top-k of the current row is recomputed, which needs that row: after a batched step (acceptDecoded) it is gone and this throws.
     void resetSampler(const Sampler::Params& params);
 
 private:
@@ -111,6 +124,8 @@ private:
     TokenDataVector getLogitsFromCtx(TokenDataVector tokens);
     void requireStarted(bool allowStreaming) const;
     void refreshCandidates();
+    void refreshEdited();
+    int32_t nVocab() const;
 
     Instance& m_instance;
     blk_ctx* m_ctx;
@@ -123,7 +138,10 @@ private:
     unsigned m_numKeep = 0;
     uint32_t m_numPast = 0;                 // position of the next token (= cells in the cache unless Self-Extend regrouped positions)
     uint32_t m_gaIndex = 0;                 // number of grouped KV tokens (only used if gaFactor > 1)
-    TokenDataVector m_candidates;           // device top-k of the current logits, descending
+    TokenDataVector m_candidates;           // device top-k of the current logits, descending (what is reported)
+    TokenDataVector m_edited;               // device top-k of the current logits after logit bias + penalties (what is sampled)
+    bool m_useEdited = false;               // m_edited is current: the sampler had edits for the current row
+    bool m_haveRow = false;                 // the context keeps the current logits row (not after a batched step)
 };
 
 } // namespace bl::llama

@@ -164,7 +164,7 @@ struct Server::Impl {
                     if (!job.isComplete) {                    // e.g. a verify: one prefill on a free slot, between two steps
                         job.run(w, si);
                     } else {
-                        auto& session = w.slot(si).startSession({.seed = job.params.seed, .temperature = job.params.temperature, .topP = job.params.topP});
+                        auto& session = startComplete(w.slot(si), job.params);
                         if (job.tokenize) job.prompt = w.model->vocab().tokenize(job.params.prompt, true, true);
                         session.setInitialPrompt(job.prompt);
                         busy[si] = 1;
@@ -220,8 +220,18 @@ struct Server::Impl {
                 tSample += now() - ts0;
                 if (!ctxs.empty()) {
                     const double tb0 = now();
-                    std::vector<blk_token_data> top(ctxs.size() * size_t(Sampler::MaxDeviceCandidates));
-                    if (blk_decode_batch(ws, ctxs.data(), toks.data(), int32_t(ctxs.size()), Sampler::MaxDeviceCandidates, top.data()) != BLK_OK) {
+                    constexpr int32_t K = Sampler::MaxDeviceCandidates;
+                    // rows whose sampler edits the logits (bias / penalties, after sampleNext accepted the token) need the edited
+                    // top-k too: then one edit pass covers every row; without any, exactly the plain step
+                    std::vector<Sampler::LogitEdits> edits(ctxs.size());
+                    bool anyEdits = false;
+                    for (size_t j = 0; j < who.size(); ++j) { edits[j] = active[who[j]].session->logitEdits(); anyEdits = anyEdits || !edits[j].edits.empty(); }
+                    std::vector<blk_token_data> top(ctxs.size() * size_t(K)), edited(anyEdits ? top.size() : 0);
+                    std::vector<blk_logit_edits> rows;
+                    for (const auto& e : edits) rows.push_back(abiEdits(e));
+                    const blk_status st = anyEdits ? blk_decode_batch_edited(ws, ctxs.data(), toks.data(), int32_t(ctxs.size()), K, rows.data(), top.data(), edited.data())
+                                                   : blk_decode_batch(ws, ctxs.data(), toks.data(), int32_t(ctxs.size()), K, top.data());
+                    if (st != BLK_OK) {
                         const std::string why = std::string("Failed to decode tokens: ") + blk_last_error();
                         (void)blk_timer_stop(ws, &ms);
                         while (!active.empty()) retire(active.size() - 1, true, why);
@@ -232,8 +242,10 @@ struct Server::Impl {
                     using LlamaTokenData = bl::llama::TokenData;      // (Server::TokenData is the marshalled form)
                     static_assert(sizeof(LlamaTokenData) == sizeof(blk_token_data));
                     for (size_t j = 0; j < who.size(); ++j) {
-                        const LlamaTokenData* cand = reinterpret_cast<const LlamaTokenData*>(top.data() + j * size_t(Sampler::MaxDeviceCandidates));
-                        active[who[j]].preds.push_back(active[who[j]].session->acceptDecoded(toks[j], std::span<const LlamaTokenData>(cand, size_t(Sampler::MaxDeviceCandidates))));
+                        const LlamaTokenData* cand = reinterpret_cast<const LlamaTokenData*>(top.data() + j * size_t(K));
+                        std::span<const LlamaTokenData> ed;
+                        if (anyEdits) ed = {reinterpret_cast<const LlamaTokenData*>(edited.data() + j * size_t(K)), size_t(K)};
+                        active[who[j]].preds.push_back(active[who[j]].session->acceptDecoded(toks[j], std::span<const LlamaTokenData>(cand, size_t(K)), ed));
                     }
                     tAccept += now() - tc0;
                 }
@@ -247,6 +259,19 @@ struct Server::Impl {
         idleCv.wait(lk, [&] { return queue.empty() && running == 0; });
     }
 
+    // a /complete session: the reference's sampler, replaced by one with the request's bias / penalties when it asks for them
+    static Session& startComplete(Instance& inst, const CompleteRequestParams& p) {
+        auto& session = inst.startSession({.seed = p.seed, .temperature = p.temperature, .topP = p.topP});
+        const auto& rp = p.repetitionPenalty;
+        if (!p.logitBias.empty() || !(rp.repeat == 1.0f && rp.freq == 0.0f && rp.present == 0.0f)) {
+            Sampler::Params sp;
+            sp.rngSeed = p.seed; sp.topP = p.topP; sp.temp = p.temperature;
+            sp.repetitionPenalty = rp;
+            sp.logitBias.insert(p.logitBias.begin(), p.logitBias.end());
+            session.resetSampler(sp);
+        }
+        return session;
+    }
     static CompleteReponse marshal(const Model& model, const std::vector<TokenPrediction>& preds) {
         CompleteReponse response;
         response.reserve(preds.size());
@@ -276,7 +301,7 @@ struct Server::Impl {
         Job job;
         job.isComplete = true; job.prompt = prompt; job.tokenize = tokenize; job.params = params; job.completeCb = cbp;
         job.run = [prompt = std::move(prompt), tokenize, params = std::move(params), cbp](Worker& w, size_t) mutable {
-            auto& session = w.instance->startSession({.seed = params.seed, .temperature = params.temperature, .topP = params.topP});
+            auto& session = startComplete(*w.instance, params);
             if (tokenize) prompt = w.model->vocab().tokenize(params.prompt, true, true);
             session.setInitialPrompt(prompt);
             auto preds = session.complete({.prompt = {}, .suffix = {}, .maxTokens = int32_t(params.maxTokens)});

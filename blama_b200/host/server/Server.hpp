@@ -6,9 +6,11 @@
 // involved (SURVEY.md section 8e).
 #pragma once
 #include "../llama/Instance.hpp"
+#include "../llama/Sampler.hpp"
 
 #include <cstdint>
 #include <functional>
+#include <map>
 #include <memory>
 #include <string>
 #include <vector>
@@ -39,6 +41,10 @@ public:
         std::string suffix;           // parsed by the HTTP layer but never forwarded (reference Server.cpp:53-56)
         float temperature = 0.8f;
         float topP = 0.95f;
+        // extension, off by default (the HTTP body does not carry them): the logit-bias and repetition-penalty stages of the
+        // reference's sampler chain (Sampler::Params::logitBias / repetitionPenalty), applied through Session::resetSampler
+        Sampler::Params::RepetitionPenalty repetitionPenalty;
+        std::map<int32_t, float> logitBias;
     };
     struct TokenData {
         std::string tokenStr;

@@ -42,6 +42,15 @@ HOST_SYMBOLS = {
     "blh_lc_similarity": (_f32, [_vp, _i32, _vp, _i32]),
     "blh_lc_score": (_f32, [_vp, _i32]),
     "blh_sampler_draw": (C.c_int, [_u32, _f32, _f32, _i32, _f32, _i32, _vp, _i32, _i32, _i32, _vp]),
+    "blh_sampler_draw_penalized": (C.c_int, [_u32, _f32, _f32, _i32, _f32, _i32, _i32, _f32, _f32, _f32, _vp, _vp, C.c_int,
+                                             _vp, _i32, _vp, _i32, _i32, _vp]),
+    "blh_sampler_logit_edits": (C.c_int, [_i32, _f32, _f32, _f32, _vp, _vp, C.c_int, _vp, _i32, _i32, _i32, _vp, C.c_int, _vp, _vp]),
+    "blh_sampler_check": (C.c_int, [_i32, C.c_char_p]),
+    "blh_session_reset_sampler": (C.c_int, [_vp, _u32, _f32, _f32, _i32, _f32, _f32, _f32, _vp, _vp, C.c_int]),
+    "blh_session_logit_edits": (C.c_int, [_vp, _vp, C.c_int, _vp, _vp]),
+    "blh_session_candidates": (C.c_int, [_vp, _vp, C.c_int, _vp]),
+    "blh_server_submit_complete_ex": (C.c_int, [_vp, _vp, C.c_int, _u32, _u32, _f32, _f32, _i32, _f32, _f32, _f32, _vp, _vp, C.c_int,
+                                                C.POINTER(C.c_int64)]),
     "blh_server_create": (C.c_int, [_vp, C.c_int, _u32, _u32, C.POINTER(_vp)]),
     "blh_server_create_ex": (C.c_int, [_vp, C.c_int, _u32, _u32, _u32, C.POINTER(_vp)]),
     "blh_server_free": (None, [_vp]),
@@ -108,6 +117,27 @@ def as_td(pairs) -> np.ndarray:
     return out
 
 
+EDIT_DTYPE = capi.EDIT_DTYPE
+
+
+def _bias_arrays(logit_bias):
+    """{token: bias} -> (ids int32, values float32)"""
+    items = sorted((logit_bias or {}).items())
+    return np.array([k for k, _ in items], dtype=np.int32), np.array([v for _, v in items], dtype=np.float32)
+
+
+def _stages_active(penalty_last_n, repeat_penalty, freq_penalty, present_penalty, logit_bias) -> bool:
+    return bool(logit_bias) or (repeat_penalty, freq_penalty, present_penalty) != (1.0, 0.0, 0.0)
+
+
+def _edits_out(call, cap: int = 1 << 16):
+    """call(out, cap, byref(n), out3) -> rc: (EDIT_DTYPE array, (repeat, freq, present))"""
+    out = np.zeros(cap, dtype=EDIT_DTYPE); n = _i32(0); p3 = np.zeros(3, dtype=np.float32)
+    _check(call(_p(out), cap, C.byref(n), _p(p3)))
+    assert n.value <= cap
+    return out[: n.value].copy(), tuple(float(x) for x in p3)
+
+
 class Model:
     def __init__(self, path: str, device: int = 0, gpu: bool = True, prefix_bos: bool = False, vocab_only: bool = False):
         h = _vp()
@@ -171,9 +201,31 @@ class Instance:
         return c
 
     def start_session(self, seed: int = 0, temperature: float = 0.8, top_p: float = 0.95, sequential_verify: bool = False,
-                      infinite_context: bool = True):
+                      infinite_context: bool = True, penalty_last_n: int = 64, repeat_penalty: float = 1.0, freq_penalty: float = 0.0,
+                      present_penalty: float = 0.0, logit_bias: Optional[dict] = None):
+        """logit_bias {token: bias} and the repetition penalties are the first two stages of the reference's sampler chain (off by
+        default); when given, the session's sampler is replaced by one that has them (Session::resetSampler) before any decode"""
         _check(lib().blh_session_start_ex(self.h, seed, temperature, top_p, int(sequential_verify), int(infinite_context)))
+        if _stages_active(penalty_last_n, repeat_penalty, freq_penalty, present_penalty, logit_bias):
+            self.reset_sampler(seed, temperature, top_p, penalty_last_n, repeat_penalty, freq_penalty, present_penalty, logit_bias)
         return self
+
+    def reset_sampler(self, seed: int = 0, temperature: float = 0.8, top_p: float = 0.95, penalty_last_n: int = 64, repeat_penalty: float = 1.0,
+                      freq_penalty: float = 0.0, present_penalty: float = 0.0, logit_bias: Optional[dict] = None):
+        """Session::resetSampler: a new sampler chain (empty penalty window) for the rest of the session"""
+        ids, vals = _bias_arrays(logit_bias)
+        _check(lib().blh_session_reset_sampler(self.h, seed, temperature, top_p, penalty_last_n, repeat_penalty, freq_penalty, present_penalty,
+                                               _p(ids), _p(vals), len(ids)))
+
+    def sampling_candidates(self) -> np.ndarray:
+        """the list the next draw samples from (the edited top-64 with logit bias / penalties active, else the raw top-64)"""
+        out = np.zeros(64, dtype=TD_DTYPE); n = _i32(0)
+        _check(lib().blh_session_candidates(self.h, _p(out), 64, C.byref(n)))
+        return out[: min(n.value, 64)].copy()
+
+    def logit_edits(self):
+        """the session sampler's edit list now: (EDIT_DTYPE array, (repeat, freq, present))"""
+        return _edits_out(lambda out, cap, n, p3: lib().blh_session_logit_edits(self.h, out, cap, n, p3))
 
     def start_session_self_extend(self, ga_factor: int, ga_width: int, seed: int = 0, temperature: float = 0.8, top_p: float = 0.95):
         """Session with group attention (Self-Extend, reference Session.cpp:348-368)"""
@@ -266,6 +318,33 @@ def sampler_draw(cand, n_draws: int, seed: int = 0, temp: float = 0.8, top_p: fl
     return out
 
 
+def sampler_draw_penalized(logits: np.ndarray, n_draws: int, history: Sequence[int] = (), seed: int = 0, temp: float = 0.8, top_p: float = 0.95,
+                           top_k: int = 40, min_p: float = 0.05, min_keep: int = 0, penalty_last_n: int = 64, repeat_penalty: float = 1.0,
+                           freq_penalty: float = 0.0, present_penalty: float = 0.0, logit_bias: Optional[dict] = None) -> np.ndarray:
+    """the host Sampler's full-row path: accept `history`, then per draw edit a copy of `logits` with bias + penalties, draw, accept"""
+    lg = np.ascontiguousarray(logits, dtype=np.float32)
+    h = np.ascontiguousarray(history, dtype=np.int32)
+    ids, vals = _bias_arrays(logit_bias)
+    out = np.zeros(max(1, n_draws), dtype=np.int32)
+    _check(lib().blh_sampler_draw_penalized(seed, temp, top_p, top_k, min_p, min_keep, penalty_last_n, repeat_penalty, freq_penalty, present_penalty,
+                                            _p(ids), _p(vals), len(ids), _p(h), len(h), _p(lg), len(lg), n_draws, _p(out)))
+    return out[:n_draws]
+
+
+def sampler_check(mirostat: int = 0, grammar: str = ""):
+    """raises HostError when the Sampler refuses these parameters"""
+    _check(lib().blh_sampler_check(mirostat, grammar.encode()))
+
+
+def sampler_logit_edits(n_vocab: int, history: Sequence[int] = (), penalty_last_n: int = 64, repeat_penalty: float = 1.0, freq_penalty: float = 0.0,
+                        present_penalty: float = 0.0, logit_bias: Optional[dict] = None, reset_after: bool = False):
+    """Sampler::logitEdits after accepting `history` (then reset() when reset_after): (EDIT_DTYPE array, (repeat, freq, present))"""
+    h = np.ascontiguousarray(history, dtype=np.int32)
+    ids, vals = _bias_arrays(logit_bias)
+    return _edits_out(lambda out, cap, n, p3: lib().blh_sampler_logit_edits(penalty_last_n, repeat_penalty, freq_penalty, present_penalty, _p(ids),
+                                                                            _p(vals), len(ids), _p(h), len(h), int(reset_after), n_vocab, out, cap, n, p3))
+
+
 # ---- wire format (host only) ----------------------------------------------------------------------------------------------
 def _text_out(call, cap: int = 1 << 16) -> str:
     """call(buf, cap, byref(len)) -> rc; grows the buffer once when the text is longer than cap"""
@@ -331,10 +410,17 @@ class Server:
     def workers(self) -> int:
         return lib().blh_server_workers(self.h)
 
-    def submit_complete(self, prompt: Sequence[int], max_tokens: int, seed: int = 0, temp: float = 0.8, top_p: float = 0.95) -> int:
+    def submit_complete(self, prompt: Sequence[int], max_tokens: int, seed: int = 0, temp: float = 0.8, top_p: float = 0.95,
+                        penalty_last_n: int = 64, repeat_penalty: float = 1.0, freq_penalty: float = 0.0, present_penalty: float = 0.0,
+                        logit_bias: Optional[dict] = None) -> int:
         p = np.ascontiguousarray(prompt, dtype=np.int32)
         t = C.c_int64(0)
-        _check(lib().blh_server_submit_complete(self.h, _p(p), len(p), max_tokens, seed, temp, top_p, C.byref(t)))
+        if not _stages_active(penalty_last_n, repeat_penalty, freq_penalty, present_penalty, logit_bias):
+            _check(lib().blh_server_submit_complete(self.h, _p(p), len(p), max_tokens, seed, temp, top_p, C.byref(t)))
+        else:
+            ids, vals = _bias_arrays(logit_bias)
+            _check(lib().blh_server_submit_complete_ex(self.h, _p(p), len(p), max_tokens, seed, temp, top_p, penalty_last_n, repeat_penalty,
+                                                       freq_penalty, present_penalty, _p(ids), _p(vals), len(ids), C.byref(t)))
         return t.value
 
     def submit_verify(self, prompt: Sequence[int], tokens: Sequence[int], claimed: np.ndarray, n_claimed=None, seed: int = 0,

@@ -150,6 +150,30 @@ BLK_API blk_status blk_decode_topk(blk_ctx*, int32_t token, int32_t k, blk_token
  * need a blk_decode first). */
 BLK_API blk_status blk_decode_batch(blk_ctx* ws, blk_ctx* const* ctxs, const int32_t* tokens, int32_t n, int32_t k, blk_token_data* out);
 
+/* ---- logit bias and repetition penalties (llama.cpp b5187 llama_sampler_logit_bias_apply + llama_sampler_penalties_apply) ----
+ * The two stages at the head of the reference's sampler chain change logits before its top-k, so the top-k of the raw row no
+ * longer decides the draw.  These entry points apply them on the device to a COPY of the last logits row and select the top-k
+ * of that copy; the raw row, its top-k (the reported top-10), blk_gather_last, blk_get_logits_last and the state blob stay raw.
+ * Per edited id, in this order (float arithmetic, no contraction):
+ *     if (bias != 0)  logit += bias;
+ *     if (count > 0)  { logit = logit <= 0 ? logit * repeat : logit / repeat;  logit -= (float)count * freq + present; }
+ * Edit lists come from outside the library and are checked before anything is launched (BLK_ERR_ARG): ids in [0, n_vocab) and
+ * strictly ascending, counts >= 0, biases not NaN or +inf (-inf bans an id), repeat finite and > 0, freq / present finite.
+ * Lists of any length are staged (a bias map may ban thousands of ids). */
+typedef struct { int32_t token; int32_t count; float bias; } blk_logit_edit;      /* count 0 = bias only */
+typedef struct { float repeat, freq, present; const blk_logit_edit* edits; int32_t n_edits; } blk_logit_edits;
+/* blk_decode_topk plus the edit pass: raw = top-k of the new raw row (what blk_decode_topk returns), edited = top-k of the edited
+ * row.  One synchronise. */
+BLK_API blk_status blk_decode_topk_edited(blk_ctx*, int32_t token, int32_t k, const blk_logit_edits* edits, blk_token_data* raw,
+                                          blk_token_data* edited);
+/* top-k of the edited copy of the kept last row (after a prompt prefill, a verify fill, blk_state_set, or for a sampler replaced
+ * after a decode).  Needs a last row, as blk_topk_last does. */
+BLK_API blk_status blk_topk_last_edited(blk_ctx*, int32_t k, const blk_logit_edits* edits, blk_token_data* edited);
+/* blk_decode_batch plus the edit pass of every row (per_row[n]): raw as blk_decode_batch's out, edited[i * k ..] = top-k of row i
+ * after its own edits.  One edit launch and one selection launch for all rows. */
+BLK_API blk_status blk_decode_batch_edited(blk_ctx* ws, blk_ctx* const* ctxs, const int32_t* tokens, int32_t n, int32_t k,
+                                           const blk_logit_edits* per_row, blk_token_data* raw, blk_token_data* edited);
+
 /* Device-resident greedy decode loop (measurement aid for bench.py's `value`): n_steps decode steps back to back with the
  * arg-max token fed back ON THE DEVICE, no host round trip inside the loop.  Asynchronous unless last_token != NULL. */
 BLK_API blk_status blk_decode_loop(blk_ctx*, int32_t first_token, int32_t n_steps, int32_t* last_token);
@@ -222,6 +246,10 @@ BLK_API blk_status blk_test_decode_attn(int32_t device, const float* q, const fl
                                         int32_t n_head_kv, int32_t d_head, int32_t form, int64_t seed, float* out, int32_t* used_form);
 BLK_API blk_status blk_test_decode_attn_batch(int32_t device, int32_t n, const float* q, const float* k, const float* v, const int32_t* n_kv,
                                               int32_t n_head, int32_t n_head_kv, int32_t d_head, int64_t seed, float* out);
+/* The edit pass of blk_decode_batch_edited on host rows: logits [n_rows][n_vocab] and per_row[n_rows] in, out [n_rows][k] = the
+ * edited rows' top-k (descending, ties to the lower id), through the same two launches. */
+BLK_API blk_status blk_test_logit_edits(int32_t device, const float* logits, int32_t n_rows, int32_t n_vocab, const blk_logit_edits* per_row,
+                                        int32_t k, blk_token_data* out);
 /* dequantise through the device re-tile + dequant kernels */
 BLK_API blk_status blk_test_dequant(int32_t device, int32_t type, const void* w_blocks, int64_t rows, int64_t k, float* out);
 
