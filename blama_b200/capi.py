@@ -86,7 +86,7 @@ SYMBOLS = {
     "blk_profile_verify": (_i32, [_vp, _vp, _i32, C.c_char_p, _i32]),
     "blk_bench_kernel": (_i32, [_vp, _i32, _i32, _f32p, C.POINTER(C.c_int64)]),
     "blk_test_gemv": (_i32, [_i32, _i32, _vp, _i64, _i64, _vp, _vp]),
-    "blk_test_gemm": (_i32, [_i32, _i32, _vp, _i64, _i64, _vp, _i64, _vp]),
+    "blk_test_gemm": (_i32, [_i32, _i32, _vp, _i32, _i64, _vp, _i64, _i32, _i32, _vp, C.c_float, _vp, _vp, _vp]),
     "blk_bench_gemm": (_i32, [_i32, _i32, _vp, _i64, _i64, _i64, _i32, _f32p]),
     "blk_test_dequant": (_i32, [_i32, _i32, _vp, _i64, _i64, _vp]),
     "blk_test_rmsnorm": (_i32, [_i32, _vp, _vp, _i32, _i32, C.c_float, _vp]),
@@ -95,6 +95,8 @@ SYMBOLS = {
     "blk_test_decode_attn": (_i32, [_i32, _vp, _vp, _vp, _i32, _i32, _i32, _i32, _i32, _i32, _i64, _vp, C.POINTER(_i32)]),
     "blk_test_decode_attn_batch": (_i32, [_i32, _i32, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _i64, _vp]),
     "blk_test_logit_edits": (_i32, [_i32, _vp, _i32, _i32, _vp, _i32, _vp]),
+    "blk_test_row_topk": (_i32, [_i32, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "blk_test_claimed_logits": (_i32, [_i32, _i32, _vp, _i64, _i64, _vp, _i32, _vp, _vp, _vp]),
 }
 
 _lib: Optional[C.CDLL] = None
@@ -443,13 +445,82 @@ def test_gemv(gtype: int, blocks: np.ndarray, rows: int, k: int, x: np.ndarray, 
     return y
 
 
-def test_gemm(gtype: int, blocks: np.ndarray, rows: int, k: int, x: np.ndarray, device: int = 0) -> np.ndarray:
-    b = np.ascontiguousarray(blocks, dtype=np.uint8)
+class TestMatrix(C.Structure):
+    """blk_test_matrix: one weight matrix of blk_test_gemm"""
+    _fields_ = [("type", C.c_int32), ("blocks", C.c_void_p), ("rows", C.c_int64), ("bias", C.c_void_p)]
+    __test__ = False
+
+
+class GemmPlan(C.Structure):
+    """blk_test_gemm_plan: what a blk_test_gemm call ran"""
+    _fields_ = [("n_sm", C.c_int32), ("launches", C.c_int32), ("k_splits", C.c_int32), ("n_whole", C.c_int32), ("deferred", C.c_int32),
+                ("panel", C.c_int32)]
+
+    def as_dict(self) -> dict:
+        return {f: int(getattr(self, f)) for f, _ in self._fields_}
+
+
+GEMM_STORE, GEMM_ACCUM, GEMM_SWIGLU = 0, 1, 2
+
+
+def test_gemm_layer(op: int, mats, k: int, x: np.ndarray, form: int = 0, split: int = 0, c: Optional[np.ndarray] = None,
+                    norm_w: Optional[np.ndarray] = None, eps: float = 1e-5, device: int = 0):
+    """The prefill GEMM as a multi-token pass calls it (blk_test_gemm).  mats: [(ggml type, blocks, rows, bias or None), ...].
+    op GEMM_STORE: C = X W_i^T (+bias_i) side by side; GEMM_ACCUM: C += X W^T (c = the residual) then, with norm_w, the RMSNorm;
+    GEMM_SWIGLU: H = silu(X Wg^T) * (X Wu^T).  form 0 fused / 1 panel; split 0 none / 1 workspace / 2 workspace + deferred reduce.
+    Returns (C or None, H / xn or None, plan dict).  c: the initial C (op GEMM_STORE: NaN when omitted, so a column left unwritten shows)."""
     xx = np.ascontiguousarray(x, dtype=np.float32)
-    n_tok = xx.shape[0]
-    y = np.zeros((n_tok, rows), dtype=np.float32)
-    _check(lib().blk_test_gemm(device, gtype, _p(b), rows, k, _p(xx), n_tok, _p(y)))
+    T = xx.shape[0]
+    keep = []
+    arr = (TestMatrix * len(mats))()
+    for i, (gtype, blocks, rows, bias) in enumerate(mats):
+        b = np.ascontiguousarray(blocks, dtype=np.uint8)
+        bb = None if bias is None else np.ascontiguousarray(bias, dtype=np.float32)
+        keep += [b, bb]
+        arr[i] = TestMatrix(gtype, b.ctypes.data, rows, bb.ctypes.data if bb is not None else None)
+    n_out = mats[0][2] if op == GEMM_SWIGLU else sum(m[2] for m in mats)
+    cc = None
+    if op != GEMM_SWIGLU:
+        cc = np.full((T, n_out), np.nan, dtype=np.float32) if c is None else np.array(c, dtype=np.float32, order="C", copy=True)
+        assert cc.shape == (T, n_out)
+    w = None if norm_w is None else np.ascontiguousarray(norm_w, dtype=np.float32)
+    h = np.zeros((T, n_out), dtype=np.float32) if (op == GEMM_SWIGLU or w is not None) else None
+    plan = GemmPlan()
+    _check(lib().blk_test_gemm(device, op, C.cast(arr, C.c_void_p), len(mats), k, _p(xx), T, form, split, _p(w) if w is not None else None, eps,
+                               _p(cc) if cc is not None else None, _p(h) if h is not None else None, C.byref(plan)))
+    return cc, h, plan.as_dict()
+
+
+def test_gemm(gtype: int, blocks: np.ndarray, rows: int, k: int, x: np.ndarray, device: int = 0, form: int = 0, split: int = 0) -> np.ndarray:
+    """Y[t][r] = W[r,:] . X[t,:] through the prefill GEMM: one matrix, store (test_gemm_layer with GEMM_STORE); returns Y [n_tok][rows]"""
+    y, _, _ = test_gemm_layer(GEMM_STORE, [(gtype, blocks, rows, None)], k, x, form=form, split=split, device=device)
     return y
+
+
+def test_row_topk(logits: np.ndarray, claimed: np.ndarray, n_claimed: np.ndarray, rows_per_launch: int = 256, top: bool = True, device: int = 0):
+    """row_topk_gather_kernel (blk_test_row_topk): (gathered [n][10], top ids [n][10], top logits [n][10]) (the last two None without top)"""
+    lg = np.ascontiguousarray(logits, dtype=np.float32)
+    n, V = lg.shape
+    cl = np.ascontiguousarray(claimed, dtype=np.int32).reshape(n, 10)
+    nc = np.ascontiguousarray(n_claimed, dtype=np.int32).reshape(n)
+    g = np.zeros((n, 10), dtype=np.float32)
+    ti = np.zeros((n, 10), dtype=np.int32) if top else None
+    tl = np.zeros((n, 10), dtype=np.float32) if top else None
+    _check(lib().blk_test_row_topk(device, _p(lg), n, V, rows_per_launch, _p(cl), _p(nc), _p(g), _p(ti) if top else None, _p(tl) if top else None))
+    return g, ti, tl
+
+
+def test_claimed_logits(gtype: int, blocks: np.ndarray, rows: int, k: int, xn: np.ndarray, claimed: np.ndarray, n_claimed: np.ndarray,
+                        device: int = 0) -> np.ndarray:
+    """claimed_logits_kernel (blk_test_claimed_logits): gathered [n][10]"""
+    b = np.ascontiguousarray(blocks, dtype=np.uint8)
+    xx = np.ascontiguousarray(xn, dtype=np.float32)
+    n = xx.shape[0]
+    cl = np.ascontiguousarray(claimed, dtype=np.int32).reshape(n, 10)
+    nc = np.ascontiguousarray(n_claimed, dtype=np.int32).reshape(n)
+    g = np.zeros((n, 10), dtype=np.float32)
+    _check(lib().blk_test_claimed_logits(device, gtype, _p(b), rows, k, _p(xx), n, _p(cl), _p(nc), _p(g)))
+    return g
 
 
 def test_dequant(gtype: int, blocks: np.ndarray, rows: int, k: int, device: int = 0) -> np.ndarray:
@@ -465,3 +536,6 @@ def bench_gemm(gtype: int, blocks: np.ndarray, rows: int, k: int, n_tok: int, it
     ms = C.c_float(0)
     _check(lib().blk_bench_gemm(device, gtype, _p(b), rows, k, n_tok, iters, C.byref(ms)))
     return float(ms.value)
+
+
+test_gemm.__test__ = test_gemm_layer.__test__ = test_row_topk.__test__ = test_claimed_logits.__test__ = False      # (not pytest tests)

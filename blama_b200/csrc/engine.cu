@@ -16,6 +16,7 @@
 #include <cmath>
 #include <cstdio>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <random>
 #include <tuple>
@@ -2162,29 +2163,6 @@ extern "C" blk_status blk_test_gemv(int32_t device, int32_t type, const void* bl
     });
 }
 
-extern "C" blk_status blk_test_gemm(int32_t device, int32_t type, const void* blocks, int64_t rows, int64_t k, const float* x, int64_t n_tok, float* y) {
-    return guarded([&] {
-        if (n_tok <= 0) throw BlkError(BLK_ERR_ARG, "n_tok must be positive");
-        TestMat tm; test_upload(tm, device, type, blocks, rows, k);
-        blk_ctx c; c.m = &tm.holder;
-        BLK_CUDA(cudaStreamCreateWithFlags(&c.stream, cudaStreamNonBlocking));
-        float* d_x = dalloc<float>(&c, (size_t)n_tok * k);
-        __nv_bfloat16* d_xb = dalloc<__nv_bfloat16>(&c, (size_t)n_tok * k);
-        float* d_y = dalloc<float>(&c, (size_t)n_tok * rows);
-        BLK_CUDA(cudaMemcpyAsync(d_x, x, (size_t)n_tok * k * 4, cudaMemcpyHostToDevice, c.stream));
-        BLK_CUDA(convert_f32_to_bf16(d_x, d_xb, (size_t)n_tok * k, c.stream));
-        __nv_bfloat16* panel = nullptr;        // BLK_TEST_PANEL=1: the two-pass form (dequantise to a bf16 panel, TMA-fed GEMM)
-        const GemmPart part{&tm.W, nullptr, 0};
-        { const char* tp = getenv("BLK_TEST_PANEL"); if (tp && tp[0] == '1' && type != GT_F32 && type != GT_F16) panel = dalloc<__nv_bfloat16>(&c, prefill_panel_elems(&part, 1, false)); }
-        cudaError_t err = cudaSuccess;
-        if (panel && !prefill_panel_fill(&part, 1, false, panel, c.stream, &err)) panel = nullptr;
-        BLK_CUDA(err);
-        BLK_CUDA(prefill_gemm(tm.W, d_xb, (int)n_tok, d_y, rows, nullptr, 0, c.stream, panel));
-        BLK_CUDA(cudaMemcpyAsync(y, d_y, (size_t)n_tok * rows * 4, cudaMemcpyDeviceToHost, c.stream));
-        BLK_CUDA(cudaStreamSynchronize(c.stream));
-    });
-}
-
 extern "C" blk_status blk_bench_gemm(int32_t device, int32_t type, const void* blocks, int64_t rows, int64_t k, int64_t n_tok, int32_t iters, float* avg_ms) {
     return guarded([&] {
         if (n_tok <= 0 || iters <= 0 || !avg_ms) throw BlkError(BLK_ERR_ARG, "blk_bench_gemm: bad arguments");
@@ -2270,6 +2248,149 @@ extern "C" blk_status blk_test_rmsnorm(int32_t device, const float* x, const flo
         bf16_to_f32_kernel<<<grid_of((size_t)T * K), 256>>>(dy, dout, (size_t)T * K);
         BLK_CUDA(cudaGetLastError());
         BLK_CUDA(cudaMemcpy(out, dout, (size_t)T * K * 4, cudaMemcpyDeviceToHost));
+    });
+}
+
+// The prefill GEMM as run_layers calls it, on host buffers: op 0 = QKV / lm_head store (prefill_gemm, or prefill_gemm_multi for 2 - 3
+// matrices side by side), op 1 = Wo / down accumulate onto c_inout (then the RMSNorm when norm_w is given), op 2 = gate + up SwiGLU.
+// form 1 fills the bf16 panel first (prefill_panel_fill); split 1 / 2 hands over the split-K workspace, 2 with the deferred reduce the
+// RMSNorm consumes.  Everything from the GEMM on runs inside ChainPdl(n_tok), as in a pass.
+extern "C" blk_status blk_test_gemm(int32_t device, int32_t op, const blk_test_matrix* mats, int32_t n_mats, int64_t k, const float* x, int64_t n_tok,
+                                    int32_t form, int32_t split, const float* norm_w, float eps, float* c_inout, float* h_or_xn, blk_test_gemm_plan* plan) {
+    return guarded([&] {
+        const bool ok = mats && x && n_tok > 0 && n_tok <= (1 << 20) && k > 0 && (form == 0 || form == 1) && split >= 0 && split <= 2 &&
+                        ((op == 0 && n_mats >= 1 && n_mats <= 3) || (op == 1 && n_mats == 1) || (op == 2 && n_mats == 2)) &&
+                        (op == 2 ? h_or_xn != nullptr : c_inout != nullptr) && (split != 2 || (op == 1 && norm_w)) &&
+                        (!norm_w || (op == 1 && h_or_xn && k > 0 && mats[0].rows % 8 == 0 && mats[0].rows <= 8192));
+        if (!ok) throw BlkError(BLK_ERR_ARG, "blk_test_gemm: bad arguments");
+        std::vector<std::unique_ptr<TestMat>> tm;
+        for (int i = 0; i < n_mats; i++) {
+            if (mats[i].rows <= 0 || !mats[i].blocks) throw BlkError(BLK_ERR_ARG, "blk_test_gemm: bad matrix");
+            tm.push_back(std::make_unique<TestMat>());
+            test_upload(*tm.back(), device, mats[i].type, mats[i].blocks, mats[i].rows, k);
+        }
+        int sms = 0;
+        BLK_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+        Scratch sc;
+        cudaStream_t st = nullptr;
+        BLK_CUDA(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
+        struct StreamGuard { cudaStream_t s; ~StreamGuard() { cudaStreamDestroy(s); } } sg{st};
+        const int T = (int)n_tok;
+        float* dx = sc.get<float>((size_t)T * k);
+        __nv_bfloat16* dxb = sc.get<__nv_bfloat16>((size_t)T * k);
+        BLK_CUDA(cudaMemcpyAsync(dx, x, (size_t)T * k * 4, cudaMemcpyHostToDevice, st));
+        BLK_CUDA(convert_f32_to_bf16(dx, dxb, (size_t)T * k, st));
+        GemmPart parts[3];
+        long long ldc = 0;
+        for (int i = 0; i < n_mats; i++) {
+            float* b = nullptr;
+            if (mats[i].bias) {
+                b = sc.get<float>((size_t)mats[i].rows);
+                BLK_CUDA(cudaMemcpyAsync(b, mats[i].bias, (size_t)mats[i].rows * 4, cudaMemcpyHostToDevice, st));
+            }
+            parts[i] = {&tm[i]->W, b, (int)ldc};      // column offsets as in QKV: the matrices side by side
+            ldc += mats[i].rows;
+        }
+        const long long n_out = op == 2 ? mats[0].rows : ldc;
+        float* dc = nullptr; __nv_bfloat16* dh = nullptr;
+        if (op == 2) {
+            dh = sc.get<__nv_bfloat16>((size_t)T * n_out);
+            BLK_CUDA(cudaMemsetAsync(dh, 0xff, (size_t)T * n_out * 2, st));      // NaN: a column the GEMM never writes shows
+        } else {
+            dc = sc.get<float>((size_t)T * n_out);
+            BLK_CUDA(cudaMemcpyAsync(dc, c_inout, (size_t)T * n_out * 4, cudaMemcpyHostToDevice, st));
+        }
+        float* dw = nullptr; __nv_bfloat16* dxn = nullptr;
+        if (norm_w) {
+            dw = sc.get<float>((size_t)n_out); dxn = sc.get<__nv_bfloat16>((size_t)T * n_out);
+            BLK_CUDA(cudaMemcpyAsync(dw, norm_w, (size_t)n_out * 4, cudaMemcpyHostToDevice, st));
+        }
+        __nv_bfloat16* panel = nullptr;
+        if (form == 1) {
+            panel = sc.get<__nv_bfloat16>(prefill_panel_elems(parts, n_mats, op == 2));
+            cudaError_t err = cudaSuccess;
+            if (!prefill_panel_fill(parts, n_mats, op == 2, panel, st, &err)) throw BlkError(BLK_ERR_ARG, "blk_test_gemm: these weights take the fused form only");
+            BLK_CUDA(err);
+        }
+        PendingReduce pend;
+        const size_t ws_elems = (size_t)sms * 65536;
+        const SplitKWs sk{split ? sc.get<float>(ws_elems) : nullptr, ws_elems, split == 2 ? &pend : nullptr};
+        GemmPlan gp;
+        {
+            const ChainPdl chain_scope(T);
+            const SplitKWs* skp = split ? &sk : nullptr;
+            if (op == 0 && n_mats == 1) BLK_CUDA(prefill_gemm(*parts[0].W, dxb, T, dc, ldc, parts[0].bias, 0, st, panel, skp, &gp));
+            else if (op == 0) BLK_CUDA(prefill_gemm_multi(parts, n_mats, dxb, T, dc, ldc, st, panel, skp, &gp));
+            else if (op == 1) BLK_CUDA(prefill_gemm(*parts[0].W, dxb, T, dc, ldc, nullptr, 1, st, panel, skp, &gp));
+            else BLK_CUDA(prefill_gemm_swiglu(*parts[0].W, *parts[1].W, dxb, T, dh, n_out, st, panel, skp, &gp));
+            if (norm_w) rmsnorm_bf16_launch(dc, dw, (int)n_out, eps, dxn, T, st, &pend);
+            BLK_CUDA(cudaGetLastError());
+        }
+        if (pend.ws) throw BlkError(BLK_ERR_CUDA, "blk_test_gemm: a deferred split-K reduce was left unconsumed");
+        if (op == 2 || norm_w) {
+            float* df = sc.get<float>((size_t)T * n_out);
+            bf16_to_f32_kernel<<<grid_of((size_t)T * n_out), 256, 0, st>>>(op == 2 ? dh : dxn, df, (size_t)T * n_out);
+            BLK_CUDA(cudaGetLastError());
+            BLK_CUDA(cudaMemcpyAsync(h_or_xn, df, (size_t)T * n_out * 4, cudaMemcpyDeviceToHost, st));
+        }
+        if (op != 2) BLK_CUDA(cudaMemcpyAsync(c_inout, dc, (size_t)T * n_out * 4, cudaMemcpyDeviceToHost, st));
+        BLK_CUDA(cudaStreamSynchronize(st));
+        if (plan) *plan = blk_test_gemm_plan{gp.n_sm, gp.launches, gp.k_splits, gp.n_whole, gp.deferred ? 1 : 0, gp.panel ? 1 : 0};
+    });
+}
+
+// row_topk_gather_kernel over host logits [n_rows][n_vocab], launched as a verify pass does: rows_per_launch rows per launch, row0 = the
+// first row of the launch, logits of the launch's rows only.  top_ids == nullptr: the gather alone.
+extern "C" blk_status blk_test_row_topk(int32_t device, const float* logits, int32_t n_rows, int32_t n_vocab, int32_t rows_per_launch,
+                                        const int32_t* claimed, const int32_t* n_claimed, float* gathered, int32_t* top_ids, float* top_logits) {
+    return guarded([&] {
+        if (blk_init() != BLK_OK) throw BlkError(BLK_ERR_NO_DEVICE, g_last_error);
+        if (!logits || !claimed || !n_claimed || !gathered || n_rows <= 0 || n_vocab < 10 || rows_per_launch <= 0 || (!top_ids != !top_logits))
+            throw BlkError(BLK_ERR_ARG, "blk_test_row_topk: bad arguments");
+        BLK_CUDA(cudaSetDevice(device));
+        Scratch sc;
+        const size_t n = (size_t)n_rows;
+        float* dl = sc.get<float>(n * n_vocab);
+        int32_t* dcl = sc.get<int32_t>(n * 10); int32_t* dnc = sc.get<int32_t>(n);
+        float* dg = sc.get<float>(n * 10); int32_t* dti = sc.get<int32_t>(n * 10); float* dtl = sc.get<float>(n * 10);
+        BLK_CUDA(cudaMemcpy(dl, logits, n * n_vocab * 4, cudaMemcpyHostToDevice));
+        BLK_CUDA(cudaMemcpy(dcl, claimed, n * 10 * 4, cudaMemcpyHostToDevice));
+        BLK_CUDA(cudaMemcpy(dnc, n_claimed, n * 4, cudaMemcpyHostToDevice));
+        BLK_CUDA(cudaMemset(dg, 0xff, n * 10 * 4));
+        for (int r0 = 0; r0 < n_rows; r0 += rows_per_launch) {
+            const int rows = std::min(rows_per_launch, n_rows - r0);
+            RowTopkArgs ta{};
+            ta.logits = dl + (size_t)r0 * n_vocab; ta.ld = n_vocab; ta.n_vocab = n_vocab; ta.row0 = r0;
+            ta.claimed = dcl; ta.n_claimed = dnc; ta.gathered = dg;
+            ta.top_ids = top_ids ? dti : nullptr; ta.top_logits = dtl;
+            row_topk_gather_kernel<<<rows, 256>>>(ta);
+            BLK_CUDA(cudaGetLastError());
+        }
+        BLK_CUDA(cudaMemcpy(gathered, dg, n * 10 * 4, cudaMemcpyDeviceToHost));
+        if (top_ids) {
+            BLK_CUDA(cudaMemcpy(top_ids, dti, n * 10 * 4, cudaMemcpyDeviceToHost));
+            BLK_CUDA(cudaMemcpy(top_logits, dtl, n * 10 * 4, cudaMemcpyDeviceToHost));
+        }
+    });
+}
+
+// claimed_logits_kernel (the sparse vocabulary projection of a verify pass) over weights of ggml type `type` and xn [n][k] (rounded to
+// bf16 on the device as the pass's RMSNorm output is)
+extern "C" blk_status blk_test_claimed_logits(int32_t device, int32_t type, const void* w_blocks, int64_t rows, int64_t k, const float* xn, int32_t n,
+                                              const int32_t* claimed, const int32_t* n_claimed, float* gathered) {
+    return guarded([&] {
+        if (!w_blocks || !xn || !claimed || !n_claimed || !gathered || n <= 0 || rows <= 0 || k <= 0) throw BlkError(BLK_ERR_ARG, "blk_test_claimed_logits: bad arguments");
+        TestMat tm; test_upload(tm, device, type, w_blocks, rows, k);
+        Scratch sc;
+        float* dx = sc.get<float>((size_t)n * k); __nv_bfloat16* dxb = sc.get<__nv_bfloat16>((size_t)n * k);
+        int32_t* dcl = sc.get<int32_t>((size_t)n * 10); int32_t* dnc = sc.get<int32_t>(n); float* dg = sc.get<float>((size_t)n * 10);
+        BLK_CUDA(cudaMemcpy(dx, xn, (size_t)n * k * 4, cudaMemcpyHostToDevice));
+        BLK_CUDA(cudaMemcpy(dcl, claimed, (size_t)n * 40, cudaMemcpyHostToDevice));
+        BLK_CUDA(cudaMemcpy(dnc, n_claimed, (size_t)n * 4, cudaMemcpyHostToDevice));
+        BLK_CUDA(cudaMemset(dg, 0xff, (size_t)n * 40));
+        BLK_CUDA(convert_f32_to_bf16(dx, dxb, (size_t)n * k, nullptr));
+        BLK_CUDA(prefill_claimed_logits(tm.W, dxb, dcl, dnc, n, dg, nullptr));
+        BLK_CUDA(cudaMemcpy(gathered, dg, (size_t)n * 40, cudaMemcpyDeviceToHost));
     });
 }
 

@@ -58,7 +58,7 @@ GemmKernel pick_kernel(int ta, int tb) {
 
 // panel: nullptr for the fused (in-kernel dequantisation) form, else the bf16 panel (panel_layout) the B tiles are read from
 cudaError_t launch_gemm(PrefillGemmArgs& a, int ta, int tb, const __nv_bfloat16* X, cudaStream_t st, const __nv_bfloat16* panel = nullptr,
-                        const SplitKWs* sk = nullptr) {
+                        const SplitKWs* sk = nullptr, GemmPlan* plan = nullptr) {
     EncodeTiledFn enc = encode_tiled();
     if (!enc) return cudaErrorNotSupported;
     if (a.K % PG_BK || a.T <= 0 || a.n_tiles <= 0) return cudaErrorInvalidValue;
@@ -100,12 +100,14 @@ cudaError_t launch_gemm(PrefillGemmArgs& a, int ta, int tb, const __nv_bfloat16*
     const int grid = items < sms ? items : sms;
     e = launch_chain(kernel, dim3((unsigned)grid), dim3(PG_THREADS), PG_SMEM_BYTES, st, tmap, a);
     if (e == cudaSuccess) e = cudaGetLastError();
+    if (plan) { plan->n_sm = sms; plan->launches++; plan->k_splits = a.k_splits; plan->n_whole = a.n_whole; plan->deferred = false; plan->panel = panel != nullptr; }
     if (e != cudaSuccess || a.k_splits == 1) return e;
     if (sk && sk->defer && a.mode == PG_ACCUM && a.n_whole == 0 && a.nseg == 1 && a.seg[0].col0 == 0 && !a.seg[0].bias &&
         a.seg[0].W.N % PG_BN == 0 && a.ldc == a.seg[0].W.N) {
         // every tile is split and full width: the caller's next RMSNorm over C adds the partial sums (same order: splits, then the residual)
         if (sk->defer->ws) return cudaErrorInvalidValue;      // an earlier deferred reduce was never consumed: fail loudly, never drop partial sums
         *sk->defer = PendingReduce{a.ws, a.k_splits, (a.T + PG_BM - 1) / PG_BM};
+        if (plan) plan->deferred = true;
         return cudaSuccess;
     }
     e = launch_chain(splitk_reduce_kernel, dim3((unsigned)(tiles - a.n_whole), 32), dim3(256), 0, st, a);
@@ -144,13 +146,13 @@ long long panel_layout(const GemmPart* parts, int n_parts, bool swiglu, long lon
 } // namespace
 
 cudaError_t prefill_gemm(const QMat& W, const __nv_bfloat16* X, int T, float* C, long long ldc, const float* bias, int mode, cudaStream_t st,
-                         const __nv_bfloat16* panel, const SplitKWs* sk) {
+                         const __nv_bfloat16* panel, const SplitKWs* sk, GemmPlan* plan) {
     PrefillGemmArgs a{};
     a.nseg = 1; a.seg[0] = {W, bias, 0, 0};
     a.C = C; a.ldc = ldc; a.T = T; a.K = W.K; a.mode = mode;
     a.n_tiles = (W.N + PG_BN - 1) / PG_BN;
     const bool use_panel = panel && panel_type_ok(W.type) && W.K % 64 == 0;
-    return launch_gemm(a, W.type, W.type, X, st, use_panel ? panel : nullptr, (W.N % 4 == 0 && ldc % 4 == 0) ? sk : nullptr);
+    return launch_gemm(a, W.type, W.type, X, st, use_panel ? panel : nullptr, (W.N % 4 == 0 && ldc % 4 == 0) ? sk : nullptr, plan);
 }
 // the dequantisation passes alone, so that a caller can run them on a second stream one GEMM ahead; false = this combination takes
 // the fused form (the GEMM call must then get panel = nullptr)
@@ -171,7 +173,7 @@ size_t prefill_panel_elems(const GemmPart* parts, int n_parts, bool swiglu) {
 }
 
 cudaError_t prefill_gemm_multi(const GemmPart* parts, int n_parts, const __nv_bfloat16* X, int T, float* C, long long ldc, cudaStream_t st,
-                               const __nv_bfloat16* panel, const SplitKWs* sk) {
+                               const __nv_bfloat16* panel, const SplitKWs* sk, GemmPlan* plan) {
     bool all_panel = panel != nullptr && n_parts >= 1 && n_parts <= 3;
     for (int i = 0; i < n_parts && all_panel; i++) all_panel = panel_type_ok(parts[i].W->type) && parts[i].W->K == parts[0].W->K && parts[i].col0 % 4 == 0;
     bool fuse = n_parts >= 2 && n_parts <= 3 && parts[0].W->type == parts[1].W->type;
@@ -179,7 +181,7 @@ cudaError_t prefill_gemm_multi(const GemmPart* parts, int n_parts, const __nv_bf
     if (fuse && n_parts == 3 && !pick_kernel(parts[0].W->type, parts[2].W->type)) fuse = false;
     if (!all_panel && !fuse) {
         for (int i = 0; i < n_parts; i++) {
-            cudaError_t e = prefill_gemm(*parts[i].W, X, T, C + parts[i].col0, ldc, parts[i].bias, 0, st, nullptr, nullptr);     // (column-offset C: no split-K)
+            cudaError_t e = prefill_gemm(*parts[i].W, X, T, C + parts[i].col0, ldc, parts[i].bias, 0, st, nullptr, nullptr, plan);     // (column-offset C: no split-K)
             if (e != cudaSuccess) return e;
         }
         return cudaSuccess;
@@ -192,22 +194,22 @@ cudaError_t prefill_gemm_multi(const GemmPart* parts, int n_parts, const __nv_bf
     for (int i = 0; i < n_parts; i++) a.seg[i] = {*parts[i].W, parts[i].bias, parts[i].col0, (int)(row0[i] / PG_BN)};
     bool sk_ok = ldc % 4 == 0;
     for (int i = 0; i < n_parts; i++) sk_ok = sk_ok && parts[i].W->N % 4 == 0;
-    return launch_gemm(a, parts[0].W->type, n_parts == 3 ? parts[2].W->type : parts[0].W->type, X, st, all_panel ? panel : nullptr, sk_ok ? sk : nullptr);
+    return launch_gemm(a, parts[0].W->type, n_parts == 3 ? parts[2].W->type : parts[0].W->type, X, st, all_panel ? panel : nullptr, sk_ok ? sk : nullptr, plan);
 }
 
 cudaError_t prefill_gemm_swiglu(const QMat& gate, const QMat& up, const __nv_bfloat16* X, int T, __nv_bfloat16* H, long long ldh, cudaStream_t st,
-                                const __nv_bfloat16* panel, const SplitKWs* sk) {
+                                const __nv_bfloat16* panel, const SplitKWs* sk, GemmPlan* plan) {
     if (gate.type != up.type || gate.N != up.N || gate.K != up.K || ldh % 8) return cudaErrorInvalidValue;
     PrefillGemmArgs a{};
     a.nseg = 2; a.seg[0] = {gate, nullptr, 0, 0}; a.seg[1] = {up, nullptr, 0, 0};
     a.H = H; a.ldh = ldh; a.T = T; a.K = gate.K; a.mode = PG_SWIGLU;
     a.n_tiles = (gate.N + 127) / 128;
-    if (!(panel && panel_type_ok(gate.type) && gate.K % 64 == 0)) return launch_gemm(a, gate.type, gate.type, X, st, nullptr, sk);
+    if (!(panel && panel_type_ok(gate.type) && gate.K % 64 == 0)) return launch_gemm(a, gate.type, gate.type, X, st, nullptr, sk, plan);
     const GemmPart parts[2] = {{&gate, nullptr, 0}, {&up, nullptr, 0}};
     long long row0[2];
     panel_layout(parts, 2, true, row0);
     a.panel_up_row0 = (int)row0[1];
-    return launch_gemm(a, gate.type, gate.type, X, st, panel, sk);
+    return launch_gemm(a, gate.type, gate.type, X, st, panel, sk, plan);
 }
 
 namespace {

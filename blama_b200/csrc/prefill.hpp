@@ -18,18 +18,21 @@ namespace blk {
 // that follows adds them while it reads the row anyway (rmsnorm_bf16_launch), instead of a reduce kernel of its own
 struct PendingReduce { const float* ws = nullptr; int S = 0, m_tiles = 0; };
 struct SplitKWs { float* ws; size_t elems; PendingReduce* defer = nullptr; };
+// plan != nullptr: what the call launched (unit tests check that a case runs the path it names).  launches counts GEMM kernel
+// launches and accumulates; the other fields describe the last one (k_splits 1 and n_whole = every tile when nothing was split)
+struct GemmPlan { int n_sm = 0, launches = 0, k_splits = 0, n_whole = 0; bool deferred = false, panel = false; };
 cudaError_t prefill_gemm(const QMat& W, const __nv_bfloat16* X, int T, float* C, long long ldc, const float* bias, int mode, cudaStream_t st,
-                         const __nv_bfloat16* panel = nullptr, const SplitKWs* sk = nullptr);
+                         const __nv_bfloat16* panel = nullptr, const SplitKWs* sk = nullptr, GemmPlan* plan = nullptr);
 
 // several matrices with the same K in one launch: C[:, col0_s : col0_s + N_s] = X . W_s^T (+bias_s).  Matrices 0 and 1 must share
 // a weight type.  Falls back to one launch per matrix when a column offset is not 4-element aligned.
 struct GemmPart { const QMat* W; const float* bias; int col0; };
 cudaError_t prefill_gemm_multi(const GemmPart* parts, int n_parts, const __nv_bfloat16* X, int T, float* C, long long ldc, cudaStream_t st,
-                               const __nv_bfloat16* panel = nullptr, const SplitKWs* sk = nullptr);
+                               const __nv_bfloat16* panel = nullptr, const SplitKWs* sk = nullptr, GemmPlan* plan = nullptr);
 
 // H[T][ff] (bf16) = silu(X . Wgate^T) * (X . Wup^T), one launch, SwiGLU in the GEMM epilogue
 cudaError_t prefill_gemm_swiglu(const QMat& gate, const QMat& up, const __nv_bfloat16* X, int T, __nv_bfloat16* H, long long ldh, cudaStream_t st,
-                                const __nv_bfloat16* panel = nullptr, const SplitKWs* sk = nullptr);
+                                const __nv_bfloat16* panel = nullptr, const SplitKWs* sk = nullptr, GemmPlan* plan = nullptr);
 // The dequantisation passes of the two-pass form: the panel of one GEMM over parts (prefill_gemm, prefill_gemm_multi), or with
 // swiglu = true over {gate, up} (prefill_gemm_swiglu).  A caller can run them on a second stream one GEMM ahead.
 // Return false when the combination takes the fused form (the GEMM call must then get panel = nullptr).

@@ -223,9 +223,22 @@ BLK_API blk_status blk_flush_l2(blk_ctx*);
 /* y[r] = W[r,:] . x through the decode GEMV kernel of ggml type `type` (raw ggml blocks in, host buffers) */
 BLK_API blk_status blk_test_gemv(int32_t device, int32_t type, const void* w_blocks, int64_t rows, int64_t k,
                                  const float* x, float* y);
-/* Y[t][r] = W[r,:] . X[t,:] through the prefill tcgen05 GEMM (bf16 operands, f32 accumulate) */
-BLK_API blk_status blk_test_gemm(int32_t device, int32_t type, const void* w_blocks, int64_t rows, int64_t k,
-                                 const float* x, int64_t n_tok, float* y);
+/* The prefill tcgen05 GEMM (bf16 operands, f32 accumulate) called the way a multi-token pass calls it, inside the pass's programmatic
+ * dependent launch scope.  mats: weights of ggml type `type`, rows x k (raw ggml blocks), optional bias [rows]; x [n_tok][k] f32 (rounded
+ * to bf16 on the device).
+ *   op 0: C[:, col0_i .. col0_i + rows_i) = X W_i^T (+ bias_i) for 1 - 3 matrices side by side (col0_i = rows of the matrices before i;
+ *         QKV / lm_head); c_inout [n_tok][sum rows] in / out (columns the GEMM must write can be preset to NaN)
+ *   op 1: C += X W^T, one matrix (Wo / down onto the residual); c_inout [n_tok][rows] in / out.  norm_w [rows] != NULL: then the RMSNorm
+ *         of the pass, h_or_xn [n_tok][rows] = bf16(rmsnorm(C) * norm_w) as f32
+ *   op 2: h_or_xn [n_tok][rows] = bf16(silu(X Wgate^T) * (X Wup^T)) as f32, mats = {gate, up}
+ * form: 0 fused (de-quantised inside the GEMM), 1 panel (the bf16 panel filled first; BLK_ERR_ARG for weights that take the fused form only).
+ * split: 0 no split-K workspace, 1 a workspace of n_SM x 65536 floats, 2 the same with the reduce deferred to the RMSNorm (op 1 with norm_w).
+ * plan (may be NULL) receives what ran: the SM count, GEMM launches, K splits, whole tiles (all tiles when not split), whether the reduce was
+ * deferred and whether the panel kernel ran. */
+typedef struct { int32_t type; const void* blocks; int64_t rows; const float* bias; } blk_test_matrix;
+typedef struct { int32_t n_sm, launches, k_splits, n_whole, deferred, panel; } blk_test_gemm_plan;
+BLK_API blk_status blk_test_gemm(int32_t device, int32_t op, const blk_test_matrix* mats, int32_t n_mats, int64_t k, const float* x, int64_t n_tok,
+                                 int32_t form, int32_t split, const float* norm_w, float eps, float* c_inout, float* h_or_xn, blk_test_gemm_plan* plan);
 /* average duration of the prefill GEMM on the given weights with n_tok resident bf16 activations (CUDA events) */
 BLK_API blk_status blk_bench_gemm(int32_t device, int32_t type, const void* w_blocks, int64_t rows, int64_t k, int64_t n_tok, int32_t iters, float* avg_ms);
 /* The non-GEMM kernels of the prefill path, one at a time (host buffers in / out; f16 / bf16 results come back as the exact values in
@@ -250,6 +263,14 @@ BLK_API blk_status blk_test_decode_attn_batch(int32_t device, int32_t n, const f
  * edited rows' top-k (descending, ties to the lower id), through the same two launches. */
 BLK_API blk_status blk_test_logit_edits(int32_t device, const float* logits, int32_t n_rows, int32_t n_vocab, const blk_logit_edits* per_row,
                                         int32_t k, blk_token_data* out);
+/* The output kernels of a verify pass.  blk_test_row_topk: row_topk_gather_kernel over logits [n_rows][n_vocab], rows_per_launch rows per
+ * launch as the pass chunks them: gathered[r][j] = logit of claimed[r][j] (j < n_claimed[r]; 0 past it, -inf outside the vocabulary) and,
+ * when top_ids != NULL, the top 10 of each row (descending, ties to the lower id).  blk_test_claimed_logits: claimed_logits_kernel, the same
+ * gathered[n][10] computed as dot(bf16(dequant(W[id])), bf16(xn[t])) with W of ggml type `type`, rows x k. */
+BLK_API blk_status blk_test_row_topk(int32_t device, const float* logits, int32_t n_rows, int32_t n_vocab, int32_t rows_per_launch,
+                                     const int32_t* claimed, const int32_t* n_claimed, float* gathered, int32_t* top_ids, float* top_logits);
+BLK_API blk_status blk_test_claimed_logits(int32_t device, int32_t type, const void* w_blocks, int64_t rows, int64_t k, const float* xn, int32_t n,
+                                           const int32_t* claimed, const int32_t* n_claimed, float* gathered);
 /* dequantise through the device re-tile + dequant kernels */
 BLK_API blk_status blk_test_dequant(int32_t device, int32_t type, const void* w_blocks, int64_t rows, int64_t k, float* out);
 

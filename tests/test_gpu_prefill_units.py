@@ -124,3 +124,115 @@ def test_prefill_attention_rejects_a_shape_without_a_kernel():
     with pytest.raises(capi.BlkError) as e:
         capi.test_prefill_attn(q, kv, kv, 0, 16, 1, 128)
     assert e.value.code == 4      # BLK_ERR_ARG
+
+
+# ---- the output kernels of a verify pass -------------------------------------------------------------------------------------------
+def _thread_share(V: int, t: int):
+    """the elements thread t of row_topk_gather_kernel reads: float4 words t, t + 256, ... of a row when V % 4 == 0, else t, t + 256, ..."""
+    if V % 4 == 0:
+        return [4 * i + c for i in range(t, V // 4, 256) for c in range(4)]
+    return list(range(t, V, 256))
+
+
+def _topk_rows(V: int, rng):
+    """(kind, row): the shapes of row the threshold selection can get wrong"""
+    rows = []
+    r = (rng.standard_normal(V) * 3.0).astype(np.float32)
+    rows.append(("random", r))
+    rows.append(("constant", np.full(V, 1.5, dtype=np.float32)))
+    # nine distinct maxima, then min(2000, V - 20) copies of the 10th value: more than 1024 survivors (the fallback) wherever V allows
+    r = rng.uniform(-5.0, 0.0, V).astype(np.float32)
+    pos = rng.permutation(V)
+    r[pos[:9]] = np.arange(9, dtype=np.float32) + 10.0
+    r[pos[9:9 + min(2000, V - 20)]] = 5.0
+    rows.append(("10th-value-x2000", r))
+    # seven distinct maxima, then six copies of one value straddling ranks 8 .. 13 (ties broken by the lower id), few survivors
+    r = rng.uniform(-5.0, 0.0, V).astype(np.float32)
+    r[pos[:7]] = np.arange(7, dtype=np.float32) + 10.0
+    r[pos[7:13]] = 5.0
+    rows.append(("ties-at-rank-10", r))
+    # every maximum inside one thread's share (pass 1 sees a single large thread maximum)
+    r = rng.uniform(-5.0, 0.0, V).astype(np.float32)
+    share = _thread_share(V, 37)[:12]
+    r[share] = np.arange(len(share), dtype=np.float32) + 10.0
+    rows.append(("one-thread", r))
+    # fewer than ten finite values: the rest of the top ten are -inf, lowest ids first
+    r = np.full(V, -np.inf, dtype=np.float32)
+    r[pos[:6]] = rng.standard_normal(6).astype(np.float32)
+    rows.append(("six-finite", r))
+    return rows
+
+
+@pytest.mark.parametrize("V", [128256, 152064, 32002, 1000])
+def test_row_topk_gather_bit_exact(V):
+    """row_topk_gather_kernel (top ten of each row, descending, ties to the lower id, and the logits at the claimed ids) against numpy,
+    bit for bit.  V = 32002 takes the scalar path (V % 4 != 0); the rows with 2000 copies of the 10th value, constant and mostly -inf
+    take the fallback for more than 1024 survivors.  Rows are launched five at a time, as a pass chunks them (row0 > 0)."""
+    from blama_b200 import capi
+
+    capi.init()
+    rng = np.random.default_rng(V)
+    kinds = _topk_rows(V, rng) + _topk_rows(V, np.random.default_rng(V + 1))
+    logits = np.stack([r for _, r in kinds])
+    n = len(kinds)
+    claimed = np.zeros((n, 10), dtype=np.int32)
+    n_claimed = np.zeros(n, dtype=np.int32)
+    for i in range(n):
+        claimed[i] = np.concatenate([[0, V - 1, V, -1], rng.integers(-3, V + 3, 6)])
+        rng.shuffle(claimed[i])
+        n_claimed[i] = i % 11 if i < 11 else 10
+    g, ti, tl = capi.test_row_topk(logits, claimed, n_claimed, rows_per_launch=5)
+    ids = np.arange(V)
+    for i, (kind, row) in enumerate(kinds):
+        order = np.lexsort((ids, -row.astype(np.float64)))[:10]
+        assert np.array_equal(ti[i], order), (kind, ti[i], order)
+        assert np.array_equal(tl[i], row[order]), (kind, tl[i], row[order])
+        want = np.zeros(10, dtype=np.float32)
+        for j in range(n_claimed[i]):
+            c = claimed[i, j]
+            want[j] = row[c] if 0 <= c < V else -np.inf
+        assert np.array_equal(g[i], want), (kind, g[i], want)
+    print(f"\n[row top-10 V {V}] {n} rows ({', '.join(k for k, _ in kinds[:6])}) bit-exact")
+
+
+@pytest.mark.parametrize("gtype,name", [(12, "Q4_K"), (13, "Q5_K"), (14, "Q6_K"), (8, "Q8_0")])
+def test_claimed_logits(gtype, name, oracle):
+    """claimed_logits_kernel (the sparse vocabulary projection) against float64 on bf16(dequant(W[id])) and bf16(xn), only the claimed rows
+    de-quantised: |got - ref| <= 2e-4 max|ref| as the GEMM; ids outside the vocabulary give -inf and entries past n_claimed 0, exactly."""
+    from blama_b200 import capi
+    from blama_b200 import gguf_synth as gs
+
+    capi.init()
+    V, K, n = 3001, 4096, 12
+    rng = np.random.default_rng(gtype)
+    blk = gs.random_blocks(rng, gtype, V * K, 1.0 / np.sqrt(K))
+    row_bytes = blk.size // V
+    xn = rng.standard_normal((n, K)).astype(np.float32)
+    claimed = rng.integers(-2, V + 2, (n, 10)).astype(np.int32)
+    claimed[-1, :4] = [0, V - 1, V, -1]
+    n_claimed = (np.arange(n) % 11).astype(np.int32)
+    n_claimed[-1] = 10
+    got = capi.test_claimed_logits(gtype, blk, V, K, xn, claimed, n_claimed)
+
+    def bf16(a):
+        u = np.ascontiguousarray(a, dtype=np.float32).view(np.uint32).astype(np.uint64)
+        return ((u + 0x7FFF + ((u >> 16) & 1)) & 0xFFFF0000).astype(np.uint32).view(np.float32)
+
+    xb = bf16(xn).astype(np.float64)
+    ref = np.zeros((n, 10))
+    valid = np.zeros((n, 10), dtype=bool)
+    for t in range(n):
+        for j in range(10):
+            c = int(claimed[t, j])
+            if j >= n_claimed[t]:
+                continue
+            if not 0 <= c < V:
+                ref[t, j] = -np.inf
+                continue
+            w = bf16(oracle.dequantize(gtype, blk[c * row_bytes:(c + 1) * row_bytes], K)).astype(np.float64)
+            ref[t, j] = w @ xb[t]
+            valid[t, j] = True
+    assert np.array_equal(got[~valid], ref[~valid].astype(np.float32))      # -inf outside the vocabulary, 0 past n_claimed
+    err, bound = float(np.abs(got[valid] - ref[valid]).max()), 2e-4 * float(np.abs(ref[valid]).max())
+    print(f"\n[claimed logits {name}] {int(valid.sum())} logits: max err {err:.3g} <= {bound:.3g}")
+    assert err <= bound
