@@ -540,6 +540,16 @@ template <class T> T* halloc(blk_ctx* c, size_t n) {
     c->host_allocs.push_back(p);
     return reinterpret_cast<T*>(p);
 }
+void dfree(blk_ctx* c, void* p) {
+    if (!p) return;
+    c->allocs.erase(std::remove(c->allocs.begin(), c->allocs.end(), p), c->allocs.end());
+    cudaFree(p);
+}
+void hfree(blk_ctx* c, void* p) {
+    if (!p) return;
+    c->host_allocs.erase(std::remove(c->host_allocs.begin(), c->host_allocs.end(), p), c->host_allocs.end());
+    cudaFreeHost(p);
+}
 ActBuf make_act(blk_ctx* c, int K) {
     ActBuf a;
     a.f32 = dalloc<float>(c, K); a.q = dalloc<int8_t>(c, K); a.d = dalloc<float>(c, K / 32 + 8); a.bs = dalloc<int16_t>(c, K / 16 + 8);
@@ -613,13 +623,46 @@ void set_chunking(blk_ctx* c, int n_vocab) {
     c->n_chunks = (n_vocab + (1 << c->chunk_shift) - 1) >> c->chunk_shift;
 }
 
-// the threshold top-k of the context's own logits row (c->logits -> c->top_ids / c->top_logits)
-TopkArgs own_topk_args(const blk_ctx* c) {
+// Every chunk maximum of t back to the empty key, on c's stream.  The selector takes its threshold from the chunk maxima, so they
+// must never over-estimate: the decode lm_head epilogue only raises them (atomicMax), and the selector clears what it read.
+void clear_chunk_max(blk_ctx* c, const TopkRows& t) {
+    const std::vector<int> empty((size_t)t.rows * 256, (int)0x80000000);
+    BLK_CUDA(cudaMemcpyAsync(t.chunk_max, empty.data(), empty.size() * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+}
+
+// (Re)allocates t for `rows` rows, in the state the selector expects between selections (callers have synchronised)
+void alloc_topk(blk_ctx* c, TopkRows& t, int rows) {
+    for (void* p : {(void*)t.chunk_max, (void*)t.cand_l, (void*)t.cand_i, (void*)t.counters, (void*)t.ids, (void*)t.logits}) dfree(c, p);
+    hfree(c, t.h_ids); hfree(c, t.h_logits);
+    t = TopkRows{};
+    const size_t r = rows;
+    t.chunk_max = dalloc<int>(c, r * 256);
+    t.cand_l = dalloc<float>(c, r * c->cand_cap); t.cand_i = dalloc<int>(c, r * c->cand_cap);
+    t.counters = dalloc<unsigned int>(c, 2 * r);
+    t.ids = dalloc<int32_t>(c, r * TOPK_MAX); t.logits = dalloc<float>(c, r * TOPK_MAX);
+    t.h_ids = halloc<int32_t>(c, r * TOPK_MAX); t.h_logits = halloc<float>(c, r * TOPK_MAX);
+    t.rows = rows;
+    clear_chunk_max(c, t);
+    BLK_CUDA(cudaMemsetAsync(t.counters, 0, 2 * r * sizeof(unsigned int), c->stream));
+}
+
+// the selector over rows of `logits` ld floats apart (row = blockIdx.y; a single row needs no ld) into t
+TopkArgs topk_args(const blk_ctx* c, const TopkRows& t, const float* logits, long long ld = 0) {
     TopkArgs tk{};
-    tk.logits = c->logits; tk.n = c->m->n_vocab; tk.chunk_max = c->chunk_max; tk.n_chunks = c->n_chunks;
-    tk.cand_l = c->cand_l; tk.cand_i = c->cand_i; tk.cap = c->cand_cap; tk.count = c->counters + 1; tk.done = c->counters + 2;
-    tk.out_ids = c->top_ids; tk.out_logits = c->top_logits;
+    tk.logits = logits; tk.n = c->m->n_vocab; tk.ld = ld; tk.chunk_max = t.chunk_max; tk.n_chunks = c->n_chunks;
+    tk.cand_l = t.cand_l; tk.cand_i = t.cand_i; tk.cap = c->cand_cap; tk.count = &t.counters[0]; tk.done = &t.counters[1];
+    tk.out_ids = t.ids; tk.out_logits = t.logits;
     return tk;
+}
+
+// the lists of the first `rows` rows to their pinned copies (the caller synchronises before reading them)
+void download_topk(const TopkRows& t, int rows, cudaStream_t st) {
+    BLK_CUDA(cudaMemcpyAsync(t.h_ids, t.ids, (size_t)rows * TOPK_MAX * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    BLK_CUDA(cudaMemcpyAsync(t.h_logits, t.logits, (size_t)rows * TOPK_MAX * sizeof(float), cudaMemcpyDeviceToHost, st));
+}
+
+void copy_topk(const TopkRows& t, int row, int k, blk_token_data* out) {
+    for (int j = 0; j < k; j++) { out[j].token = t.h_ids[row * TOPK_MAX + j]; out[j].logit = t.h_logits[row * TOPK_MAX + j]; }
 }
 
 // The per-op decode attention form of a context of c->n_pages KV pages (decode_kernels.cuh): the single-kernel cluster form when
@@ -704,16 +747,13 @@ void enqueue_step(blk_ctx* c, bool with_head, bool feedback = false) {
         c->launches++;
         prof_mark(c, "mega_decode");
         if (with_head) {
-            TopkArgs tk = own_topk_args(c);
+            TopkArgs tk = topk_args(c, c->top, c->logits);
             tk.feed_tok = feedback ? c->d_tok : nullptr;
             topk_select_kernel<<<16, 1024, 0, c->stream>>>(tk);
             BLK_CUDA(cudaGetLastError());
             c->launches++;
             prof_mark(c, "topk_select");
-            if (!feedback) {
-                BLK_CUDA(cudaMemcpyAsync(c->h_top_ids, c->top_ids, TOPK_MAX * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
-                BLK_CUDA(cudaMemcpyAsync(c->h_top_logits, c->top_logits, TOPK_MAX * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-            }
+            if (!feedback) download_topk(c->top, 1, c->stream);
         }
         return;
     }
@@ -754,20 +794,19 @@ void enqueue_step(blk_ctx* c, bool with_head, bool feedback = false) {
     if (with_head) {
         GemvArgs a{};
         a.nseg = 1; a.seg[0] = {m->output, nullptr, 0, 0}; a.total_pairs = m->n_vocab / 2; a.out = c->logits;
-        a.tail.kind = TAIL_CHUNKMAX; a.tail.chunk_max = c->chunk_max; a.tail.chunk_shift = c->chunk_shift;
+        a.tail.kind = TAIL_CHUNKMAX; a.tail.chunk_max = c->top.chunk_max; a.tail.chunk_shift = c->chunk_shift;
         matvec<EPI_STORE>(c, a, c->x, m->out_norm, c->act_d, "gemv_lm_head");
-        BLK_CUDA(launch_pdl(topk_select_kernel, dim3(16), dim3(1024), 0, c->stream, own_topk_args(c)));
+        BLK_CUDA(launch_pdl(topk_select_kernel, dim3(16), dim3(1024), 0, c->stream, topk_args(c, c->top, c->logits)));
         c->launches++;
         prof_mark(c, "topk_select");
     }
     BLK_CUDA(launch_pdl(advance_pos_kernel, dim3(1), dim3(32), 0, c->stream, c->d_pos, 1));
     c->launches++;
     if (feedback) {
-        BLK_CUDA(launch_pdl(feed_top1_kernel, dim3(1), dim3(32), 0, c->stream, (const int32_t*)c->top_ids, c->d_tok));
+        BLK_CUDA(launch_pdl(feed_top1_kernel, dim3(1), dim3(32), 0, c->stream, (const int32_t*)c->top.ids, c->d_tok));
         c->launches++;
     } else if (with_head) {
-        BLK_CUDA(cudaMemcpyAsync(c->h_top_ids, c->top_ids, TOPK_MAX * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
-        BLK_CUDA(cudaMemcpyAsync(c->h_top_logits, c->top_logits, TOPK_MAX * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+        download_topk(c->top, 1, c->stream);
     }
 }
 
@@ -1093,43 +1132,23 @@ void ensure_prefill_bufs(blk_ctx* c, int T) {
 // top-64 of c->logits through the threshold selector (the row did not come from the decode lm_head mat-vec)
 void topk_of_logits(blk_ctx* c) {
     blk_model* m = c->m;
-    chunk_max_kernel<<<c->n_chunks, 256, 0, c->stream>>>(c->logits, m->n_vocab, c->chunk_shift, c->chunk_max);
+    chunk_max_kernel<<<c->n_chunks, 256, 0, c->stream>>>(c->logits, m->n_vocab, c->chunk_shift, c->top.chunk_max);
     BLK_CUDA(cudaGetLastError()); c->launches++;
-    topk_select_kernel<<<16, 1024, 0, c->stream>>>(own_topk_args(c));
+    topk_select_kernel<<<16, 1024, 0, c->stream>>>(topk_args(c, c->top, c->logits));
     BLK_CUDA(cudaGetLastError()); c->launches++;
-    BLK_CUDA(cudaMemcpyAsync(c->h_top_ids, c->top_ids, TOPK_MAX * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
-    BLK_CUDA(cudaMemcpyAsync(c->h_top_logits, c->top_logits, TOPK_MAX * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    download_topk(c->top, 1, c->stream);
 }
 
 // ---- logit edit pass (logit bias + repetition penalties, blk_*_edited) ----
 static_assert(sizeof(LogitEdit) == sizeof(blk_logit_edit) && offsetof(blk_logit_edit, bias) == offsetof(LogitEdit, bias));
 
-void dfree(blk_ctx* c, void* p) {
-    if (!p) return;
-    c->allocs.erase(std::remove(c->allocs.begin(), c->allocs.end(), p), c->allocs.end());
-    cudaFree(p);
-}
-void hfree(blk_ctx* c, void* p) {
-    if (!p) return;
-    c->host_allocs.erase(std::remove(c->host_allocs.begin(), c->host_allocs.end(), p), c->host_allocs.end());
-    cudaFreeHost(p);
-}
-
-// the edited rows and their top-k scratch for `rows` rows of n_vocab ids (grown, never shrunk; callers have synchronised)
-void ensure_edit_bufs(blk_ctx* c, int rows, int n_vocab) {
-    if (rows <= c->ed_rows) return;
-    for (void* p : {(void*)c->ed_logits, (void*)c->ed_chunk_max, (void*)c->ed_cand_l, (void*)c->ed_cand_i, (void*)c->ed_counters,
-                    (void*)c->ed_top_ids, (void*)c->ed_top_logits}) dfree(c, p);
-    hfree(c, c->ed_h_top_ids); hfree(c, c->ed_h_top_logits);
-    c->ed_rows = 0;
-    c->ed_logits = dalloc<float>(c, (size_t)rows * n_vocab);
-    c->ed_chunk_max = dalloc<int>(c, (size_t)rows * 256);
-    c->ed_cand_l = dalloc<float>(c, (size_t)rows * c->cand_cap); c->ed_cand_i = dalloc<int>(c, (size_t)rows * c->cand_cap);
-    c->ed_counters = dalloc<unsigned int>(c, 2 * (size_t)rows);
-    BLK_CUDA(cudaMemset(c->ed_counters, 0, 2 * (size_t)rows * sizeof(unsigned int)));
-    c->ed_top_ids = dalloc<int32_t>(c, (size_t)rows * TOPK_MAX); c->ed_top_logits = dalloc<float>(c, (size_t)rows * TOPK_MAX);
-    c->ed_h_top_ids = halloc<int32_t>(c, (size_t)rows * TOPK_MAX); c->ed_h_top_logits = halloc<float>(c, (size_t)rows * TOPK_MAX);
-    c->ed_rows = rows;
+// the edited rows and their selection for `rows` rows (grown, never shrunk; callers have synchronised)
+void ensure_edit_bufs(blk_ctx* c, int rows) {
+    if (rows <= c->ed_top.rows) return;
+    dfree(c, c->ed_logits);
+    c->ed_logits = nullptr; c->ed_top.rows = 0;      // a failed allocation leaves nothing that looks usable
+    c->ed_logits = dalloc<float>(c, (size_t)rows * c->m->n_vocab);
+    alloc_topk(c, c->ed_top, rows);
 }
 
 // Checks n rows of edit lists (they come from outside the library) and packs them into the pinned staging block as
@@ -1177,30 +1196,22 @@ size_t pack_edits(blk_ctx* c, const blk_logit_edits* per_row, int n, int n_vocab
 }
 
 // The edit pass over n rows of `logits` (ld floats apart) with the lists pack_edits staged: edited copies + their chunk maxima,
-// the threshold selector on them (blockIdx.y = row), the per-row top-64 copied to c->ed_h_top_* (the caller synchronises).
-void launch_edited_topk(blk_ctx* c, const float* logits, long long ld, int n, int n_vocab, size_t staged, cudaStream_t st) {
+// the threshold selector on them (blockIdx.y = row), the per-row top-64 downloaded to c->ed_top (the caller synchronises).
+void launch_edited_topk(blk_ctx* c, const float* logits, long long ld, int n, size_t staged, cudaStream_t st) {
+    const int n_vocab = c->m->n_vocab;
     BLK_CUDA(cudaMemcpyAsync(c->ed_stage_d, c->ed_stage_h, staged, cudaMemcpyHostToDevice, st));
     LogitEditArgs ea{};
     ea.logits = logits; ea.ld = ld; ea.n = n_vocab;
     ea.params = reinterpret_cast<const float*>(c->ed_stage_d);
     ea.row_off = reinterpret_cast<const int32_t*>(c->ed_stage_d + (size_t)n * 3 * sizeof(float));
     ea.edits = reinterpret_cast<const LogitEdit*>(c->ed_stage_d + (size_t)n * 3 * sizeof(float) + (size_t)(n + 1) * sizeof(int32_t));
-    ea.out = c->ed_logits; ea.chunk_max = c->ed_chunk_max; ea.chunk_shift = c->chunk_shift;
+    ea.out = c->ed_logits; ea.chunk_max = c->ed_top.chunk_max; ea.chunk_shift = c->chunk_shift;
     logit_edit_kernel<<<dim3(c->n_chunks, n), 256, (size_t)sizeof(float) << c->chunk_shift, st>>>(ea);
     BLK_CUDA(cudaGetLastError());
-    TopkArgs tk{};
-    tk.logits = c->ed_logits; tk.n = n_vocab; tk.ld = n_vocab; tk.chunk_max = c->ed_chunk_max; tk.n_chunks = c->n_chunks;
-    tk.cand_l = c->ed_cand_l; tk.cand_i = c->ed_cand_i; tk.cap = c->cand_cap; tk.count = c->ed_counters; tk.done = c->ed_counters + 1;
-    tk.out_ids = c->ed_top_ids; tk.out_logits = c->ed_top_logits;
-    topk_select_kernel<<<dim3(16, n), 1024, 0, st>>>(tk);
+    topk_select_kernel<<<dim3(16, n), 1024, 0, st>>>(topk_args(c, c->ed_top, c->ed_logits, n_vocab));
     BLK_CUDA(cudaGetLastError());
     c->launches += 2;
-    BLK_CUDA(cudaMemcpyAsync(c->ed_h_top_ids, c->ed_top_ids, (size_t)n * TOPK_MAX * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    BLK_CUDA(cudaMemcpyAsync(c->ed_h_top_logits, c->ed_top_logits, (size_t)n * TOPK_MAX * sizeof(float), cudaMemcpyDeviceToHost, st));
-}
-
-void copy_edited_topk(const blk_ctx* c, int row, int k, blk_token_data* out) {
-    for (int j = 0; j < k; j++) { out[j].token = c->ed_h_top_ids[row * TOPK_MAX + j]; out[j].logit = c->ed_h_top_logits[row * TOPK_MAX + j]; }
+    download_topk(c->ed_top, n, st);
 }
 
 // causal flash attention of a prefill chunk: the query heads of a KV head share a CTA when the GQA ratio is a power of two
@@ -1459,16 +1470,7 @@ extern "C" blk_ctx* blk_ctx_create(blk_model* m, int32_t n_ctx, int32_t n_batch)
         c->scores = dalloc<float>(c.get(), (size_t)m->n_head * c->n_pages * KV_PAGE);
         c->logits = dalloc<float>(c.get(), m->n_vocab);
         set_chunking(c.get(), m->n_vocab);
-        c->cand_l = dalloc<float>(c.get(), c->cand_cap); c->cand_i = dalloc<int>(c.get(), c->cand_cap);
-        c->chunk_max = dalloc<int>(c.get(), 256);
-        {
-            std::vector<int> init(256, (int)0x80000000);
-            BLK_CUDA(cudaMemcpy(c->chunk_max, init.data(), 256 * sizeof(int), cudaMemcpyHostToDevice));
-        }
-        c->counters = dalloc<unsigned int>(c.get(), 8 + ff / 256 + 8);
-        BLK_CUDA(cudaMemset(c->counters, 0, (8 + ff / 256 + 8) * sizeof(unsigned int)));
-        c->top_ids = dalloc<int32_t>(c.get(), TOPK_MAX); c->top_logits = dalloc<float>(c.get(), TOPK_MAX);
-        c->h_top_ids = halloc<int32_t>(c.get(), TOPK_MAX); c->h_top_logits = halloc<float>(c.get(), TOPK_MAX);
+        alloc_topk(c.get(), c->top, 1);
         c->ids_cap = 4096;
         c->d_ids = dalloc<int32_t>(c.get(), c->ids_cap); c->d_gath = dalloc<float>(c.get(), c->ids_cap);
         if (m->n_vocab % 2) throw BlkError(BLK_ERR_FORMAT, "vocabulary size must be even");
@@ -1489,7 +1491,7 @@ extern "C" blk_ctx* blk_ctx_create(blk_model* m, int32_t n_ctx, int32_t n_batch)
             P.st2 = ll((size_t)m->n_head * P.max_split * 2);
 
             P.k_pools = c->d_kpools; P.v_pools = c->d_vpools; P.page_table = c->page_table; P.kv_dim = dkv;
-            P.logits = c->logits; P.chunk_max = c->chunk_max; P.chunk_shift = c->chunk_shift;
+            P.logits = c->logits; P.chunk_max = c->top.chunk_max; P.chunk_shift = c->chunk_shift;
             {   // a poll that times out reports here instead of hanging the GPU (mapped pinned host word)
                 void* hp = nullptr;
                 BLK_CUDA(cudaHostAlloc(&hp, sizeof(int), cudaHostAllocMapped)); c->host_allocs.push_back(hp);
@@ -1600,8 +1602,8 @@ extern "C" blk_status blk_state_get(blk_ctx* c, void* dst, int64_t cap, int64_t*
         StateHeader h{STATE_MAGIC, 1u, m->n_layer, kv_dim, m->n_vocab, c->n_past, c->have_logits ? 1 : 0, with_pos ? 1 : 0};
         memcpy(out, &h, sizeof(h)); out += sizeof(h);
         BLK_CUDA(cudaMemcpy(out, c->logits, (size_t)m->n_vocab * 4, cudaMemcpyDeviceToHost)); out += (size_t)m->n_vocab * 4;
-        memcpy(out, c->h_top_ids, TOPK_MAX * 4); out += TOPK_MAX * 4;
-        memcpy(out, c->h_top_logits, TOPK_MAX * 4); out += TOPK_MAX * 4;
+        memcpy(out, c->top.h_ids, TOPK_MAX * 4); out += TOPK_MAX * 4;
+        memcpy(out, c->top.h_logits, TOPK_MAX * 4); out += TOPK_MAX * 4;
         if (with_pos) {      // Self-Extend moved cell positions: they are part of the state
             const int32_t off = c->rope_off;
             memcpy(out, &off, 4); out += 4;
@@ -1628,10 +1630,10 @@ extern "C" blk_status blk_state_set(blk_ctx* c, const void* src, int64_t size) {
         BLK_CUDA(cudaStreamSynchronize(c->stream));
         reset_cells(c, h.n_past);
         BLK_CUDA(cudaMemcpy(c->logits, in, (size_t)m->n_vocab * 4, cudaMemcpyHostToDevice)); in += (size_t)m->n_vocab * 4;
-        memcpy(c->h_top_ids, in, TOPK_MAX * 4); in += TOPK_MAX * 4;
-        memcpy(c->h_top_logits, in, TOPK_MAX * 4); in += TOPK_MAX * 4;
-        BLK_CUDA(cudaMemcpy(c->top_ids, c->h_top_ids, TOPK_MAX * 4, cudaMemcpyHostToDevice));
-        BLK_CUDA(cudaMemcpy(c->top_logits, c->h_top_logits, TOPK_MAX * 4, cudaMemcpyHostToDevice));
+        memcpy(c->top.h_ids, in, TOPK_MAX * 4); in += TOPK_MAX * 4;
+        memcpy(c->top.h_logits, in, TOPK_MAX * 4); in += TOPK_MAX * 4;
+        BLK_CUDA(cudaMemcpy(c->top.ids, c->top.h_ids, TOPK_MAX * 4, cudaMemcpyHostToDevice));
+        BLK_CUDA(cudaMemcpy(c->top.logits, c->top.h_logits, TOPK_MAX * 4, cudaMemcpyHostToDevice));
         if (h.with_positions != 0) {
             materialise_positions(c);
             memcpy(&c->rope_off, in, 4); in += 4;
@@ -1689,20 +1691,13 @@ void decode_batch(blk_ctx* ws, blk_ctx* const* ctxs, const int32_t* tokens, int3
     if (per_row) {          // checked before anything is launched; the staging block is reused every step
         BLK_CUDA(cudaStreamSynchronize(ws->stream));
         staged = pack_edits(ws, per_row, n, V);
-        ensure_edit_bufs(ws, n, V);
+        ensure_edit_bufs(ws, n);
     }
     ensure_prefill_bufs(ws, n);
     if (!ws->bd_host) {
         ws->bd_host = reinterpret_cast<uint8_t*>(halloc<BatchDesc>(ws, 1));
         ws->bd_dev = reinterpret_cast<uint8_t*>(dalloc<BatchDesc>(ws, 1));
-        ws->bd_top_ids = dalloc<int32_t>(ws, BATCH_MAX * TOPK_MAX); ws->bd_top_logits = dalloc<float>(ws, BATCH_MAX * TOPK_MAX);
-        ws->bd_h_top_ids = halloc<int32_t>(ws, BATCH_MAX * TOPK_MAX); ws->bd_h_top_logits = halloc<float>(ws, BATCH_MAX * TOPK_MAX);
-        // per-row scratch of the batched threshold selector
-        ws->bd_chunk_max = dalloc<int>(ws, BATCH_MAX * 256);
-        { std::vector<int> init(BATCH_MAX * 256, (int)0x80000000); BLK_CUDA(cudaMemcpy(ws->bd_chunk_max, init.data(), init.size() * sizeof(int), cudaMemcpyHostToDevice)); }
-        ws->bd_cand_l = dalloc<float>(ws, (size_t)BATCH_MAX * ws->cand_cap); ws->bd_cand_i = dalloc<int>(ws, (size_t)BATCH_MAX * ws->cand_cap);
-        ws->bd_counters = dalloc<unsigned int>(ws, 2 * BATCH_MAX);
-        BLK_CUDA(cudaMemset(ws->bd_counters, 0, 2 * BATCH_MAX * sizeof(unsigned int)));
+        alloc_topk(ws, ws->bd_top, BATCH_MAX);
     }
     cudaStream_t st = ws->stream;
     BLK_CUDA(cudaStreamSynchronize(st));                      // the staging block is reused every step
@@ -1743,24 +1738,19 @@ void decode_batch(blk_ctx* ws, blk_ctx* const* ctxs, const int32_t* tokens, int3
     ws->launches += 2;
     // threshold top-64 of every row (the selector of the batch-1 path, blockIdx.y = row): two launches for the whole batch
     {
-        chunk_max_kernel<<<dim3(ws->n_chunks, n), 256, 0, st>>>(ws->pf_logits, V, ws->chunk_shift, ws->bd_chunk_max, (long long)V);
-        TopkArgs tk{};
-        tk.logits = ws->pf_logits; tk.n = V; tk.ld = V; tk.chunk_max = ws->bd_chunk_max; tk.n_chunks = ws->n_chunks;
-        tk.cand_l = ws->bd_cand_l; tk.cand_i = ws->bd_cand_i; tk.cap = ws->cand_cap; tk.count = ws->bd_counters; tk.done = ws->bd_counters + 1;
-        tk.out_ids = ws->bd_top_ids; tk.out_logits = ws->bd_top_logits;
-        topk_select_kernel<<<dim3(16, n), 1024, 0, st>>>(tk);
+        chunk_max_kernel<<<dim3(ws->n_chunks, n), 256, 0, st>>>(ws->pf_logits, V, ws->chunk_shift, ws->bd_top.chunk_max, (long long)V);
+        topk_select_kernel<<<dim3(16, n), 1024, 0, st>>>(topk_args(ws, ws->bd_top, ws->pf_logits, V));
         BLK_CUDA(cudaGetLastError()); ws->launches += 2;
     }
-    if (per_row) launch_edited_topk(ws, ws->pf_logits, V, n, V, staged, st);
+    if (per_row) launch_edited_topk(ws, ws->pf_logits, V, n, staged, st);
     advance_many_kernel<<<1, BATCH_MAX, 0, st>>>(dv->pos_ptr, n);
     BLK_CUDA(cudaGetLastError()); ws->launches++;
-    BLK_CUDA(cudaMemcpyAsync(ws->bd_h_top_ids, ws->bd_top_ids, (size_t)n * TOPK_MAX * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    BLK_CUDA(cudaMemcpyAsync(ws->bd_h_top_logits, ws->bd_top_logits, (size_t)n * TOPK_MAX * sizeof(float), cudaMemcpyDeviceToHost, st));
+    download_topk(ws->bd_top, n, st);
     BLK_CUDA(cudaStreamSynchronize(st));
     for (int i = 0; i < n; i++) {
         end_cells(ctxs[i], 1, false);
-        for (int j = 0; j < k; j++) { out[(size_t)i * k + j].token = ws->bd_h_top_ids[i * TOPK_MAX + j]; out[(size_t)i * k + j].logit = ws->bd_h_top_logits[i * TOPK_MAX + j]; }
-        if (per_row) copy_edited_topk(ws, i, k, edited + (size_t)i * k);
+        copy_topk(ws->bd_top, i, k, out + (size_t)i * k);
+        if (per_row) copy_topk(ws->ed_top, i, k, edited + (size_t)i * k);
     }
 }
 } // namespace
@@ -1792,9 +1782,8 @@ extern "C" blk_status blk_decode_loop(blk_ctx* c, int32_t first_token, int32_t n
             c->launches += c->launches_loop * n_steps;
         }
         end_cells(c, n_steps, true);
-        BLK_CUDA(cudaMemcpyAsync(c->h_top_ids, c->top_ids, TOPK_MAX * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
-        BLK_CUDA(cudaMemcpyAsync(c->h_top_logits, c->top_logits, TOPK_MAX * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-        if (last_token) { BLK_CUDA(cudaStreamSynchronize(c->stream)); *last_token = c->h_top_ids[0]; }
+        download_topk(c->top, 1, c->stream);
+        if (last_token) { BLK_CUDA(cudaStreamSynchronize(c->stream)); *last_token = c->top.h_ids[0]; }
     });
 }
 
@@ -1805,7 +1794,7 @@ extern "C" blk_status blk_topk_last(blk_ctx* c, int32_t k, blk_token_data* out) 
         BLK_CUDA(cudaSetDevice(c->m->device));
         BLK_CUDA(cudaStreamSynchronize(c->stream));
         check_mega(c);
-        for (int i = 0; i < k; i++) { out[i].token = c->h_top_ids[i]; out[i].logit = c->h_top_logits[i]; }
+        copy_topk(c->top, 0, k, out);
     });
 }
 
@@ -1818,10 +1807,10 @@ extern "C" blk_status blk_topk_last_edited(blk_ctx* c, int32_t k, const blk_logi
         check_mega(c);
         const int V = c->m->n_vocab;
         const size_t staged = pack_edits(c, edits, 1, V);
-        ensure_edit_bufs(c, 1, V);
-        launch_edited_topk(c, c->logits, V, 1, V, staged, c->stream);
+        ensure_edit_bufs(c, 1);
+        launch_edited_topk(c, c->logits, V, 1, staged, c->stream);
         BLK_CUDA(cudaStreamSynchronize(c->stream));
-        copy_edited_topk(c, 0, k, edited);
+        copy_topk(c->ed_top, 0, k, edited);
     });
 }
 
@@ -1833,14 +1822,14 @@ extern "C" blk_status blk_decode_topk_edited(blk_ctx* c, int32_t token, int32_t 
         BLK_CUDA(cudaStreamSynchronize(c->stream));            // the edit staging block is reused every call
         const int V = c->m->n_vocab;
         const size_t staged = pack_edits(c, edits, 1, V);
-        ensure_edit_bufs(c, 1, V);
+        ensure_edit_bufs(c, 1);
         step(c, token, true);
         // after the step's own selection (persistent kernel) or graph replay (per-op path), eagerly on the same stream
-        launch_edited_topk(c, c->logits, V, 1, V, staged, c->stream);
+        launch_edited_topk(c, c->logits, V, 1, staged, c->stream);
         BLK_CUDA(cudaStreamSynchronize(c->stream));
         check_mega(c);
-        for (int i = 0; i < k; i++) { raw[i].token = c->h_top_ids[i]; raw[i].logit = c->h_top_logits[i]; }
-        copy_edited_topk(c, 0, k, edited);
+        copy_topk(c->top, 0, k, raw);
+        copy_topk(c->ed_top, 0, k, edited);
     });
 }
 
@@ -1851,7 +1840,7 @@ extern "C" blk_status blk_decode_topk(blk_ctx* c, int32_t token, int32_t k, blk_
         step(c, token, true);
         BLK_CUDA(cudaStreamSynchronize(c->stream));
         check_mega(c);
-        for (int i = 0; i < k; i++) { out[i].token = c->h_top_ids[i]; out[i].logit = c->h_top_logits[i]; }
+        copy_topk(c->top, 0, k, out);
     });
 }
 
@@ -1902,7 +1891,7 @@ extern "C" blk_status blk_verify_prefill(blk_ctx* c, const int32_t* tokens, int3
                 BLK_CUDA(cudaMemcpyAsync(gathered + (size_t)i * 10, c->d_gath, nc * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
             }
             BLK_CUDA(cudaStreamSynchronize(c->stream));
-            if (top) for (int j = 0; j < 10; j++) { top[(size_t)i * 10 + j].token = c->h_top_ids[j]; top[(size_t)i * 10 + j].logit = c->h_top_logits[j]; }
+            if (top) copy_topk(c->top, 0, 10, top + (size_t)i * 10);
         }
     });
 }
@@ -1948,8 +1937,7 @@ extern "C" blk_status blk_bench_kernel(blk_ctx* c, int32_t which, int32_t iters,
             *avg_ms = ms / (float)iters;
             *bytes_per_launch = m->weight_bytes_per_token + (int64_t)(c->n_past + 1) * blk_model_kv_bytes_per_token(m);
             // the launches left chunk maxima behind (no top-k ran): clear them, and forget the logits
-            std::vector<int> init(256, (int)0x80000000);
-            BLK_CUDA(cudaMemcpyAsync(c->chunk_max, init.data(), 256 * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+            clear_chunk_max(c, c->top);
             BLK_CUDA(cudaStreamSynchronize(c->stream));
             c->have_logits = false;
             return;
@@ -2119,18 +2107,18 @@ extern "C" blk_status blk_test_logit_edits(int32_t device, const float* logits, 
         return fail(BLK_ERR_ARG, "blk_test_logit_edits: bad arguments");
     return guarded([&] {
         if (blk_init() != BLK_OK) throw BlkError(BLK_ERR_NO_DEVICE, g_last_error);
-        blk_model holder; holder.device = device;
+        blk_model holder; holder.device = device; holder.n_vocab = n_vocab;
         blk_ctx c; c.m = &holder;
         BLK_CUDA(cudaSetDevice(device));
         set_chunking(&c, n_vocab);
         const size_t staged = pack_edits(&c, per_row, n_rows, n_vocab);
         BLK_CUDA(cudaStreamCreateWithFlags(&c.stream, cudaStreamNonBlocking));
-        ensure_edit_bufs(&c, n_rows, n_vocab);
+        ensure_edit_bufs(&c, n_rows);
         float* d_logits = dalloc<float>(&c, (size_t)n_rows * n_vocab);
         BLK_CUDA(cudaMemcpyAsync(d_logits, logits, (size_t)n_rows * n_vocab * sizeof(float), cudaMemcpyHostToDevice, c.stream));
-        launch_edited_topk(&c, d_logits, n_vocab, n_rows, n_vocab, staged, c.stream);
+        launch_edited_topk(&c, d_logits, n_vocab, n_rows, staged, c.stream);
         BLK_CUDA(cudaStreamSynchronize(c.stream));
-        for (int r = 0; r < n_rows; r++) copy_edited_topk(&c, r, k, out + (size_t)r * k);
+        for (int r = 0; r < n_rows; r++) copy_topk(c.ed_top, r, k, out + (size_t)r * k);
     });
 }
 

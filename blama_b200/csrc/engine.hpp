@@ -41,6 +41,16 @@ struct LayerWeights {
     const float* bv = nullptr;
 };
 
+// Threshold top-64 of `rows` logits rows (topk_select_kernel, decode_kernels.cuh): the selector's scratch in the layout TopkArgs
+// indexes, the device lists and their pinned copies.  Between selections every chunk maximum holds the empty key and both
+// counters are zero (the selector restores that after reading).
+struct TopkRows {
+    int rows = 0;
+    int* chunk_max = nullptr; float* cand_l = nullptr; int* cand_i = nullptr; unsigned int* counters = nullptr;
+    int32_t* ids = nullptr; float* logits = nullptr;          // device [rows][TOPK_MAX]
+    int32_t* h_ids = nullptr; float* h_logits = nullptr;      // pinned [rows][TOPK_MAX]
+};
+
 } // namespace blk
 
 // persistent decode kernel: stream copy of the weights + phase table (mega_decode.cuh)
@@ -121,11 +131,8 @@ struct blk_ctx {
     int attn_cluster = 0, attn_cap = 0;   // cluster size (0 = three-kernel fallback) and tokens per CTA
     float* part_o = nullptr; float* scores = nullptr;
     float* logits = nullptr;              // [n_vocab] of the last decoded token
-    float* cand_l = nullptr; int* cand_i = nullptr; int n_chunks = 0; int chunk_shift = 10; int cand_cap = 2048;
-    int* chunk_max = nullptr;
-    unsigned int* counters = nullptr;      // [0] residual-norm tail, [1] top-k count, [2] top-k done, [8..] per-block quant tails
-    int32_t* top_ids = nullptr; float* top_logits = nullptr;           // device [TOPK_MAX]
-    int32_t* h_top_ids = nullptr; float* h_top_logits = nullptr;       // pinned
+    blk::TopkRows top;                    // its top-64
+    int n_chunks = 0; int chunk_shift = 10; int cand_cap = 2048;      // vocabulary chunks and candidates per row of every selection
     bool have_logits = false;
     cudaGraphExec_t g_full = nullptr, g_body = nullptr, g_loop = nullptr;
     int64_t launches_full = 0, launches_body = 0, launches_loop = 0;
@@ -151,15 +158,13 @@ struct blk_ctx {
     // scratch for gather / verify
     int32_t* d_ids = nullptr; float* d_gath = nullptr; int ids_cap = 0;
     void* flush_buf = nullptr; size_t flush_bytes = 0;
-    // batched decode step (blk_decode_batch): per-row descriptors (pinned host staging + device copy) and per-row top-k lists
+    // batched decode step (blk_decode_batch): per-row descriptors (pinned host staging + device copy) and the top-64 of every row
     uint8_t* bd_host = nullptr; uint8_t* bd_dev = nullptr;
-    int32_t* bd_top_ids = nullptr; float* bd_top_logits = nullptr; int32_t* bd_h_top_ids = nullptr; float* bd_h_top_logits = nullptr;
-    int* bd_chunk_max = nullptr; float* bd_cand_l = nullptr; int* bd_cand_i = nullptr; unsigned int* bd_counters = nullptr;      // [row][...] scratch of the batched top-k
-    // logit edit pass (blk_*_edited, logit_edit.cuh), allocated on first use for ed_rows rows: the edited copies and a top-k scratch
-    // of their own (the raw selection's scratch and results stay untouched), plus the packed edit lists (pinned staging + device copy)
-    int ed_rows = 0;
-    float* ed_logits = nullptr; int* ed_chunk_max = nullptr; float* ed_cand_l = nullptr; int* ed_cand_i = nullptr; unsigned int* ed_counters = nullptr;
-    int32_t* ed_top_ids = nullptr; float* ed_top_logits = nullptr; int32_t* ed_h_top_ids = nullptr; float* ed_h_top_logits = nullptr;
+    blk::TopkRows bd_top;
+    // logit edit pass (blk_*_edited, logit_edit.cuh), allocated on first use for ed_top.rows rows: the edited copies and a selection
+    // of their own (the raw selection stays untouched), plus the packed edit lists (pinned staging + device copy)
+    float* ed_logits = nullptr;
+    blk::TopkRows ed_top;
     uint8_t* ed_stage_h = nullptr; uint8_t* ed_stage_d = nullptr; size_t ed_stage_cap = 0;
     // persistent decode kernel (one cooperative launch per token instead of the per-op graph)
     bool mega_on = false;
